@@ -2,6 +2,7 @@
 """bench.py — throughput of the EGNO / SEGNO hot path on B200 (BASELINE.json metric: trajectories/s).
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's results as DIR/<name>.npy
     python bench.py --impl reference --gpus N ...            # the reference's CPU implementation (oracle port)
     torchrun --nproc-per-node N bench.py --gpus N ...        # one rank per GPU (weak scaling: B per GPU fixed)
 
@@ -12,6 +13,7 @@ configs[2]: N=20, num_timesteps=10, hidden 64, 4 layers) over one batch of B=256
 from __future__ import annotations
 
 import argparse
+import functools
 import json
 import os
 import subprocess
@@ -23,6 +25,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 _STDOUT_FD = None
@@ -44,12 +47,13 @@ UNIT = "trajectories/s"
 MAC_EDGE_REF = 131 * 64 + 64 * 64 + 64 * 64 + 64
 # MACs the fused edge kernel itself executes per edge (first layer's h-part runs per node, outside it)
 MAC_EDGE_KERNEL = 64 * 64 + 64 * 64 + 64 + 3 * 64
+DUMP_BYTES = 64 << 20      # --dump-outputs: upper bound of the files written
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=100, help="timed training steps")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=256, help="trajectories per GPU per step")
@@ -62,7 +66,30 @@ def parse():
     ap.add_argument("--quick", action="store_true", help="device-resident timing only (for profiler runs)")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of replaying one CUDA "
                                                             "graph per training step")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as "
+                    "DIR/<name>.npy (float32): loss, x_out, v_out, h_out (the model's outputs), grads and params (after the "
+                    "optimizer step), both flat in named_parameters() order; rows are sampled with a fixed seed to keep "
+                    f"the files within {DUMP_BYTES >> 20} MB")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of this repo's CUDA path (--impl ours)")
+    return args
+
+
+def dump_outputs(outdir, arrays):
+    """Each array -> <outdir>/<name>.npy in float32.  When the arrays together exceed DUMP_BYTES, every array keeps the
+    same share of its rows, drawn by a generator seeded with 0, so two runs of the same arguments keep the same rows."""
+    os.makedirs(outdir, exist_ok=True)
+    total = sum(4 * a.numel() for a in arrays.values())
+    room = DUMP_BYTES - 4096 * len(arrays)         # less the .npy headers
+    for name, a in arrays.items():
+        a = a.detach().float().cpu()
+        if total > room and a.dim() > 0:
+            keep = a.shape[0] * room // total
+            a = a[torch.randperm(a.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values]
+        np.save(os.path.join(outdir, name + ".npy"), a.numpy())
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -219,7 +246,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 20))
+    steps = args.steps
     warmup = max(1, min(args.warmup, 2))
     cb = cpu_reference_arm(args, steps, warmup, args.cpu_sample)
     line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,
@@ -321,9 +348,16 @@ def run_ours(args):
         resident.append(dict(x=x, nodes=nodes, ea=ea, v=v, lm=lm, target=tgt.to(dev)))
     h2d_bytes = sum(t.numel() * t.element_size() for t in host[0].values())
 
-    def loss_fn(x, nodes, ea, v, lm, target):
+    def loss_fn(x, nodes, ea, v, lm, target, keep=None):
         xo, vo, ho = model(x, nodes, edges, ea, v=v, loc_mean=lm, timesteps_out=t_out)
-        return nb.trajectory_mse(xo, target, T)[0]      # the callers' MSE (main_simulation_simple_no.py:273-276), fused
+        loss = nb.trajectory_mse(xo, target, T)[0]      # the callers' MSE (main_simulation_simple_no.py:273-276), fused
+        if keep is not None:
+            # --dump-outputs: detached views; under graph replay they are the graph's outputs, rewritten by every replay
+            keep.update(loss=loss.detach(), x_out=xo.detach(), v_out=vo.detach(), h_out=ho.detach())
+        return loss
+
+    last = {}                   # the latest timed step's results (--dump-outputs)
+    train_loss = functools.partial(loss_fn, keep=last) if args.dump_outputs else loss_fn
 
     def loss_from_raw(loc, vel, charges, target):
         # prepare_inputs on the device: one featurisation kernel (nb_nbody_features)
@@ -333,14 +367,14 @@ def run_ours(args):
 
     def eager_step(b):
         opt.zero_grad(set_to_none=True)
-        loss = loss_fn(b["x"], b["nodes"], b["ea"], b["v"], b["lm"], b["target"])
+        loss = train_loss(b["x"], b["nodes"], b["ea"], b["v"], b["lm"], b["target"])
         loss.backward()
         opt.step()
         return loss
 
     if use_graph:
         # one CUDA graph per step shape: forward + loss + backward (+ all-reduce) + Adam replayed as a single launch
-        g_res = nb.GraphedStep(loss_fn, {k: resident[0][k] for k in ("x", "nodes", "ea", "v", "lm", "target")}, opt)
+        g_res = nb.GraphedStep(train_loss, {k: resident[0][k] for k in ("x", "nodes", "ea", "v", "lm", "target")}, opt)
         g_raw = nb.GraphedStep(loss_from_raw, {k: host[0][k].to(dev) for k in ("loc", "vel", "charges", "target")}, opt)
 
         def train_step(b):
@@ -392,6 +426,12 @@ def run_ours(args):
         launches = g_res.launches_per_replay * K
     clocks = sampler.stop(window=(tw0, tw1)) if rank == 0 else None
     value = world * B * K / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        ps = list(model.parameters())                 # the optimizer's parameter order
+        gs = g_res.grads if use_graph else [p.grad for p in ps]
+        last["params"] = torch.cat([p.detach().reshape(-1) for p in ps])
+        last["grads"] = torch.cat([(torch.zeros_like(p) if g is None else g.detach()).reshape(-1) for p, g in zip(ps, gs)])
+        dump_outputs(args.dump_outputs, last)
 
     if args.quick:
         lib.nb_profile_enable(1)

@@ -38,6 +38,9 @@ class GraphedStep:
         with torch.cuda.graph(self.graph):
             self.loss = self._eager(zero=False)
         self.launches_per_replay = int(lib.nb_launch_count() - n0)   # kernels of this library inside the graph
+        # the gradient buffers every replay writes, in the optimizer's parameter order (None: no gradient); p.grad itself
+        # points elsewhere once another step over the same parameters is captured
+        self.grads = [p.grad for g in self.opt.param_groups for p in g["params"]] if self.opt is not None else []
 
     def _eager(self, zero: bool = True) -> torch.Tensor:
         if self.opt is not None and zero:

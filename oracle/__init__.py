@@ -13,8 +13,8 @@ fails loudly when its CUDA extension is missing.
 Parity pin status: the reference ships NO tests, golden vectors or known-answer
 fixtures for this path (SURVEY.md §4, §8c) -> "parity unpinned by reference
 tests".  The oracle is instead pinned against outputs of the reference's own
-modules run in the build container: ``tests/golden/make_golden.py`` imports
-``/root/reference`` (through ``oracle/ref_loader.py``), runs the real
+modules: ``tests/golden/make_golden.py`` imports the reference
+(through ``oracle/ref_loader.py``), runs the real
 ``EGNO`` / ``SEGNO.forward_step`` on seeded inputs and commits inputs, weights,
 outputs and parameter gradients under ``tests/golden/*.npz``;
 ``tests/test_oracle_golden.py`` checks the restatement in ``nbody_oracle.py``

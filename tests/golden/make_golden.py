@@ -1,8 +1,8 @@
-"""Generate golden vectors from the REAL reference (run in the build container only).
+"""Generate golden vectors from the REAL reference (needs it installed: oracle/make_ref.py).
 
     python tests/golden/make_golden.py
 
-Imports /root/reference through oracle/ref_loader.py (stubs for torch_geometric /
+Imports the reference through oracle/ref_loader.py (stubs for torch_geometric /
 matplotlib only), simulates a few trajectories with the reference's own
 ``synthetic_sim`` (np.random.seed(43), README.md:6), builds features the way the
 reference callers do, runs the reference ``EGNO`` module and ``SEGNO.forward_step``

@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Golden trajectories of the reference's simulators (build container only: imports /root/reference/synthetic_sim.py).
+"""Golden trajectories of the reference's simulators (imports the reference's synthetic_sim.py via oracle/ref_loader.py).
 
 For every case: seed the global numpy stream, draw the initial conditions with oracle.sim_oracle's samplers (which
 mirror the reference's draw order), re-seed, run the reference's own sample_trajectory -> the stored frames belong to

@@ -7,8 +7,8 @@ SEGNO/train_nbody.py:57-236) with the reference's own dataset classes, loss, Ada
   * the reference's modules  and  * the oracle restatement wrapped as a module                        (not gpu)
 
 on the same simulated data set and the same initial weights; training losses, validation loss, rollout predictions,
-per-frame test MSE and energy curves must agree.  The reference comes from /root/reference (build container) or the
-unmodified copy oracle/make_ref.py installs into oracle/_ref (git-ignored; it travels to the GPU box).
+per-frame test MSE and energy curves must agree.  The reference is imported through oracle/ref_loader.py (the
+original checkout, or the unmodified copy oracle/make_ref.py installs into oracle/_ref); the tests skip without it.
 
 Tolerances (fp32): a 1e-5 relative perturbation of the weights moves these quantities by 1e-5 .. 6e-5 (measured with
 the reference on the CPU), the CUDA path's own forward error is <= 2e-5; the bounds below leave a 20-50x margin.

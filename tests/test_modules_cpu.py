@@ -1,15 +1,12 @@
 """Host-side behaviour of the drop-in modules (no GPU): constructor / state_dict compatibility with the
 reference's checkpoints, error behaviour, and the flat parameter packing."""
-import io
-import contextlib
-
 import pytest
 import torch
 
 import no_node_comparison_b200 as nb
 from no_node_comparison_b200.functional import _EdgeCache, _ParamPack
-from oracle import nbody_oracle as O, ref_loader
-from tests.helpers import load_case
+from oracle import nbody_oracle as O
+from tests.helpers import EGNO_CASES, EGNO_MULTI_CASES, SEGNO_CASES, SEGNO_MULTI_CASES, load_case
 
 
 def _egno(**kw):
@@ -39,21 +36,25 @@ def test_segno_loads_reference_checkpoint_names_and_shapes():
     assert sum(p.numel() for p in m.parameters()) == 33602                # SURVEY.md §8a9
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="reference tree not present (GPU box)")
 def test_same_seed_gives_reference_initial_weights():
-    ref = ref_loader.load_reference()
-    torch.manual_seed(3)
-    with contextlib.redirect_stdout(io.StringIO()):
-        r = ref.EGNO(n_layers=2, in_node_nf=2, in_edge_nf=2, hidden_nf=64, with_v=True, num_modes=2,
-                     num_timesteps=10, device="cpu")
-    torch.manual_seed(3)
-    m = _egno(n_layers=2, num_timesteps=10)
-    assert all(torch.equal(a, b) for a, b in zip(r.state_dict().values(), m.state_dict().values()))
-    torch.manual_seed(3)
-    r = ref.SEGNO(in_node_nf=1, in_edge_nf=2, hidden_nf=64, device="cpu", n_layers=8, recurrent=True)
-    torch.manual_seed(3)
-    s = nb.SEGNO(in_node_nf=1, in_edge_nf=2, hidden_nf=64, device="cpu", n_layers=8, recurrent=True)
-    assert all(torch.equal(a, b) for a, b in zip(r.state_dict().values(), s.state_dict().values()))
+    """The weights of every golden case are the reference modules' initial weights under torch.manual_seed(1)
+    (tests/golden/make_golden.py); the drop-in modules must draw the same values in the same order."""
+    for name in EGNO_CASES + EGNO_MULTI_CASES:
+        d, w, _ = load_case(name)
+        T, n_layers, num_modes = (int(v) for v in d["meta"][2:5])
+        num_inputs = int(d["meta"][5]) if len(d["meta"]) > 5 else 1
+        torch.manual_seed(1)
+        m = _egno(n_layers=n_layers, num_modes=num_modes, num_timesteps=T, num_inputs=num_inputs, varDT="vardt" in name)
+        sd = m.state_dict()
+        assert list(sd) == list(w) and all(torch.equal(sd[k], w[k]) for k in w), name
+    for name in SEGNO_CASES + SEGNO_MULTI_CASES:
+        d, w, _ = load_case(name)
+        agg = None if "agg" not in d else ("sum" if int(d["agg"][0]) == 0 else "attn")
+        torch.manual_seed(1)
+        # constructor defaults for norm_diff / tanh: the golden modules were built with both False
+        s = nb.SEGNO(in_node_nf=1, in_edge_nf=2, hidden_nf=64, device="cpu", n_layers=8, recurrent=True, multiple_agg=agg)
+        sd = s.state_dict()
+        assert list(sd) == list(w) and all(torch.equal(sd[k], w[k]) for k in w), name
 
 
 def test_num_modes_clamp_matches_reference_ctor():

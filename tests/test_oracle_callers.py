@@ -4,8 +4,9 @@
   oracle.energy_charged / energy_gravity      vs  utils.conserved_energy_fun utils.py:126-219
   oracle.trajectory_mse                       vs  the loss lines of run_epoch main_simulation_simple_no.py:268-276
 
-The reference is imported from /root/reference or the unmodified copy under oracle/_ref (oracle/make_ref.py); the tests
-skip when neither is present."""
+The reference is imported through oracle/ref_loader.py (the original checkout, or the unmodified copy under oracle/_ref
+made by oracle/make_ref.py); the tests that call it skip without it.  The loss lines are written out in the test itself
+and need no reference."""
 from __future__ import annotations
 
 import numpy as np
@@ -71,9 +72,8 @@ def test_energies_match_conserved_energy_fun(ref, kind):
     assert rel_err(got, torch.as_tensor(np.asarray(want), dtype=torch.float32)) < 2e-6
 
 
-@needs_ref
 @pytest.mark.parametrize("only_first", [False, True])
-def test_trajectory_mse_matches_the_loss_lines_of_run_epoch(ref, only_first):
+def test_trajectory_mse_matches_the_loss_lines_of_run_epoch(only_first):
     """main_simulation_simple_no.py:268-276 written out with the reference's own criterion object."""
     T, B, N = 4, 3, 5
     g = torch.Generator().manual_seed(2)

@@ -1,5 +1,5 @@
-import sys, torch
-sys.path.insert(0, '/root/repo')
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import no_node_comparison_b200 as nb
 import tests.test_gpu_parity as T
 lib = nb.load_library()
