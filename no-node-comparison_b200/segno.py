@@ -56,6 +56,9 @@ class SEGNO(nn.Module):
             raise ValueError("only the SiLU activation (reference default) is implemented")
         if tanh:
             raise ValueError("tanh=True (gcl.py:57-59) is not implemented (model_confs.yaml:27 uses False)")
+        if norm_diff:
+            # EGNN's coord2radial divides coord_diff by sqrt(radial) + 1: a different model, not computed by the kernels
+            raise ValueError("norm_diff=True (coord2radial) is not implemented (model_confs.yaml uses False)")
         if multiple_agg not in (None, 'sum', 'attn'):
             raise ValueError(f"multiple_agg must be None, 'sum' or 'attn' (model.py:82-90), got {multiple_agg!r}")
         self.hidden_nf = hidden_nf

@@ -225,14 +225,16 @@ def segno_gcl(p: Dict[str, Tensor], h: Tensor, row: Tensor, col: Tensor, x: Tens
 
 
 def segno_forward(p: Dict[str, Tensor], his: Tensor, x: Tensor, row: Tensor, col: Tensor, v: Tensor,
-                  edge_attr: Tensor, T: int, recurrent: bool = True) -> Tuple[Tensor, Tensor, Tensor]:
+                  edge_attr: Tensor, T: int, recurrent: bool = True,
+                  coords_weight: float = 1.0) -> Tuple[Tensor, Tensor, Tensor]:
     """The *intended* SEGNO forward: forward_step(embedding(his), ...) (SEGNO/models/model.py:73,:95-102).
 
     (The literal SEGNO.forward at reference HEAD, model.py:53-92, returns its inputs — SURVEY.md §0.)
     Returns (x, h, v) in the reference's return order."""
     h = linear(his, p, "embedding")                                   # :73
     for _ in range(T):                                                # :96-100 (n_layers := T)
-        h, x, v = segno_gcl(p, h, row, col, x, v, edge_attr, n_layers=T, recurrent=recurrent)
+        h, x, v = segno_gcl(p, h, row, col, x, v, edge_attr, n_layers=T, recurrent=recurrent,
+                            coords_weight=coords_weight)
     return x, h, v
 
 

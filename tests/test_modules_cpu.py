@@ -74,6 +74,9 @@ def test_unsupported_configurations_raise():
     assert _egno(num_inputs=2).embedding.weight.shape == (64, 2 + 2 * 32)
     with pytest.raises(ValueError):
         nb.SEGNO(in_node_nf=1, in_edge_nf=2, hidden_nf=64, tanh=True)
+    # norm_diff=True would divide coord_diff by sqrt(radial) + 1 (EGNN's coord2radial): refused, not silently ignored
+    with pytest.raises(ValueError, match="norm_diff"):
+        nb.SEGNO(in_node_nf=1, in_edge_nf=2, hidden_nf=64, norm_diff=True)
 
 
 def test_cpu_tensors_are_rejected_no_fallback():
