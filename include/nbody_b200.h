@@ -222,6 +222,11 @@ int nb_profile_read(double* ms /*[NB_PROFILE_CATEGORIES]*/, long long* counts /*
  * while another thread is inside a forward / backward call. */
 int nb_set_edge_impl(int impl);
 int nb_get_edge_impl(void);
+/* Edge impl 2, forward: 1 (default) = units of one graph-instance with at least three 128-edge tiles (N = 17 .. 27) run
+ * three tiles in flight per SM (k_edge_fwd_sel3), 0 = they run the two-CTA-per-SM kernel every other shape runs
+ * (cross-check).  M and Fsum are bitwise equal either way. */
+int nb_set_edge_fwd3(int on);
+int nb_get_edge_fwd3(void);
 /* Node-level 64-wide GEMMs and weight-gradient reductions: 1 = tcgen05 kernels (default, product path), 0 = fp32 SIMT
  * kernels (cross-check; the variant the host emulator runs). */
 int nb_set_node_impl(int impl);

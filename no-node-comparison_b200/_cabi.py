@@ -61,6 +61,8 @@ EXPORTS = {
     "nb_set_segno_fused": (C.c_int, [C.c_int]),
     "nb_get_segno_fused": (C.c_int, []),
     "nb_get_edge_impl": (C.c_int, []),
+    "nb_set_edge_fwd3": (C.c_int, [C.c_int]),
+    "nb_get_edge_fwd3": (C.c_int, []),
     "nb_tc_selftest": (C.c_int, [C.c_int32, c_f, c_f, c_f, c_f]),
     "nb_silu_selftest": (C.c_int, [C.c_int64, c_f, c_f, c_f, c_f]),
 }

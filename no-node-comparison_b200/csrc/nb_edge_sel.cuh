@@ -586,6 +586,338 @@ __global__ void __launch_bounds__(NB_THREADS, 2) k_edge_fwd_sel(NbEdgeFwdArgs a)
   if (warp == 0) nb_tmem_dealloc(tm, NB_SF_TMEM_COLS);
 }
 
+// ----------------------------------------------------------------------------- forward, three tiles in flight
+// Whole-graph units of at least three tiles (G = 1, N = 17 .. 27), one CTA per SM.  The tile of k_edge_fwd_sel is a
+// dependent chain of four MMA round trips; at two CTAs per SM an SM has two such chains and no pipe is saturated.  Here
+// the CTA runs three chains: warp group g (warps 4g .. 4g + 3, one thread per tile row, all 64 columns) walks tiles
+// g, g + 3, ... of each unit with its own selector / activation / force tiles and TMEM columns, and warp 12 issues every
+// MMA from one thread.  The issuer serves the groups stage by stage in tile order (gathers of a round of three tiles,
+// then their W2 products, then W3 + M scatter, then the F scatters), so the M / Fsum scatters of a unit are issued, and
+// run, in tile order with tile 0 clearing the accumulators: the per-row arithmetic and the accumulation order are
+// those of k_edge_fwd_sel<false>, and M / Fsum are bitwise equal to it.
+//   groups -> issuer: ready[g] (one arrival after the group's named barrier);  issuer -> group: done[g] (tcgen05.commit)
+// Unit boundaries overlap the next unit's tiles: the node tile and positions are double-buffered (each thread stages its
+// share of the next unit's rows while its first tile of the current unit waits for W2; ntfull[b] counts 384 arrivals),
+// and the group holding a unit's last tile reads the accumulators out while the other groups start the next unit; the
+// issuer holds the next unit's first M scatter until that read-out has arrived on accfree.
+//
+// TMEM columns: group g: [128 g, 128 g + 64) pre-activations | [128 g + 64, +32) hi, [128 g + 96, +32) lo pieces of the
+//               A operand;  [384, 448) M accumulators | [448, 456) Fsum accumulators
+#define NB_F3_GROUPS 3
+#define NB_F3_THREADS (128 * NB_F3_GROUPS + 32)
+#define NB_F3_ISSUER_WARP (4 * NB_F3_GROUPS)
+#define NB_F3_W 0                                    // W2 hi/lo, W3 hi/lo                4 x 8 KB
+#define NB_F3_NT (4 * NB_TC_TILE_BYTES(64))          // node tile hi/lo, two buffers      4 x 8 KB
+#define NB_F3_GRP (NB_F3_NT + 4 * NB_TC_TILE_BYTES(64))
+#define NB_F3_GRP_BYTES (3 * NB_TC_TILE_BYTES(128) + 2 * NB_TILE * 16)  // per group: Sel | T hi | T lo | F hi | F lo
+#define NB_F3_FL (NB_F3_GRP + NB_F3_GROUPS * NB_F3_GRP_BYTES)
+#define NB_F3_NFLOAT (3 * NB_H + 2 * 32 * 3)
+#define NB_EDGE_FWD_SEL3_SMEM(RU) (NB_F3_FL + NB_F3_NFLOAT * 4 + (RU) * 4 + 16 * 8 + 1024)
+#define NB_F3_TMEM_COLS 512
+#define NB_F3_TM_M 384
+#define NB_F3_TM_F 448
+
+__device__ __forceinline__ void nb_named_sync(int id, int nthreads) {
+  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
+}
+__device__ __forceinline__ void nb_mbar_arrive(uint64_t* bar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(nb_smem_u32(bar)) : "memory");
+}
+
+__global__ void __launch_bounds__(NB_F3_THREADS, 1) k_edge_fwd_sel3(NbEdgeFwdArgs a) {
+  NB_PDL_ENTER();
+  extern __shared__ __align__(1024) unsigned char nb_smraw[];
+  unsigned char* base = nb_smraw + ((1024u - (nb_smem_u32(nb_smraw) & 1023u)) & 1023u);
+  unsigned char* W2h = base + NB_F3_W;
+  unsigned char* W2l = W2h + NB_TC_TILE_BYTES(64);
+  unsigned char* W3h = W2l + NB_TC_TILE_BYTES(64);
+  unsigned char* W3l = W3h + NB_TC_TILE_BYTES(64);
+  unsigned char* NT = base + NB_F3_NT;  // buffer b: hi at NT + 2 b x 8 KB, lo 8 KB above
+  float* fl = reinterpret_cast<float*>(base + NB_F3_FL);
+  float* vb2 = fl;
+  float* vb3 = vb2 + NB_H;
+  float* vw4 = vb3 + NB_H;
+  float* xsb = vw4 + NB_H;  // [2][32][3] positions of the unit's nodes, one buffer per node-tile buffer
+  uint32_t* rowinfo = reinterpret_cast<uint32_t*>(xsb + 2 * 32 * 3);
+  const NbEdgeGeom g = a.g;
+  const int RU = g.G * g.EPG;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(rowinfo + RU + (RU & 1));
+  uint64_t* ready = bars;       // [3]
+  uint64_t* done = bars + 3;    // [3]
+  uint64_t* ntfull = bars + 6;  // [2]
+  uint64_t* accfree = bars + 8;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 9);
+  constexpr int NC = 128 * NB_F3_GROUPS;  // compute threads
+
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int grp = warp >> 2, q = warp & 3;
+  const int row = 32 * q + lane;
+
+  if (tid < NB_THREADS) {
+    nb_tc_stage_weight(W2h, W2l, a.w.W2, tid);
+    nb_tc_stage_weight(W3h, W3l, a.w.W3, tid);
+  }
+  for (int idx = tid; idx < 4 * NB_TC_TILE_BYTES(64) / 16; idx += NB_F3_THREADS)
+    reinterpret_cast<uint4*>(NT)[idx] = make_uint4(0u, 0u, 0u, 0u);
+  nb_sel_build_rowinfo(rowinfo, g, tid, NB_F3_THREADS);
+  if (tid < NB_H) {
+    vb2[tid] = __ldg(a.w.b2 + tid);
+    vb3[tid] = __ldg(a.w.b3 + tid);
+    vw4[tid] = __ldg(a.w.w4 + tid);
+  }
+  if (tid == 0) {
+    for (int i = 0; i < NB_F3_GROUPS; ++i) {
+      nb_mbar_init(ready + i, 1);
+      nb_mbar_init(done + i, 1);
+    }
+    nb_mbar_init(ntfull, NC);
+    nb_mbar_init(ntfull + 1, NC);
+    nb_mbar_init(accfree, 128);
+    nb_mbar_fence_init();
+  }
+  if (warp == 0) nb_tmem_alloc(tmem_slot, NB_F3_TMEM_COLS);
+  __syncthreads();
+  // weight rows of both node-tile buffers: 54,55 <- w_rad ; 56 + 2f, 57 + 2f <- w_ef[f]
+  for (int idx = tid; idx < 2 * 10 * 8; idx += NB_F3_THREADS) {
+    const int b = idx / 80, k = (idx % 80) >> 3, j = idx & 7;
+    const int f = (k >> 1) - 1;  // -1: radial
+    float v[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      const int c = 8 * j + i;
+      v[i] = f < 0 ? __ldg(a.w.W1 + (int64_t)c * a.w.ldw1 + a.w.col_rad)
+                   : (f < g.nef ? __ldg(a.w.W1 + (int64_t)c * a.w.ldw1 + a.w.col_ef + f) : 0.f);
+    }
+    unsigned char* nh = NT + 2 * b * NB_TC_TILE_BYTES(64);
+    nb_tc_store8(nh, nh + NB_TC_TILE_BYTES(64), NB_SEL_XC0 + k, j, v);
+  }
+  // the CTA's first unit -> buffer 0
+  if (blockIdx.x < g.n_units) {
+    const NbSelUnit U = nb_sel_unit<false>(g, blockIdx.x, 0);
+    nb_sel_stage_unit(NT, NT + NB_TC_TILE_BYTES(64), a.P, a.Q, U, tid, NB_F3_THREADS);
+    if (tid < U.nrecv * 3) xsb[tid] = __ldg(a.x + (int64_t)U.recv0 * 3 + tid);
+  }
+  nb_fence_async_smem();
+  nb_tc_fence_before();
+  __syncthreads();
+  nb_tc_fence_after();
+  const uint32_t tm = *tmem_slot;
+  const uint32_t idesc_fwd = nb_idesc_bf16(128, 64, 0, 0);  // A K-major, B K-major (W^T)
+  const uint32_t idesc_gat = nb_idesc_bf16(128, 64, 0, 1);  // A K-major, B MN-major
+  const uint32_t idesc_sc = nb_idesc_bf16(64, 64, 1, 1);    // Sel^T . tile
+  const uint32_t idesc_sc8 = nb_idesc_bf16(64, 8, 1, 1);
+
+  if (warp == NB_F3_ISSUER_WARP) {
+    // ---------------------------------------------------------------- MMA issuer
+    if (nb_elect_one()) {
+      const uint32_t sW2h = nb_smem_u32(W2h), sW2l = nb_smem_u32(W2l), sW3h = nb_smem_u32(W3h), sW3l = nb_smem_u32(W3l);
+      const uint32_t sGrp = nb_smem_u32(base + NB_F3_GRP);
+      uint32_t ph_ready = 0;  // bit g: phase of ready[g]
+      int k = 0;
+      for (int uo = blockIdx.x; uo < g.n_units; uo += gridDim.x, ++k) {
+        const int ntl = (nb_sel_unit<false>(g, uo, 0).R + NB_TILE - 1) / NB_TILE;
+        const uint32_t sNh = nb_smem_u32(NT + 2 * (k & 1) * NB_TC_TILE_BYTES(64)), sNl = sNh + NB_TC_TILE_BYTES(64);
+        if (k > 0) nb_mbar_wait(ntfull + (k & 1), ((k - 1) >> 1) & 1);
+        for (int t0 = 0; t0 < ntl; t0 += NB_F3_GROUPS) {
+          const int ng = min(NB_F3_GROUPS, ntl - t0);
+#pragma unroll 1
+          for (int st = 0; st < 4; ++st)
+#pragma unroll 1
+            for (int gi = 0; gi < ng; ++gi) {
+              const uint32_t sSel = sGrp + gi * NB_F3_GRP_BYTES, sTh = sSel + NB_TC_TILE_BYTES(128),
+                             sTl = sTh + NB_TC_TILE_BYTES(128), sFh = sTl + NB_TC_TILE_BYTES(128), sFl = sFh + NB_TILE * 16;
+              const uint32_t tg = tm + 128u * gi;
+              const uint32_t acc = (t0 + gi > 0) ? 1u : 0u;
+              nb_mbar_wait(ready + gi, (ph_ready >> gi) & 1u);
+              ph_ready ^= 1u << gi;
+              nb_tc_fence_after();
+              if (st == 0) {
+                nb_issue_gather(tg, sSel, sNh, sNl, 4, idesc_gat, 0u);
+              } else if (st == 1) {
+                nb_issue_w3_ta(tg, tg + 64, tg + 96, sW2h, sW2l, false, idesc_fwd, 0u);
+              } else if (st == 2) {
+                nb_issue_w3_ta(tg, tg + 64, tg + 96, sW3h, sW3l, false, idesc_fwd, 0u);
+                nb_mma_commit(done + gi);
+                if (t0 + gi == 0 && k > 0) {  // the previous unit's accumulators have been read out
+                  nb_mbar_wait(accfree, (k - 1) & 1);
+                  nb_tc_fence_after();
+                }
+                nb_issue_scatter(tm + NB_F3_TM_M, sSel, sTh, sTl, idesc_sc, acc);  // runs underneath the phi_x head
+                continue;
+              } else {
+                nb_issue_scatter8(tm + NB_F3_TM_F, sSel, sFh, sFl, idesc_sc8, acc);
+              }
+              nb_mma_commit(done + gi);
+            }
+        }
+      }
+    }
+    __syncwarp();
+  } else {
+    // ---------------------------------------------------------------- tile groups
+    unsigned char* Sel = base + NB_F3_GRP + grp * NB_F3_GRP_BYTES;
+    unsigned char* Th = Sel + NB_TC_TILE_BYTES(128);
+    unsigned char* Tl = Th + NB_TC_TILE_BYTES(128);
+    unsigned char* Fh = Tl + NB_TC_TILE_BYTES(128);
+    unsigned char* Fl = Fh + NB_TILE * 16;
+    const uint32_t lq = (uint32_t)(32 * q) << 16;
+    const uint32_t tpre = tm + lq + 128u * grp;  // this thread's row of the group's pre-activations
+    const uint32_t ta_h = tpre + 64, ta_l = tpre + 96;
+    const float b4 = __ldg(a.w.b4);
+    uint32_t phase = 0;
+    bool pend = false;  // the group's last F scatter has not been waited for
+    int k = 0;
+    for (int uo = blockIdx.x; uo < g.n_units; uo += gridDim.x, ++k) {
+      const NbSelUnit U = nb_sel_unit<false>(g, uo, 0);
+      const int R = U.R, ntl = (R + NB_TILE - 1) / NB_TILE;
+      const int b = k & 1;
+      if (k > 0) nb_mbar_wait(ntfull + b, ((k - 1) >> 1) & 1);
+      const float* xs = xsb + b * 96;
+      for (int t = grp; t < ntl; t += NB_F3_GROUPS) {
+        const int r0 = t * NB_TILE;
+        // ---- geometry + selector row
+        float dx = 0.f, dy = 0.f, dz = 0.f, r2 = 0.f;
+        float e[NB_MAX_EF];
+#pragma unroll
+        for (int f = 0; f < NB_MAX_EF; ++f) e[f] = 0.f;
+        int li = 0, lj = 0, gt = 0, rem = 0;
+        const bool valid = nb_sel_row<false>(g, U, rowinfo, r0 + row, li, lj, gt, rem);
+        if (valid) {
+          dx = xs[li * 3 + 0] - xs[lj * 3 + 0];
+          dy = xs[li * 3 + 1] - xs[lj * 3 + 1];
+          dz = xs[li * 3 + 2] - xs[lj * 3 + 2];
+          r2 = dx * dx + dy * dy + dz * dz;
+          const int64_t eoff = ((int64_t)nb_ef_graph(g, gt) * g.EPG + rem) * g.nef;
+#pragma unroll
+          for (int f = 0; f < NB_MAX_EF; ++f)
+            if (f < g.nef) e[f] = __ldg(a.ef + eoff + f);
+        }
+        if (pend) {  // the group's previous scatters read Sel / T / F
+          nb_mbar_wait(done + grp, phase);
+          phase ^= 1;
+          nb_tc_fence_after();
+        }
+        nb_sel_write_row(Sel, row, 0, valid, li, U.RC + lj, r2, e);
+        nb_sel_write_row(Sel, row, 1, valid, li, U.RC + lj, r2, e);
+        nb_fence_async_smem();
+        nb_tc_fence_before();
+        nb_named_sync(1 + grp, 128);
+        if (row == 0) nb_mbar_arrive(ready + grp);
+        nb_mbar_wait(done + grp, phase);
+        phase ^= 1;
+        nb_tc_fence_after();
+        // ---- z1 = SiLU(pre1) -> A operand
+#pragma unroll
+        for (int hf = 0; hf < 2; ++hf) {
+          float v[32];
+          nb_tmem_ld32(tpre + 32 * hf, v);
+#pragma unroll
+          for (int i = 0; i < 32; ++i) v[i] = NB_FWD_SILU(i, v[i]);
+          nb_store32_ta(nullptr, nullptr, row, hf, v, ta_h + 16 * hf, ta_l + 16 * hf);
+        }
+        nb_tmem_st_wait();
+        nb_tc_fence_before();
+        nb_named_sync(1 + grp, 128);
+        if (row == 0) nb_mbar_arrive(ready + grp);
+        if (t == grp && uo + (int)gridDim.x < g.n_units) {
+          // this thread's share of the next unit's node tile and positions, underneath the W2 product; the other
+          // buffer's last readers (the previous unit's gathers and geometry) finished before this group's gather did
+          const NbSelUnit Un = nb_sel_unit<false>(g, uo + gridDim.x, 0);
+          unsigned char* nh = NT + 2 * (b ^ 1) * NB_TC_TILE_BYTES(64);
+          const float xv = tid < Un.nrecv * 3 ? __ldg(a.x + (int64_t)Un.recv0 * 3 + tid) : 0.f;
+          nb_sel_stage_unit(nh, nh + NB_TC_TILE_BYTES(64), a.P, a.Q, Un, tid, NC);
+          if (tid < Un.nrecv * 3) xsb[(b ^ 1) * 96 + tid] = xv;
+          nb_fence_async_smem();
+          nb_mbar_arrive(ntfull + (b ^ 1));
+        }
+        nb_mbar_wait(done + grp, phase);
+        phase ^= 1;
+        nb_tc_fence_after();
+        // ---- m = SiLU(pre2 + b2) -> A operand and the scatter's B operand
+#pragma unroll
+        for (int hf = 0; hf < 2; ++hf) {
+          float v[32];
+          nb_tmem_ld32(tpre + 32 * hf, v);
+#pragma unroll
+          for (int i = 0; i < 32; ++i) v[i] = NB_FWD_SILU(i, v[i] + vb2[32 * hf + i]);
+          nb_store32_ta(Th, Tl, row, hf, v, ta_h + 16 * hf, ta_l + 16 * hf);
+        }
+        nb_tmem_st_wait();
+        nb_fence_async_smem();
+        nb_tc_fence_before();
+        nb_named_sync(1 + grp, 128);
+        if (row == 0) nb_mbar_arrive(ready + grp);
+        nb_mbar_wait(done + grp, phase);
+        phase ^= 1;
+        nb_tc_fence_after();
+        // ---- c = w4 . SiLU(pre3 + b3) + b4 (two 32-term chains, as k_edge_fwd_sel) ; F = rij c -> force tile
+        float cp[2];
+#pragma unroll
+        for (int hf = 0; hf < 2; ++hf) {
+          float v[32];
+          nb_tmem_ld32(tpre + 32 * hf, v);
+          cp[hf] = 0.f;
+#pragma unroll
+          for (int i = 0; i < 32; ++i) cp[hf] = fmaf(vw4[32 * hf + i], NB_FWD_SILU(i, v[i] + vb3[32 * hf + i]), cp[hf]);
+        }
+        {
+          const float c = cp[0] + cp[1] + b4;
+          float fx = dx * c, fy = dy * c, fz = dz * c;  // 0 for padded rows
+          if (g.clamp_edge) {
+            fx = fminf(fmaxf(fx, -100.f), 100.f);
+            fy = fminf(fmaxf(fy, -100.f), 100.f);
+            fz = fminf(fmaxf(fz, -100.f), 100.f);
+          }
+          const uint32_t px = nb_pack_split(fx), py = nb_pack_split(fy), pz = nb_pack_split(fz);
+          *reinterpret_cast<uint4*>(Fh + row * 16) = make_uint4((px & 0xffffu) | (py << 16), pz & 0xffffu, 0u, 0u);
+          *reinterpret_cast<uint4*>(Fl + row * 16) = make_uint4((px >> 16) | (py & 0xffff0000u), pz >> 16, 0u, 0u);
+        }
+        nb_fence_async_smem();
+        nb_tc_fence_before();
+        nb_named_sync(1 + grp, 128);
+        if (row == 0) nb_mbar_arrive(ready + grp);
+        pend = true;
+      }
+      if (grp == (ntl - 1) % NB_F3_GROUPS) {
+        // ---- unit read-out (accumulator row i <-> TMEM lane (i % 16) + 32 (i / 16)); the last F scatter completes
+        // after every other scatter of the unit
+        nb_mbar_wait(done + grp, phase);
+        phase ^= 1;
+        pend = false;
+        nb_tc_fence_after();
+        const int nl = 16 * q + lane;
+#pragma unroll
+        for (int hf = 0; hf < 2; ++hf) {
+          float v[32];
+          nb_tmem_ld32(tm + lq + NB_F3_TM_M + 32 * hf, v);
+          if (lane < 16 && nl < U.nrecv) {
+            float* dst = a.M + (int64_t)(U.recv0 + nl) * NB_H + 32 * hf;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) nb_st4(dst + 4 * j, make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]));
+          }
+        }
+        float f4[4];
+        nb_tmem_ld4(tm + lq + NB_F3_TM_F, f4);
+        if (lane < 16 && nl < U.nrecv) {
+          float* dst = a.Fsum + (int64_t)(U.recv0 + nl) * 3;
+          dst[0] = f4[0];
+          dst[1] = f4[1];
+          dst[2] = f4[2];
+        }
+        nb_tc_fence_before();
+        nb_mbar_arrive(accfree);
+      }
+    }
+    if (pend) {
+      nb_mbar_wait(done + grp, phase);
+      nb_tc_fence_after();
+    }
+  }
+  nb_tc_fence_before();
+  __syncthreads();
+  if (warp == 0) nb_tmem_dealloc(tm, NB_F3_TMEM_COLS);
+}
+
 // ----------------------------------------------------------------------------- backward
 // 512 threads: thread (warp w, lane l) owns row 32 (w & 3) + l and the 16 columns of quarter (w >> 2).
 //   S1  selector row (for the scatters); pre1 = P_i + Q_j + w_rad r2 + W_e e summed in fp32 from shared-memory

@@ -640,6 +640,11 @@ extern "C" int nb_set_edge_impl(int impl) {
   return NB_OK;
 }
 extern "C" int nb_get_edge_impl(void) { return g_edge_impl; }
+// edge impl 2, forward: 1 = whole-graph units of three or more tiles run k_edge_fwd_sel3 (three tiles in flight per SM),
+// 0 = every shape runs k_edge_fwd_sel (the cross-check; both give bitwise equal results)
+static int g_edge_fwd3 = 1;
+extern "C" int nb_set_edge_fwd3(int on) { g_edge_fwd3 = on ? 1 : 0; return NB_OK; }
+extern "C" int nb_get_edge_fwd3(void) { return g_edge_fwd3; }
 
 #ifndef NB_EMU
 // unit geometry of the selector kernels: G graph-instances with G*N <= 27 nodes and (for G > 1) at most 128 rows
@@ -679,6 +684,18 @@ static int launch_edge_fwd(NbEdgeFwdArgs& a, void* st) {
   if (g_edge_impl == 2) {
     // no silent switch to another variant: a shape the selector kernels cannot walk is an error
     if (!sel_geom(a.g)) { nb_set_error("selector edge kernels support at most 255 nodes per graph (N=%d)", a.g.N); return NB_ERR_INVALID; }
+    // one graph-instance of at least three tiles per unit (N = 17 .. 27): every warp group of k_edge_fwd_sel3 has a tile
+    // in every unit.  Smaller units (two tiles at N = 12 .. 16, packed graphs below) and the blocked walk keep the
+    // two-CTA kernel.
+    if (g_edge_fwd3 && !a.g.blk && a.g.G == 1 && a.g.EPG > 2 * NB_TILE) {
+      const size_t smem3 = NB_EDGE_FWD_SEL3_SMEM(a.g.EPG);
+      const int grid3 = imin(a.g.n_units, nb_num_sms());
+      int pi3 = prof_begin(0, st);
+      NB_SET_SMEM(k_edge_fwd_sel3, smem3);
+      NB_LAUNCH_COUNTED(k_edge_fwd_sel3, (unsigned)grid3, NB_F3_THREADS, smem3, st, a);
+      prof_end(0, pi3, st);
+      return nb_check_launch("k_edge_fwd_sel3");
+    }
     const size_t smem_sel = NB_EDGE_FWD_SEL_SMEM(a.g.blk ? 0 : a.g.G * a.g.EPG);
     int grid_sel = imin(a.g.n_units, 2 * nb_num_sms());
     int pi_sel = prof_begin(0, st);
