@@ -126,6 +126,19 @@ int nb_egno_backward(const NbEgnoConfig* cfg, const float* params, const float* 
                      const float* saved, const float* g_x_out, const float* g_v_out, const float* g_h_out,
                      float* grad_params, float* g_x_in, float* g_v_in, float* workspace, void* stream);
 
+/* nb_egno_backward plus the gradients of the other inputs (num_inputs = 1 only; the reference's autograd gives them):
+ *   g_nodes[BN, in_node_nf], g_edge_fea[B*N*(N-1), in_edge_nf], g_loc_mean[BN, 3], each nullable (NULL: not formed).
+ * Every other output is bitwise what nb_egno_backward writes.  g_nodes or g_edge_fea (in_edge_nf > 0) need
+ * `input_grad_workspace` of nb_egno_input_grad_workspace_floats(cfg) floats: the edge-feature gradient of every replicated
+ * edge row of every layer, n_layers * T * B*N(N-1) * in_edge_nf floats, reduced in a fixed order at the end.  With all
+ * three NULL this is nb_egno_backward (same launches, same results). */
+int64_t nb_egno_input_grad_workspace_floats(const NbEgnoConfig* cfg);
+int nb_egno_backward_ex(const NbEgnoConfig* cfg, const float* params, const float* nodes, const float* edge_fea,
+                        const float* loc_mean, const int64_t* timesteps_out, const int64_t* timesteps_in,
+                        const float* saved, const float* g_x_out, const float* g_v_out, const float* g_h_out,
+                        float* grad_params, float* g_x_in, float* g_v_in, float* g_nodes, float* g_edge_fea,
+                        float* g_loc_mean, float* workspace, float* input_grad_workspace, void* stream);
+
 /* Replaces SEGNO.forward_step applied to embedding(his) (SEGNO/models/model.py:73,95-102) with
  * SEGNO_GCL.forward (SEGNO/models/models/gcl.py:111-119), unsorted_segment_sum / _mean (:7-23).
  *   his[BN,in_node_nf] x[BN,3] v[BN,3] edge_attr[B*N*(N-1),in_edge_nf] -> x_out[BN,3] h_out[BN,H] v_out[BN,3] */
@@ -136,6 +149,16 @@ int nb_segno_forward(const NbSegnoConfig* cfg, const float* params, const float*
 int nb_segno_backward(const NbSegnoConfig* cfg, const float* params, const float* his, const float* edge_attr,
                       const float* saved, const float* g_x_out, const float* g_h_out, const float* g_v_out,
                       float* grad_params, float* g_x_in, float* g_v_in, float* g_h_in, float* workspace, void* stream);
+
+/* nb_segno_backward plus g_his[BN, in_node_nf] (h_given = 0 only; with h_given = 1 the input gradient is g_h_in) and
+ * g_edge_attr[B*N*(N-1), in_edge_nf], both nullable.  g_edge_attr (in_edge_nf > 0) needs `input_grad_workspace` of
+ * nb_segno_input_grad_workspace_floats(cfg) floats: one slice of per-row gradients per sub-step, T * B*N(N-1) *
+ * in_edge_nf floats, reduced in a fixed order.  With both NULL this is nb_segno_backward. */
+int64_t nb_segno_input_grad_workspace_floats(const NbSegnoConfig* cfg);
+int nb_segno_backward_ex(const NbSegnoConfig* cfg, const float* params, const float* his, const float* edge_attr,
+                         const float* saved, const float* g_x_out, const float* g_h_out, const float* g_v_out,
+                         float* grad_params, float* g_x_in, float* g_v_in, float* g_h_in, float* g_his,
+                         float* g_edge_attr, float* workspace, float* input_grad_workspace, void* stream);
 
 /* Multi-input SEGNO (SEGNO.forward with x[BN, L, 3], SEGNO/models/model.py:65-90): the reference embeds every observed
  * frame, integrates from frame i to frame i + 1 (forward_step = nb_segno_forward with cfg.h_given = 1) and merges the

@@ -31,6 +31,10 @@ EXPORTS = {
     "nb_egno_backward": (C.c_int, [C.POINTER(NbEgnoConfig)] + [c_f] * 15),
     "nb_segno_forward": (C.c_int, [C.POINTER(NbSegnoConfig)] + [c_f] * 11),
     "nb_segno_backward": (C.c_int, [C.POINTER(NbSegnoConfig)] + [c_f] * 13),
+    "nb_egno_input_grad_workspace_floats": (C.c_int64, [C.POINTER(NbEgnoConfig)]),
+    "nb_egno_backward_ex": (C.c_int, [C.POINTER(NbEgnoConfig)] + [c_f] * 19),
+    "nb_segno_input_grad_workspace_floats": (C.c_int64, [C.POINTER(NbSegnoConfig)]),
+    "nb_segno_backward_ex": (C.c_int, [C.POINTER(NbSegnoConfig)] + [c_f] * 16),
     "nb_segno_embed_forward": (C.c_int, [C.POINTER(NbSegnoConfig), c_f, C.c_int64, c_f, c_f, c_f]),
     "nb_segno_embed_backward_workspace_floats": (C.c_int64, [C.POINTER(NbSegnoConfig), C.c_int64]),
     "nb_segno_embed_backward": (C.c_int, [C.POINTER(NbSegnoConfig), C.c_int64] + [c_f] * 5),

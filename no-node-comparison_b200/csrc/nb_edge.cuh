@@ -277,11 +277,16 @@ struct NbEdgeBwdArgs {
   float* gQ;           // [NGT*N][64]  overwritten
   float* gx;           // [NGT*N][3]   accumulated into
   float* partial;      // [gridDim.x][NB_EB_PLEN]
+  // EGRAD instantiations only: dL/d(edge features) of every replicated edge row, [NGT*EPG][nef], row gt*EPG + e_local
+  // (overwritten, one plain store per row and feature)
+  float* gef;
 };
 
 #define NB_EDGE_BWD_SMEM_FLOATS(GN) \
   (4 * NB_H * NB_H + 4 * NB_H + 3 * NB_TILE * NB_LDA + NB_TILE * (2 + 1 + 3 + NB_MAX_EF + 3 + 3) + (GN) * (NB_H + 3))
 
+// EGRAD: also dL/de = W_e^T g1 per edge row into a.gef (false: the kernel without input gradients, unchanged)
+template <bool EGRAD>
 __global__ void __launch_bounds__(NB_THREADS) k_edge_bwd(NbEdgeBwdArgs a) {
   NB_PDL_ENTER();
   NB_DYN_SMEM(sm);
@@ -473,6 +478,14 @@ __global__ void __launch_bounds__(NB_THREADS) k_edge_bwd(NbEdgeBwdArgs a) {
           rG[row] = fmaf(2.f * ri.rD[row], gr2, rG[row]);
           rG[NB_TILE + row] = fmaf(2.f * ri.rD[NB_TILE + row], gr2, rG[NB_TILE + row]);
           rG[2 * NB_TILE + row] = fmaf(2.f * ri.rD[2 * NB_TILE + row], gr2, rG[2 * NB_TILE + row]);
+        }
+        if constexpr (EGRAD) {  // dL/de_f = w_ef[f] . g1: the unit's rows are the replicated rows gt0*EPG + r
+#pragma unroll
+          for (int f = 0; f < NB_MAX_EF; ++f)
+            if (f < g.nef) {
+              const float ge = nb_reduce_tx(we[f].x * g1[0] + we[f].y * g1[1] + we[f].z * g1[2] + we[f].w * g1[3]);
+              if (tx == 0 && row < nv) a.gef[((int64_t)gt0 * g.EPG + r0 + row) * g.nef + f] = ge;
+            }
         }
         nb_st4(Gs + row * NB_LDA + tx * 4, make_float4(g1[0], g1[1], g1[2], g1[3]));
       }

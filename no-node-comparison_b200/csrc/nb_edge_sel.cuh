@@ -1057,7 +1057,8 @@ __device__ __forceinline__ void nb_issue_scatter_fold(uint32_t tmem_d, uint32_t 
 }
 #define NB_SB_ONES64_BYTES NB_TC_TILE_BYTES(128)  // whole-graph units only: all-ones SW128 tile (second MN block of the fold)
 
-template <bool BLK>
+// EGRAD: S5 also forms dL/de = W_e^T g1 per edge row (a.gef); false is the kernel without input gradients, unchanged
+template <bool BLK, bool EGRAD>
 __global__ void __launch_bounds__(NB_SB_THREADS, 1) k_edge_bwd_sel(NbEdgeBwdArgs a) {
   NB_PDL_ENTER();
 #ifdef NB_STAGE_CLOCKS
@@ -1088,6 +1089,7 @@ __global__ void __launch_bounds__(NB_SB_THREADS, 1) k_edge_bwd_sel(NbEdgeBwdArgs
   float* Pf = reinterpret_cast<float*>(base + NB_SB_NT);  // [receivers][64] fp32: P rows of the unit (P includes b1)
   float* Qf = Pf + (BLK ? a.g.IB : a.g.G * a.g.N) * NB_H; // [senders][NB_SB_QLD] fp32: Q rows; receivers + senders <= 54: 14.7 KB
   float* gMs = reinterpret_cast<float*>(base + NB_SB_GM);  // [32][64] fp32: dL/dM_i of the unit's receivers (added in S4)
+  float* epart = gMs + 32 * NB_H;  // EGRAD only: [NB_MAX_EF][4][128] quarter sums of dL/de, the unused second half of NB_SB_GM
   unsigned char* ones = base + NB_SB_ONES;
   unsigned char* RGh = base + NB_SB_RG;
   unsigned char* RGl = RGh + NB_TILE * 16;
@@ -1470,6 +1472,16 @@ __global__ void __launch_bounds__(NB_SB_THREADS, 1) k_edge_bwd_sel(NbEdgeBwdArgs
           gr2 = fmaf(vwr[cb + i], v[i], gr2);  // dL/dr2 = w_rad . g1
         }
         cpart[cq * NB_TILE + row] = gr2;
+        if constexpr (EGRAD) {  // dL/de_f = w_ef[f] . g1: this quarter's 16 columns
+#pragma unroll
+          for (int f = 0; f < NB_MAX_EF; ++f)
+            if (f < g.nef) {
+              float ge = 0.f;
+#pragma unroll
+              for (int i = 0; i < 16; ++i) ge = fmaf(Wef[f * NB_H + cb + i], v[i], ge);
+              epart[(f * 4 + cq) * NB_TILE + row] = ge;
+            }
+        }
         nb_tc_store8(Tmh, Tml, row, 2 * cq, v);
         nb_tc_store8(Tmh, Tml, row, 2 * cq + 1, v + 8);
       }
@@ -1487,6 +1499,18 @@ __global__ void __launch_bounds__(NB_SB_THREADS, 1) k_edge_bwd_sel(NbEdgeBwdArgs
         } else {
           *reinterpret_cast<uint4*>(RGh + row * 16) = rh;
           *reinterpret_cast<uint4*>(RGl + row * 16) = rl;
+        }
+        if constexpr (EGRAD) {  // the four quarters in a fixed order; one plain store per replicated row and feature
+          int li5 = 0, lj5, gt5 = 0, rem5 = 0;
+          if (nb_sel_row<BLK>(g, U, rowinfo, r0 + row, li5, lj5, gt5, rem5)) {
+            float* dst = a.gef + ((int64_t)gt5 * g.EPG + rem5) * g.nef;
+#pragma unroll
+            for (int f = 0; f < NB_MAX_EF; ++f)
+              if (f < g.nef) {
+                const float* ep = epart + f * 4 * NB_TILE + row;
+                dst[f] = (ep[0] + ep[NB_TILE]) + (ep[2 * NB_TILE] + ep[3 * NB_TILE]);
+              }
+          }
         }
       }
       nb_fence_async_smem();

@@ -469,6 +469,44 @@ __global__ void __launch_bounds__(256) k_sum_over_t(const float* __restrict__ sr
   }
 }
 
+// ----------------------------------------------------------------------------- input gradients (nb_*_backward_ex)
+// dst[i] = sum over the slices s = 0 .. nslices-1, in that order, of src[s * n + i]
+__global__ void __launch_bounds__(256) k_sum_slices(const float* __restrict__ src, float* __restrict__ dst, int64_t n,
+                                                    int nslices) {
+  NB_PDL_ENTER();
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    float s = 0.f;
+    for (int k = 0; k < nslices; ++k) s += src[(int64_t)k * n + i];
+    dst[i] = s;
+  }
+}
+// the embedding's input gradient: out[r][f] = sum_c g[r][c] W[c][f] for the first F0 of the ldw input columns
+__global__ void __launch_bounds__(256) k_embed_input_grad(const float* __restrict__ g, const float* __restrict__ W, int ldw,
+                                                          int F0, int64_t rows, float* __restrict__ out) {
+  NB_PDL_ENTER();
+  const int64_t total = rows * F0;
+  for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = idx / F0;
+    const int f = (int)(idx - r * F0);
+    const float* gr = g + r * NB_H;
+    float s = 0.f;
+#pragma unroll 8
+    for (int c = 0; c < NB_H; ++c) s = fmaf(gr[c], __ldg(W + (int64_t)c * ldw + f), s);
+    out[idx] = s;
+  }
+}
+// EGNO loc_mean: x1 = x0 + conv(x0 - mean) with the mean added back, so one layer contributes
+// dL/dmean = sum_t (dL/dx1[t] - dL/dx0[t]); layers accumulate in the order of the backward sweep
+__global__ void __launch_bounds__(256) k_loc_mean_grad(const float* __restrict__ gx1, const float* __restrict__ gx0,
+                                                       float* __restrict__ g_mean, int n3, int T, int accumulate) {
+  NB_PDL_ENTER();
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n3; i += (int64_t)gridDim.x * blockDim.x) {
+    float s = 0.f;
+    for (int t = 0; t < T; ++t) s += gx1[(int64_t)t * n3 + i] - gx0[(int64_t)t * n3 + i];
+    g_mean[i] = accumulate ? g_mean[i] + s : s;
+  }
+}
+
 // EGNO coordinate update (basic.py:172-178):  s = w2 . SiLU(UV) + b2 ;  x' = x + s v + clamp(Fsum/(N-1), +-100)
 struct NbXupdArgs {
   int64_t rows;

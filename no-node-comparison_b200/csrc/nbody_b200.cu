@@ -782,17 +782,30 @@ static int launch_edge_bwd(NbEdgeBwdArgs& a, float* dst, const EdgeGradDst& d, i
     const size_t smem_sel = NB_EDGE_BWD_SEL_SMEM(a.g.blk ? 0 : a.g.G * a.g.EPG) +
                             (a.g.blk ? NB_EDGE_BWD_SEL_BLK_EXTRA(a.g.N) : NB_SB_ONES64_BYTES);
     int pi_sel = prof_begin(1, st);
-    if (a.g.blk) {
-      NB_SET_SMEM(k_edge_bwd_sel<true>, smem_sel);
-      NB_LAUNCH_COUNTED(k_edge_bwd_sel<true>, (unsigned)grid, NB_SB_THREADS, smem_sel, st, a);
+    if (a.gef) {
+      if (a.g.blk) {
+        NB_SET_SMEM((k_edge_bwd_sel<true, true>), smem_sel);
+        NB_LAUNCH_COUNTED((k_edge_bwd_sel<true, true>), (unsigned)grid, NB_SB_THREADS, smem_sel, st, a);
+      } else {
+        NB_SET_SMEM((k_edge_bwd_sel<false, true>), smem_sel);
+        NB_LAUNCH_COUNTED((k_edge_bwd_sel<false, true>), (unsigned)grid, NB_SB_THREADS, smem_sel, st, a);
+      }
+    } else if (a.g.blk) {
+      NB_SET_SMEM((k_edge_bwd_sel<true, false>), smem_sel);
+      NB_LAUNCH_COUNTED((k_edge_bwd_sel<true, false>), (unsigned)grid, NB_SB_THREADS, smem_sel, st, a);
     } else {
-      NB_SET_SMEM(k_edge_bwd_sel<false>, smem_sel);
-      NB_LAUNCH_COUNTED(k_edge_bwd_sel<false>, (unsigned)grid, NB_SB_THREADS, smem_sel, st, a);
+      NB_SET_SMEM((k_edge_bwd_sel<false, false>), smem_sel);
+      NB_LAUNCH_COUNTED((k_edge_bwd_sel<false, false>), (unsigned)grid, NB_SB_THREADS, smem_sel, st, a);
     }
     prof_end(1, pi_sel, st);
     NB_TRY(nb_check_launch("k_edge_bwd_sel"));
     done = true;
   } else if (g_edge_impl >= 1) {
+    if (a.gef) {
+      nb_set_error("edge-feature gradients need edge impl 2 (selector kernels) or 0 (SIMT); the tcgen05 cross-check "
+                   "kernels of edge impl 1 do not form them");
+      return NB_ERR_INVALID;
+    }
     const size_t smem_tc = NB_EDGE_BWD_TC_SMEM(a.g.G * a.g.N);
     NB_SET_SMEM(k_edge_bwd_tc, smem_tc);
     int pi_tc = prof_begin(1, st);
@@ -804,9 +817,14 @@ static int launch_edge_bwd(NbEdgeBwdArgs& a, float* dst, const EdgeGradDst& d, i
 #endif
   if (!done) {
     const size_t smem = NB_EDGE_BWD_SMEM_FLOATS(a.g.G * a.g.N) * sizeof(float);
-    NB_SET_SMEM(k_edge_bwd, smem);
     int pi = prof_begin(1, st);
-    NB_LAUNCH_COUNTED(k_edge_bwd, (unsigned)grid, NB_THREADS, smem, st, a);
+    if (a.gef) {
+      NB_SET_SMEM(k_edge_bwd<true>, smem);
+      NB_LAUNCH_COUNTED(k_edge_bwd<true>, (unsigned)grid, NB_THREADS, smem, st, a);
+    } else {
+      NB_SET_SMEM(k_edge_bwd<false>, smem);
+      NB_LAUNCH_COUNTED(k_edge_bwd<false>, (unsigned)grid, NB_THREADS, smem, st, a);
+    }
     prof_end(1, pi, st);
     NB_TRY(nb_check_launch("k_edge_bwd"));
   }
@@ -1289,16 +1307,48 @@ extern "C" int nb_egno_forward(const NbEgnoConfig* cfg, const float* params, con
   return nb_check_launch("nb_egno_forward");
 }
 
+// input-gradient workspace of nb_egno_backward_ex: the per-row edge-feature gradients of every layer launch
+// (n_layers * T * B*N(N-1) * in_edge_nf floats: each launch writes its own slice, no read-modify-write across layers),
+// then the embedding-output gradient summed over the T frames
+static inline int64_t egno_edge_rows(const NbEgnoConfig* c) { return (int64_t)c->B * c->N * (c->N - 1); }
+extern "C" int64_t nb_egno_input_grad_workspace_floats(const NbEgnoConfig* cfg) {
+  if (egno_validate(cfg) != NB_OK) return -1;
+  return align64((int64_t)cfg->n_layers * cfg->T * egno_edge_rows(cfg) * cfg->in_edge_nf) +
+         align64((int64_t)cfg->B * cfg->N * NB_H);
+}
+
 extern "C" int nb_egno_backward(const NbEgnoConfig* cfg, const float* params, const float* nodes, const float* edge_fea,
                                 const float* loc_mean, const int64_t* timesteps_out, const int64_t* timesteps_in,
                                 const float* saved, const float* g_x_out, const float* g_v_out, const float* g_h_out,
                                 float* grad_params, float* g_x_in, float* g_v_in, float* workspace, void* stream) {
+  return nb_egno_backward_ex(cfg, params, nodes, edge_fea, loc_mean, timesteps_out, timesteps_in, saved, g_x_out, g_v_out,
+                             g_h_out, grad_params, g_x_in, g_v_in, nullptr, nullptr, nullptr, workspace, nullptr, stream);
+}
+
+extern "C" int nb_egno_backward_ex(const NbEgnoConfig* cfg, const float* params, const float* nodes, const float* edge_fea,
+                                   const float* loc_mean, const int64_t* timesteps_out, const int64_t* timesteps_in,
+                                   const float* saved, const float* g_x_out, const float* g_v_out, const float* g_h_out,
+                                   float* grad_params, float* g_x_in, float* g_v_in, float* g_nodes, float* g_edge_fea,
+                                   float* g_loc_mean, float* workspace, float* input_grad_workspace, void* stream) {
   NB_RANGE("nb_egno_backward");
   EgnoCtx X;
   NB_TRY(egno_ctx_init(&X, cfg, params, stream));
   if (!saved) { nb_set_error("nb_egno_backward needs the saved buffer of a forward call"); return NB_ERR_INVALID; }
   const int T = cfg->T, Ln = cfg->n_layers, modes = cfg->num_modes;
   const int64_t Nn = X.Nn, Nn0 = X.Nn0;
+  // input gradients (single input frame only): per-row edge-feature gradients of every layer, summed at the end
+  const bool want_ef = g_edge_fea && cfg->in_edge_nf > 0;
+  if ((g_nodes || g_edge_fea || g_loc_mean) && egno_L(cfg) > 1) {
+    nb_set_error("gradients w.r.t. nodes / edge_fea / loc_mean are implemented for num_inputs = 1 only");
+    return NB_ERR_INVALID;
+  }
+  if ((g_nodes || want_ef) && !input_grad_workspace) {
+    nb_set_error("nb_egno_backward_ex needs the input-gradient workspace (nb_egno_input_grad_workspace_floats)");
+    return NB_ERR_INVALID;
+  }
+  const int64_t ef_slice = (int64_t)T * egno_edge_rows(cfg) * cfg->in_edge_nf;   // one layer launch
+  float* gef_rows = input_grad_workspace;
+  float* gh_sum = input_grad_workspace ? input_grad_workspace + align64(ef_slice * Ln) : nullptr;
   const int64_t nh = align64(Nn * NB_H), n3 = align64(Nn * 3), cf = egno_coef_floats(cfg);
   const int64_t lf = align64(egno_layer_floats(Nn, Nn0));
   float* w = workspace;
@@ -1462,6 +1512,7 @@ extern "C" int nb_egno_backward(const NbEgnoConfig* cfg, const float* params, co
       egno_geom_frames(cfg, ea.g);
       ea.w = egno_edge_w(X, l);
       ea.x = x1; ea.P = b.P; ea.Q = b.Q; ea.ef = edge_fea; ea.gM = gM; ea.gFsum = gFsum; ea.gP = gP; ea.gQ = gQ; ea.gx = gx;
+      if (want_ef) ea.gef = gef_rows + (int64_t)l * ef_slice;
       EdgeGradDst d;
       d.w1 = L.e_w1; d.W2 = L.e_w2; d.b2 = L.e_b2; d.W3 = L.c_w1; d.b3 = L.c_b1; d.w4 = L.c_w2; d.b4 = L.c_b2;
       d.ldw1 = X.lo.E; d.col_rad = 0; d.col_ef = 1 + 2 * NB_H; d.b_unused = 0;
@@ -1519,6 +1570,11 @@ extern "C" int nb_egno_backward(const NbEgnoConfig* cfg, const float* params, co
         t.partial = partial;
         NB_LAUNCH_COUNTED(k_tcx_bwd, (unsigned)grid, 256, 0, side, t);
         NB_TRY(nb_check_launch("k_tcx_bwd"));
+        if (g_loc_mean) {   // same stream, right behind k_tcx_bwd: both planes are final there
+          NB_LAUNCH_COUNTED(k_loc_mean_grad, (unsigned)ew_grid(Nn0 * 3), 256, 0, side, (const float*)gx, (const float*)gx0,
+                            g_loc_mean, (int)(Nn0 * 3), T, l == Ln - 1 ? 0 : 1);
+          NB_TRY(nb_check_launch("k_loc_mean_grad"));
+        }
         NbFinArgs f;
         memset(&f, 0, sizeof(f));
         int nw = 2 * 2 * modes * 2;
@@ -1637,6 +1693,15 @@ extern "C" int nb_egno_backward(const NbEgnoConfig* cfg, const float* params, co
   const NbFrameMap fm = egno_frame_map(cfg);
   if (g_x_in) NB_LAUNCH_COUNTED(k_sum_over_t, (unsigned)ew_grid(Nn0 * 3 * fm.L), 256, 0, stream, (const float*)gxb[gxi], g_x_in, (int)(Nn0 * 3), T, fm);
   if (g_v_in) NB_LAUNCH_COUNTED(k_sum_over_t, (unsigned)ew_grid(Nn0 * 3 * fm.L), 256, 0, stream, gv_in, g_v_in, (int)(Nn0 * 3), T, fm);
+  if (g_nodes) {   // dL/dnodes = (sum_t dL/dh_emb[t]) W_emb[:, :in_node_nf]
+    NB_LAUNCH_COUNTED(k_sum_over_t, (unsigned)ew_grid(Nn0 * NB_H), 256, 0, stream, gh_in, gh_sum, (int)(Nn0 * NB_H), T, fm);
+    NB_LAUNCH_COUNTED(k_embed_input_grad, (unsigned)ew_grid(Nn0 * cfg->in_node_nf), 256, 0, stream, (const float*)gh_sum,
+                      params + X.lo.emb_w, X.lo.F, cfg->in_node_nf, Nn0, g_nodes);
+  }
+  if (want_ef)     // fixed-order sum over the n_layers * T slices of B*N(N-1) rows
+    NB_LAUNCH_COUNTED(k_sum_slices, (unsigned)ew_grid(egno_edge_rows(cfg) * cfg->in_edge_nf), 256, 0, stream,
+                      (const float*)gef_rows, g_edge_fea, egno_edge_rows(cfg) * cfg->in_edge_nf, Ln * T);
+  if (g_loc_mean && !cfg->use_time_conv) cudaMemsetAsync(g_loc_mean, 0, Nn0 * 3 * sizeof(float), cst);
   defer_join(D, stream);
   return nb_check_launch("nb_egno_backward");
 }
@@ -1863,13 +1928,39 @@ extern "C" int nb_segno_forward(const NbSegnoConfig* cfg, const float* params, c
   return nb_check_launch("nb_segno_forward");
 }
 
+// input-gradient workspace of nb_segno_backward_ex: the per-row edge-attribute gradients of every sub-step launch
+// (T * B*N(N-1) * in_edge_nf floats), summed in a fixed order at the end
+extern "C" int64_t nb_segno_input_grad_workspace_floats(const NbSegnoConfig* cfg) {
+  if (segno_validate(cfg) != NB_OK) return -1;
+  return align64((int64_t)cfg->T * cfg->B * cfg->N * (cfg->N - 1) * cfg->in_edge_nf);
+}
+
 extern "C" int nb_segno_backward(const NbSegnoConfig* cfg, const float* params, const float* his,
                                  const float* edge_attr, const float* saved, const float* g_x_out,
                                  const float* g_h_out, const float* g_v_out, float* grad_params, float* g_x_in,
                                  float* g_v_in, float* g_h_in, float* workspace, void* stream) {
+  return nb_segno_backward_ex(cfg, params, his, edge_attr, saved, g_x_out, g_h_out, g_v_out, grad_params, g_x_in, g_v_in,
+                              g_h_in, nullptr, nullptr, workspace, nullptr, stream);
+}
+
+extern "C" int nb_segno_backward_ex(const NbSegnoConfig* cfg, const float* params, const float* his,
+                                    const float* edge_attr, const float* saved, const float* g_x_out,
+                                    const float* g_h_out, const float* g_v_out, float* grad_params, float* g_x_in,
+                                    float* g_v_in, float* g_h_in, float* g_his, float* g_edge_attr, float* workspace,
+                                    float* input_grad_workspace, void* stream) {
   NB_RANGE("nb_segno_backward");
   NB_TRY(segno_validate(cfg));
   if (!saved) { nb_set_error("nb_segno_backward needs the saved buffer of a forward call"); return NB_ERR_INVALID; }
+  if (g_his && cfg->h_given) {
+    nb_set_error("g_his is the gradient of the raw node features: with h_given = 1 the hidden state's gradient is g_h_in");
+    return NB_ERR_INVALID;
+  }
+  const bool want_ef = g_edge_attr && cfg->in_edge_nf > 0;
+  if (want_ef && !input_grad_workspace) {
+    nb_set_error("nb_segno_backward_ex needs the input-gradient workspace (nb_segno_input_grad_workspace_floats)");
+    return NB_ERR_INVALID;
+  }
+  const int64_t ef_slice = (int64_t)cfg->B * cfg->N * (cfg->N - 1) * cfg->in_edge_nf;   // one sub-step launch
   SegnoCtx X;
   X.c = cfg; segno_layout(cfg, &X.lo); X.Nn = (int64_t)cfg->B * cfg->N; X.params = params; X.st = stream;
   const SegnoLayout& lo = X.lo;
@@ -2024,6 +2115,7 @@ extern "C" int nb_segno_backward(const NbSegnoConfig* cfg, const float* params, 
     ea.g = edge_geom(cfg->B, cfg->B, cfg->N, cfg->in_edge_nf, 1);
     ea.w = segno_edge_w(X);
     ea.x = b.x; ea.P = P_all + (int64_t)k * nh; ea.Q = Q_all + (int64_t)k * nh; ea.ef = edge_attr; ea.gM = gM; ea.gFsum = gFsum; ea.gP = gP; ea.gQ = gQ; ea.gx = gx;
+    if (want_ef) ea.gef = input_grad_workspace + (int64_t)k * ef_slice;
     NB_TRY(launch_edge_bwd(ea, grad_params, ed, 1, stream, &run_base, &run_parts));
 #ifndef NB_EMU
     if (defer && k > 0 && k_hi - k >= DEFER_CHUNK) {   // sub-steps [k, k_hi): every operand is final once this launch is done
@@ -2106,7 +2198,13 @@ extern "C" int nb_segno_backward(const NbSegnoConfig* cfg, const float* params, 
     f.seg[1] = fseg(NB_H * F, NB_H, NB_H, lo.emb_b, 0, 1);
     NB_TRY(launch_finalize(f, stream));
     NB_TRY(q_flush(stream));
+    if (g_his)   // dL/dhis = dL/dh_emb W_emb
+      NB_LAUNCH_COUNTED(k_embed_input_grad, (unsigned)ew_grid(Nn * F), 256, 0, stream, gh_in, params + lo.emb_w, F, F, Nn,
+                        g_his);
   }
+  if (want_ef)     // fixed-order sum over the T sub-step slices
+    NB_LAUNCH_COUNTED(k_sum_slices, (unsigned)ew_grid(ef_slice), 256, 0, stream, (const float*)input_grad_workspace,
+                      g_edge_attr, ef_slice, T);
   if (g_x_in) cudaMemcpyAsync(g_x_in, gx, Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, cst);
   if (g_v_in) {
     if (gv_in) cudaMemcpyAsync(g_v_in, gv_in, Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, cst);

@@ -165,9 +165,12 @@ class EGNO(nn.Module):
         N = n0 // B
         if self.use_time_conv and self.num_modes > T // 2 + 1:
             raise ValueError(f"num_modes={self.num_modes} exceeds T//2+1 for T={T} (the reference shape-errors too)")
-        for name, t in (("h", h), ("edge_fea", edge_fea)):
-            if t.requires_grad:
-                raise ValueError(f"gradients w.r.t. {name} are not implemented (the reference callers detach it)")
+        if L > 1:   # one input frame: the backward also returns dL/dh, dL/dedge_fea and dL/dloc_mean
+            for name, t in (("h", h), ("edge_fea", edge_fea)):
+                if t.requires_grad:
+                    raise ValueError(f"gradients w.r.t. {name} are not implemented (the reference callers detach it)")
+            if loc_mean.requires_grad:
+                raise ValueError("gradients w.r.t. loc_mean are not implemented for num_inputs > 1")
         x = _require_cuda_f32("x", x, lead + (n0, 3))
         v = _require_cuda_f32("v", v, lead + (n0, 3))
         h = _require_cuda_f32("h", h, lead + (n0, self.in_node_nf))

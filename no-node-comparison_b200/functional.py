@@ -137,6 +137,13 @@ def dp_param(t: torch.Tensor, dp):
     return t if dp is None else _AllReduceGrad.apply(dp, t)
 
 
+def _require_edge_grad_impl(lib) -> None:
+    """The edge-feature gradient is formed inside the selector (impl 2) and SIMT (impl 0) edge backward kernels only."""
+    if lib.nb_get_edge_impl() == 1:
+        raise RuntimeError("gradients w.r.t. edge features are not formed by the nb_set_edge_impl(1) cross-check kernels "
+                           "(k_edge_bwd_tc); use edge impl 2 (default) or 0")
+
+
 class EgnoFunction(torch.autograd.Function):
     """x, v, h = EGNO.forward(...)   (reference: EGNO/model/egno.py:37-111)."""
 
@@ -178,17 +185,33 @@ class EgnoFunction(torch.autograd.Function):
         gx_in = torch.empty(in_shape, device=dev, dtype=torch.float32)
         gv_in = torch.empty(in_shape, device=dev, dtype=torch.float32)
         ws = torch.empty(lib.nb_egno_workspace_floats(ctypes.byref(cfg), 1), device=dev, dtype=torch.float32)
-        check(lib.nb_egno_backward(ctypes.byref(cfg), _ptr(flat), _ptr(nodes), _ptr(edge_fea), _ptr(loc_mean),
-                                   _ptr(tsteps), _ptr(tsteps_in), _ptr(saved), _ptr(gx_out), _ptr(gv_out), _ptr(gh_out),
-                                   _ptr(grad_flat), _ptr(gx_in), _ptr(gv_in), _ptr(ws), _stream_ptr(dev)),
-              "nb_egno_backward")
+        want_nodes, want_ef, want_lm = ctx.needs_input_grad[4], ctx.needs_input_grad[5], ctx.needs_input_grad[7]
+        g_nodes = g_ef = g_lm = None
+        if want_nodes or want_ef or want_lm:
+            # per-shard input gradients: under data parallelism nothing beyond the parameter bucket is reduced
+            if want_ef:
+                _require_edge_grad_impl(lib)
+            g_nodes = torch.empty_like(nodes) if want_nodes else None
+            g_ef = torch.empty_like(edge_fea) if want_ef else None
+            g_lm = torch.empty_like(loc_mean) if want_lm else None
+            iws = torch.empty(lib.nb_egno_input_grad_workspace_floats(ctypes.byref(cfg)), device=dev, dtype=torch.float32)
+            check(lib.nb_egno_backward_ex(ctypes.byref(cfg), _ptr(flat), _ptr(nodes), _ptr(edge_fea), _ptr(loc_mean),
+                                          _ptr(tsteps), _ptr(tsteps_in), _ptr(saved), _ptr(gx_out), _ptr(gv_out),
+                                          _ptr(gh_out), _ptr(grad_flat), _ptr(gx_in), _ptr(gv_in), _ptr(g_nodes),
+                                          _ptr(g_ef), _ptr(g_lm), _ptr(ws), _ptr(iws), _stream_ptr(dev)),
+                  "nb_egno_backward_ex")
+        else:
+            check(lib.nb_egno_backward(ctypes.byref(cfg), _ptr(flat), _ptr(nodes), _ptr(edge_fea), _ptr(loc_mean),
+                                       _ptr(tsteps), _ptr(tsteps_in), _ptr(saved), _ptr(gx_out), _ptr(gv_out), _ptr(gh_out),
+                                       _ptr(grad_flat), _ptr(gx_in), _ptr(gv_in), _ptr(ws), _stream_ptr(dev)),
+                  "nb_egno_backward")
         _maybe_allreduce(grad_flat, ctx.dp_group)
         grads, o = [], 0
         for shp in ctx.param_shapes:
             n = shp.numel()
             grads.append(grad_flat[o:o + n].view(shp))
             o += n
-        return (None, None, None, gx_in, None, None, gv_in, None, None, None, *grads)
+        return (None, None, None, gx_in, g_nodes, g_ef, gv_in, g_lm, None, None, *grads)
 
 
 class SegnoFunction(torch.autograd.Function):
@@ -232,9 +255,25 @@ class SegnoFunction(torch.autograd.Function):
         gv_in = torch.empty((Nn, 3), device=dev, dtype=torch.float32)
         ws = torch.empty(lib.nb_segno_workspace_floats(ctypes.byref(cfg), 1), device=dev, dtype=torch.float32)
         gh_in = torch.empty((Nn, 64), device=dev, dtype=torch.float32) if cfg.h_given else None
-        check(lib.nb_segno_backward(ctypes.byref(cfg), _ptr(flat), _ptr(his), _ptr(edge_attr), _ptr(saved),
-                                    _ptr(gx_out), _ptr(gh_out), _ptr(gv_out), _ptr(grad_flat), _ptr(gx_in),
-                                    _ptr(gv_in), _ptr(gh_in), _ptr(ws), _stream_ptr(dev)), "nb_segno_backward")
+        want_his = ctx.needs_input_grad[3] and not cfg.h_given
+        want_ef = ctx.needs_input_grad[6]
+        g_his = g_ea = None
+        if want_his or want_ef:
+            if want_ef:
+                _require_edge_grad_impl(lib)
+            g_his = torch.empty_like(his) if want_his else None
+            g_ea = torch.empty_like(edge_attr) if want_ef else None
+            iws = torch.empty(lib.nb_segno_input_grad_workspace_floats(ctypes.byref(cfg)), device=dev, dtype=torch.float32)
+            check(lib.nb_segno_backward_ex(ctypes.byref(cfg), _ptr(flat), _ptr(his), _ptr(edge_attr), _ptr(saved),
+                                           _ptr(gx_out), _ptr(gh_out), _ptr(gv_out), _ptr(grad_flat), _ptr(gx_in),
+                                           _ptr(gv_in), _ptr(gh_in), _ptr(g_his), _ptr(g_ea), _ptr(ws), _ptr(iws),
+                                           _stream_ptr(dev)), "nb_segno_backward_ex")
+            if want_his:
+                gh_in = g_his
+        else:
+            check(lib.nb_segno_backward(ctypes.byref(cfg), _ptr(flat), _ptr(his), _ptr(edge_attr), _ptr(saved),
+                                        _ptr(gx_out), _ptr(gh_out), _ptr(gv_out), _ptr(grad_flat), _ptr(gx_in),
+                                        _ptr(gv_in), _ptr(gh_in), _ptr(ws), _stream_ptr(dev)), "nb_segno_backward")
         _maybe_allreduce(grad_flat, ctx.dp_group)
         grads, o = [], 0
         for shp in ctx.param_shapes:
@@ -246,7 +285,7 @@ class SegnoFunction(torch.autograd.Function):
         grads[-4:] = [None] * 4
         if cfg.h_given:   # a segment of the multi-input forward: `his` is the hidden state, the embedding is outside
             grads[0] = grads[1] = None
-        return (None, None, None, gh_in, gx_in, gv_in, None, *grads)
+        return (None, None, None, gh_in, gx_in, gv_in, g_ea, *grads)
 
 
 class SegnoMultiFunction(torch.autograd.Function):

@@ -165,8 +165,6 @@ class SEGNO(nn.Module):
                                         *params, *attn_params)
 
     def _segment(self, his, x, edges, v, edge_attr, T, h_given):
-        if edge_attr.requires_grad or (his.requires_grad and not h_given):
-            raise ValueError("gradients w.r.t. his / edge_attr are not implemented (the reference callers detach them)")
         T = int(T)
         n0 = x.shape[0]
         dev = x.device
@@ -199,5 +197,5 @@ class SEGNO(nn.Module):
 
     def forward_step(self, h, x, edges, v, edge_attr, T=10):
         """model.py:95-102: T weight-shared SEGNO_GCL sub-steps from an already embedded hidden state `h` [BN, 64];
-        returns (x, h, v).  Differentiable w.r.t. h, x and v (dL/dh is handed back by the C call)."""
+        returns (x, h, v).  Differentiable w.r.t. h, x, v and edge_attr (the C call hands back dL/dh and dL/dedge_attr)."""
         return self._segment(h, x, edges, v, edge_attr, int(T), h_given=True)
