@@ -139,6 +139,26 @@ int nb_egno_backward_ex(const NbEgnoConfig* cfg, const float* params, const floa
                         float* grad_params, float* g_x_in, float* g_v_in, float* g_nodes, float* g_edge_fea,
                         float* g_loc_mean, float* workspace, float* input_grad_workspace, void* stream);
 
+/* The same forward and backward with floating-point times: timesteps_out[B,T] and (num_inputs > 1) timesteps_in[B,L] are
+ * fp32, the reference's `timesteps.float()`, and may be non-integral.  Integral values give the int64 entry points'
+ * results bit for bit.  The workspaces, the saved buffer and the other arguments are those of nb_egno_forward /
+ * nb_egno_backward_ex, including the num_inputs = 1 restriction on g_nodes / g_edge_fea / g_loc_mean.  The backward adds
+ * the time gradients, each nullable and allowed for every num_inputs:
+ *   g_t_out[B,T] = dL/dtimesteps_out, g_t_in[B,L] = dL/dtimesteps_in (num_inputs > 1 only; NULL otherwise)
+ * through the sinusoidal embeddings, from the embedding-output gradient the backward forms anyway.  They need no
+ * workspace; with time_emb_dim = 0 the times are unused and g_t_out is zero.  With both NULL the backward launches what
+ * nb_egno_backward_ex launches (with k_time_table_f for k_time_table). */
+int nb_egno_forward_ft(const NbEgnoConfig* cfg, const float* params, const float* x, const float* nodes,
+                       const float* edge_fea, const float* v, const float* loc_mean, const float* timesteps_out,
+                       const float* timesteps_in, float* x_out, float* v_out, float* h_out, float* saved,
+                       float* workspace, void* stream);
+int nb_egno_backward_ft(const NbEgnoConfig* cfg, const float* params, const float* nodes, const float* edge_fea,
+                        const float* loc_mean, const float* timesteps_out, const float* timesteps_in,
+                        const float* saved, const float* g_x_out, const float* g_v_out, const float* g_h_out,
+                        float* grad_params, float* g_x_in, float* g_v_in, float* g_nodes, float* g_edge_fea,
+                        float* g_loc_mean, float* g_t_out, float* g_t_in, float* workspace,
+                        float* input_grad_workspace, void* stream);
+
 /* Replaces SEGNO.forward_step applied to embedding(his) (SEGNO/models/model.py:73,95-102) with
  * SEGNO_GCL.forward (SEGNO/models/models/gcl.py:111-119), unsorted_segment_sum / _mean (:7-23).
  *   his[BN,in_node_nf] x[BN,3] v[BN,3] edge_attr[B*N*(N-1),in_edge_nf] -> x_out[BN,3] h_out[BN,H] v_out[BN,3] */

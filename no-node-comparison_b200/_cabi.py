@@ -33,6 +33,8 @@ EXPORTS = {
     "nb_segno_backward": (C.c_int, [C.POINTER(NbSegnoConfig)] + [c_f] * 13),
     "nb_egno_input_grad_workspace_floats": (C.c_int64, [C.POINTER(NbEgnoConfig)]),
     "nb_egno_backward_ex": (C.c_int, [C.POINTER(NbEgnoConfig)] + [c_f] * 19),
+    "nb_egno_forward_ft": (C.c_int, [C.POINTER(NbEgnoConfig)] + [c_f] * 14),
+    "nb_egno_backward_ft": (C.c_int, [C.POINTER(NbEgnoConfig)] + [c_f] * 21),
     "nb_segno_input_grad_workspace_floats": (C.c_int64, [C.POINTER(NbSegnoConfig)]),
     "nb_segno_backward_ex": (C.c_int, [C.POINTER(NbSegnoConfig)] + [c_f] * 16),
     "nb_segno_embed_forward": (C.c_int, [C.POINTER(NbSegnoConfig), c_f, C.c_int64, c_f, c_f, c_f]),

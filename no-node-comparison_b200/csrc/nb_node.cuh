@@ -315,16 +315,101 @@ struct NbEmbedArgs {
 };
 
 // table[t][b][j] = sin(ts * freq[j]) (j < D/2) | cos(ts * freq[j - D/2]),  ts = timesteps[b][t]   (layer_no.py:8-17)
+__device__ __forceinline__ float nb_time_emb(const NbEmbedArgs& a, int j, float ts) {
+  const int half = a.D >> 1;
+  const float arg = ts * a.freq[j < half ? j : j - half];
+  return j < half ? sinf(arg) : cosf(arg);
+}
 __global__ void __launch_bounds__(256) k_time_table(NbEmbedArgs a, int input_times) {
   NB_PDL_ENTER();
-  const int total = a.T * a.B * a.D, half = a.D >> 1;
+  const int total = a.T * a.B * a.D;
   float* tab = input_times ? a.table_in : a.table;
   for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += gridDim.x * blockDim.x) {
     const int j = idx % a.D, tb = idx / a.D, b = tb % a.B, t = tb / a.B;
     const float ts = input_times ? (float)__ldg(a.tsteps_in + (int64_t)b * a.L + a.tmap[t])
                                  : (float)__ldg(a.tsteps + (int64_t)b * a.T + t);
-    const float arg = ts * a.freq[j < half ? j : j - half];
-    tab[idx] = j < half ? sinf(arg) : cosf(arg);
+    tab[idx] = nb_time_emb(a, j, ts);
+  }
+}
+// the same table from fp32 times (`timesteps.float()` of a floating-point tensor): integral values give the int64
+// kernel's table bit for bit, since (float)int64 is exact below 2^24
+__global__ void __launch_bounds__(256) k_time_table_f(NbEmbedArgs a, const float* __restrict__ ts_out,
+                                                      const float* __restrict__ ts_in, int input_times) {
+  NB_PDL_ENTER();
+  const int total = a.T * a.B * a.D;
+  float* tab = input_times ? a.table_in : a.table;
+  for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += gridDim.x * blockDim.x) {
+    const int j = idx % a.D, tb = idx / a.D, b = tb % a.B, t = tb / a.B;
+    const float ts = input_times ? __ldg(ts_in + (int64_t)b * a.L + a.tmap[t]) : __ldg(ts_out + (int64_t)b * a.T + t);
+    tab[idx] = nb_time_emb(a, j, ts);
+  }
+}
+
+// dL/dtimes through the sinusoidal embeddings, from G = dL/d(embedding output) [T][Nn0][64] and W = W_emb [64][ldw]:
+//   gt_out[b][t] = sum_j (Gs[t][b] . W[:, c_out + j]) demb_j/dt,   Gs[t][b] = sum over the nodes k = b mod B of G[t][k]
+// (the `k mod B` broadcast of egno.py:66,69), with d sin(t f)/dt = f cos(t f) and d cos(t f)/dt = -f sin(t f);
+// c_out = F0 for one input frame, F0 + D for several, whose input-time columns c_in = F0 give gt_in[b][l] as the same
+// sum over the frames t with tmap[t] = l.  One CTA per trajectory b; every sum runs in a fixed order (no atomics).
+// gt_out and gt_in are nullable.
+constexpr int NB_TGRAD_THREADS = 256;
+__global__ void __launch_bounds__(NB_TGRAD_THREADS) k_time_grad(NbEmbedArgs a, const float* __restrict__ ts_out,
+                                                                const float* __restrict__ ts_in,
+                                                                const float* __restrict__ G, const float* __restrict__ W,
+                                                                int ldw, float* __restrict__ gt_out,
+                                                                float* __restrict__ gt_in) {
+  NB_PDL_ENTER();
+  __shared__ float gs[NB_MAX_T * NB_H];   // Gs[t][:] of this trajectory
+  __shared__ float q[NB_MAX_T * 128];     // [t][in-time columns | out-time columns] terms of the sums over j
+  __shared__ float pin[NB_MAX_T];         // per-frame input-time sums
+  const int b = blockIdx.x, tid = threadIdx.x, D = a.D, T = a.T, N = a.Nn0 / a.B;
+  const bool multi = a.L > 1;
+  const int ncol = multi ? 2 * D : D, c0 = a.F0;
+  for (int i = tid; i < T * NB_H; i += NB_TGRAD_THREADS) {
+    const int t = i / NB_H, c = i % NB_H;
+    const float* g = G + ((int64_t)t * a.Nn0 + b) * NB_H + c;
+    float s = 0.f;
+    for (int n = 0; n < N; ++n) s += __ldg(g + (int64_t)n * a.B * NB_H);
+    gs[i] = s;
+  }
+  __syncthreads();
+  for (int i = tid; i < T * ncol; i += NB_TGRAD_THREADS) {
+    const int t = i / ncol, j = i % ncol;
+    const float* gt = gs + t * NB_H;
+    float p = 0.f;
+#pragma unroll 8
+    for (int c = 0; c < NB_H; ++c) p = fmaf(gt[c], __ldg(W + (int64_t)c * ldw + c0 + j), p);
+    const bool in = multi && j < D;
+    const int jj = multi && !in ? j - D : j, half = D >> 1;
+    const float ts = in ? __ldg(ts_in + (int64_t)b * a.L + a.tmap[t]) : __ldg(ts_out + (int64_t)b * T + t);
+    const float f = a.freq[jj < half ? jj : jj - half], arg = ts * f;
+    q[t * 128 + j] = p * (jj < half ? f * cosf(arg) : -f * sinf(arg));
+  }
+  __syncthreads();
+  const int warp = tid >> 5, lane = tid & 31;
+  for (int t = warp; t < T; t += NB_TGRAD_THREADS / 32) {
+    const float* qt = q + t * 128;
+    float so = 0.f, si = 0.f;
+    for (int j = lane; j < D; j += 32) {
+      so += qt[(multi ? D : 0) + j];
+      if (multi) si += qt[j];
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      so += __shfl_xor_sync(0xffffffffu, so, o);
+      si += __shfl_xor_sync(0xffffffffu, si, o);
+    }
+    if (lane == 0) {
+      if (gt_out) gt_out[(int64_t)b * T + t] = so;
+      pin[t] = si;
+    }
+  }
+  if (!multi || !gt_in) return;
+  __syncthreads();
+  if (tid < a.L) {
+    float s = 0.f;
+    for (int t = 0; t < T; ++t)
+      if (a.tmap[t] == tid) s += pin[t];
+    gt_in[(int64_t)b * a.L + tid] = s;
   }
 }
 

@@ -967,16 +967,21 @@ static void egno_geom_frames(const NbEgnoConfig* c, NbEdgeGeom& g) {
 }
 // embedding inputs (egno.py:50,59-76): fills the kernel arguments, builds the time table(s), materialises the input
 // rows 64 wide into ein0 (features 0..63) and ein1 (features 64.., only when F > 64)
+// the time inputs of an EGNO call: int64 frame indices (nb_egno_forward, nb_egno_backward[_ex]) or fp32 times
+// (nb_egno_forward_ft, nb_egno_backward_ft); exactly one of the two pairs is set
+struct EgnoTimes {
+  const int64_t *out, *in;
+  const float *fout, *fin;
+};
 static int egno_embed_inputs(const NbEgnoConfig* cfg, const EgnoLayout& lo, NbEmbedArgs& e, const float* nodes,
-                             const int64_t* ts_out, const int64_t* ts_in, float* table, float* ein0, float* ein1,
-                             void* stream) {
+                             const EgnoTimes& ts, float* table, float* ein0, float* ein1, void* stream) {
   memset(&e, 0, sizeof(e));
   e.T = cfg->T; e.Nn0 = cfg->B * cfg->N; e.B = cfg->B; e.F0 = cfg->in_node_nf; e.D = cfg->time_emb_dim;
-  e.nodes = nodes; e.tsteps = ts_out; e.tsteps_in = ts_in;
+  e.nodes = nodes; e.tsteps = ts.out; e.tsteps_in = ts.in;
   const NbFrameMap fm = egno_frame_map(cfg);
   e.L = fm.L;
   for (int t = 0; t < NB_MAX_T; ++t) e.tmap[t] = fm.m[t];
-  if (fm.L > 1 && !ts_in) { nb_set_error("num_inputs > 1 needs timesteps_in"); return NB_ERR_INVALID; }
+  if (fm.L > 1 && (ts.fout ? !ts.fin : !ts.in)) { nb_set_error("num_inputs > 1 needs timesteps_in"); return NB_ERR_INVALID; }
   const int half = e.D / 2;
   for (int k = 0; k < half; ++k) {
     float sc = (float)(log(10000.0) / (double)(half - 1));  // layer_no.py:10-11 (fp32 arange * python scalar)
@@ -987,8 +992,13 @@ static int egno_embed_inputs(const NbEgnoConfig* cfg, const EgnoLayout& lo, NbEm
   const int64_t Nn = (int64_t)e.T * e.Nn0;
   if (e.D > 0) {
     const unsigned tg = (unsigned)imin(cdiv((int64_t)e.T * e.B * e.D, 256), 4 * nb_num_sms());
-    NB_LAUNCH_COUNTED(k_time_table, tg, 256, 0, stream, e, 0);
-    if (fm.L > 1) NB_LAUNCH_COUNTED(k_time_table, tg, 256, 0, stream, e, 1);
+    if (ts.fout) {
+      NB_LAUNCH_COUNTED(k_time_table_f, tg, 256, 0, stream, e, ts.fout, ts.fin, 0);
+      if (fm.L > 1) NB_LAUNCH_COUNTED(k_time_table_f, tg, 256, 0, stream, e, ts.fout, ts.fin, 1);
+    } else {
+      NB_LAUNCH_COUNTED(k_time_table, tg, 256, 0, stream, e, 0);
+      if (fm.L > 1) NB_LAUNCH_COUNTED(k_time_table, tg, 256, 0, stream, e, 1);
+    }
     NB_TRY(nb_check_launch("k_time_table"));
   }
   NB_LAUNCH_COUNTED(k_embed_inputs, (unsigned)ew_grid(Nn * 16), 256, 0, stream, e, ein0, 0);
@@ -1157,10 +1167,9 @@ static NbEdgeW egno_edge_w(const EgnoCtx& X, int l) {
   return w;
 }
 
-extern "C" int nb_egno_forward(const NbEgnoConfig* cfg, const float* params, const float* x, const float* nodes,
-                               const float* edge_fea, const float* v, const float* loc_mean,
-                               const int64_t* timesteps_out, const int64_t* timesteps_in, float* x_out, float* v_out,
-                               float* h_out, float* saved, float* workspace, void* stream) {
+static int egno_forward(const NbEgnoConfig* cfg, const float* params, const float* x, const float* nodes,
+                        const float* edge_fea, const float* v, const float* loc_mean, const EgnoTimes& times,
+                        float* x_out, float* v_out, float* h_out, float* saved, float* workspace, void* stream) {
   NB_RANGE("nb_egno_forward");
   EgnoCtx X;
   NB_TRY(egno_ctx_init(&X, cfg, params, stream));
@@ -1182,7 +1191,7 @@ extern "C" int nb_egno_forward(const NbEgnoConfig* cfg, const float* params, con
   {
     // h = Linear([nodes | time embeddings]) (egno.py:72-76): inputs materialised 64 wide (scratch: P, Q), then one GEMM
     NbEmbedArgs e;
-    NB_TRY(egno_embed_inputs(cfg, X.lo, e, nodes, timesteps_out, timesteps_in, ttab, P, Q, stream));
+    NB_TRY(egno_embed_inputs(cfg, X.lo, e, nodes, times, ttab, P, Q, stream));
     {
       NbGemmArgs ga = gemm_args((int)Nn);
       ga.nsrc = 1; ga.src[0] = gsrc(P, NB_H, 0, params + X.lo.emb_w, 1, X.lo.F);
@@ -1307,6 +1316,22 @@ extern "C" int nb_egno_forward(const NbEgnoConfig* cfg, const float* params, con
   return nb_check_launch("nb_egno_forward");
 }
 
+extern "C" int nb_egno_forward(const NbEgnoConfig* cfg, const float* params, const float* x, const float* nodes,
+                               const float* edge_fea, const float* v, const float* loc_mean,
+                               const int64_t* timesteps_out, const int64_t* timesteps_in, float* x_out, float* v_out,
+                               float* h_out, float* saved, float* workspace, void* stream) {
+  const EgnoTimes times = {timesteps_out, timesteps_in, nullptr, nullptr};
+  return egno_forward(cfg, params, x, nodes, edge_fea, v, loc_mean, times, x_out, v_out, h_out, saved, workspace, stream);
+}
+
+extern "C" int nb_egno_forward_ft(const NbEgnoConfig* cfg, const float* params, const float* x, const float* nodes,
+                                  const float* edge_fea, const float* v, const float* loc_mean, const float* timesteps_out,
+                                  const float* timesteps_in, float* x_out, float* v_out, float* h_out, float* saved,
+                                  float* workspace, void* stream) {
+  const EgnoTimes times = {nullptr, nullptr, timesteps_out, timesteps_in};
+  return egno_forward(cfg, params, x, nodes, edge_fea, v, loc_mean, times, x_out, v_out, h_out, saved, workspace, stream);
+}
+
 // input-gradient workspace of nb_egno_backward_ex: the per-row edge-feature gradients of every layer launch
 // (n_layers * T * B*N(N-1) * in_edge_nf floats: each launch writes its own slice, no read-modify-write across layers),
 // then the embedding-output gradient summed over the T frames
@@ -1316,6 +1341,12 @@ extern "C" int64_t nb_egno_input_grad_workspace_floats(const NbEgnoConfig* cfg) 
   return align64((int64_t)cfg->n_layers * cfg->T * egno_edge_rows(cfg) * cfg->in_edge_nf) +
          align64((int64_t)cfg->B * cfg->N * NB_H);
 }
+
+static int egno_backward(const NbEgnoConfig* cfg, const float* params, const float* nodes, const float* edge_fea,
+                         const float* loc_mean, const EgnoTimes& times, const float* saved, const float* g_x_out,
+                         const float* g_v_out, const float* g_h_out, float* grad_params, float* g_x_in, float* g_v_in,
+                         float* g_nodes, float* g_edge_fea, float* g_loc_mean, float* g_t_out, float* g_t_in,
+                         float* workspace, float* input_grad_workspace, void* stream);
 
 extern "C" int nb_egno_backward(const NbEgnoConfig* cfg, const float* params, const float* nodes, const float* edge_fea,
                                 const float* loc_mean, const int64_t* timesteps_out, const int64_t* timesteps_in,
@@ -1330,6 +1361,29 @@ extern "C" int nb_egno_backward_ex(const NbEgnoConfig* cfg, const float* params,
                                    const float* saved, const float* g_x_out, const float* g_v_out, const float* g_h_out,
                                    float* grad_params, float* g_x_in, float* g_v_in, float* g_nodes, float* g_edge_fea,
                                    float* g_loc_mean, float* workspace, float* input_grad_workspace, void* stream) {
+  const EgnoTimes times = {timesteps_out, timesteps_in, nullptr, nullptr};
+  return egno_backward(cfg, params, nodes, edge_fea, loc_mean, times, saved, g_x_out, g_v_out, g_h_out, grad_params,
+                       g_x_in, g_v_in, g_nodes, g_edge_fea, g_loc_mean, nullptr, nullptr, workspace, input_grad_workspace,
+                       stream);
+}
+
+extern "C" int nb_egno_backward_ft(const NbEgnoConfig* cfg, const float* params, const float* nodes, const float* edge_fea,
+                                   const float* loc_mean, const float* timesteps_out, const float* timesteps_in,
+                                   const float* saved, const float* g_x_out, const float* g_v_out, const float* g_h_out,
+                                   float* grad_params, float* g_x_in, float* g_v_in, float* g_nodes, float* g_edge_fea,
+                                   float* g_loc_mean, float* g_t_out, float* g_t_in, float* workspace,
+                                   float* input_grad_workspace, void* stream) {
+  const EgnoTimes times = {nullptr, nullptr, timesteps_out, timesteps_in};
+  return egno_backward(cfg, params, nodes, edge_fea, loc_mean, times, saved, g_x_out, g_v_out, g_h_out, grad_params,
+                       g_x_in, g_v_in, g_nodes, g_edge_fea, g_loc_mean, g_t_out, g_t_in, workspace, input_grad_workspace,
+                       stream);
+}
+
+static int egno_backward(const NbEgnoConfig* cfg, const float* params, const float* nodes, const float* edge_fea,
+                         const float* loc_mean, const EgnoTimes& times, const float* saved, const float* g_x_out,
+                         const float* g_v_out, const float* g_h_out, float* grad_params, float* g_x_in, float* g_v_in,
+                         float* g_nodes, float* g_edge_fea, float* g_loc_mean, float* g_t_out, float* g_t_in,
+                         float* workspace, float* input_grad_workspace, void* stream) {
   NB_RANGE("nb_egno_backward");
   EgnoCtx X;
   NB_TRY(egno_ctx_init(&X, cfg, params, stream));
@@ -1340,6 +1394,14 @@ extern "C" int nb_egno_backward_ex(const NbEgnoConfig* cfg, const float* params,
   const bool want_ef = g_edge_fea && cfg->in_edge_nf > 0;
   if ((g_nodes || g_edge_fea || g_loc_mean) && egno_L(cfg) > 1) {
     nb_set_error("gradients w.r.t. nodes / edge_fea / loc_mean are implemented for num_inputs = 1 only");
+    return NB_ERR_INVALID;
+  }
+  if ((g_t_out || g_t_in) && !times.fout) {
+    nb_set_error("time gradients need floating-point times (nb_egno_backward_ft)");
+    return NB_ERR_INVALID;
+  }
+  if (g_t_in && egno_L(cfg) == 1) {
+    nb_set_error("g_t_in needs num_inputs > 1 (a single input frame has no input times)");
     return NB_ERR_INVALID;
   }
   if ((g_nodes || want_ef) && !input_grad_workspace) {
@@ -1405,7 +1467,7 @@ extern "C" int nb_egno_backward_ex(const NbEgnoConfig* cfg, const float* params,
     NbSide* sd = side_get();
     cudaEventRecord(sd->fork2, cst);
     cudaStreamWaitEvent(sd->s2, sd->fork2, 0);
-    NB_TRY(egno_embed_inputs(cfg, X.lo, emb_args, nodes, timesteps_out, timesteps_in, ttab, P, Q, (void*)sd->s2));
+    NB_TRY(egno_embed_inputs(cfg, X.lo, emb_args, nodes, times, ttab, P, Q, (void*)sd->s2));
     embed_built = true;
   }
 #endif
@@ -1681,7 +1743,7 @@ extern "C" int nb_egno_backward_ex(const NbEgnoConfig* cfg, const float* params,
   {
     // dW_emb = gh^T [nodes | time embeddings], db_emb = column sums of gh: the inputs are re-materialised 64 wide
     // (scratch: P, Q, free by now) and reduced by the weight-gradient kernel; columns >= F are not written.
-    if (!embed_built) NB_TRY(egno_embed_inputs(cfg, X.lo, emb_args, nodes, timesteps_out, timesteps_in, ttab, P, Q, stream));
+    if (!embed_built) NB_TRY(egno_embed_inputs(cfg, X.lo, emb_args, nodes, times, ttab, P, Q, stream));
     const int F = X.lo.F;
     NB_TRY(wgrad_to((int)Nn, 1, wpair(gh_in, P), wpair(nullptr, nullptr), grad_params, X.lo.emb_w, F, 1, X.lo.emb_b, 0,
                     stream, F < NB_H ? F : NB_H));
@@ -1702,6 +1764,15 @@ extern "C" int nb_egno_backward_ex(const NbEgnoConfig* cfg, const float* params,
     NB_LAUNCH_COUNTED(k_sum_slices, (unsigned)ew_grid(egno_edge_rows(cfg) * cfg->in_edge_nf), 256, 0, stream,
                       (const float*)gef_rows, g_edge_fea, egno_edge_rows(cfg) * cfg->in_edge_nf, Ln * T);
   if (g_loc_mean && !cfg->use_time_conv) cudaMemsetAsync(g_loc_mean, 0, Nn0 * 3 * sizeof(float), cst);
+  if (g_t_out || g_t_in) {   // dL/dtimes from the same gh_in as the embedding's weight gradient
+    if (cfg->time_emb_dim == 0) {   // the times are unused
+      if (g_t_out) cudaMemsetAsync(g_t_out, 0, (int64_t)cfg->B * T * sizeof(float), cst);
+    } else {
+      NB_LAUNCH_COUNTED(k_time_grad, (unsigned)cfg->B, NB_TGRAD_THREADS, 0, stream, emb_args, times.fout, times.fin, gh_in,
+                        params + X.lo.emb_w, X.lo.F, g_t_out, g_t_in);
+      NB_TRY(nb_check_launch("k_time_grad"));
+    }
+  }
   defer_join(D, stream);
   return nb_check_launch("nb_egno_backward");
 }

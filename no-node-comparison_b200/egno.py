@@ -130,12 +130,11 @@ class EGNO(nn.Module):
         return self
 
     @staticmethod
-    def _integral_times(name, t, dev):
-        """The reference embeds `timesteps.float()` (layer_no.py:12); the kernels take int64 frame indices (what every
-        reference caller passes).  Floating-point times are accepted only when they are integral."""
-        if t.is_floating_point() and not bool((t == t.round()).all()):
-            raise ValueError(f"{name} holds non-integral times; only integer frame indices are implemented")
-        return t.to(device=dev, dtype=torch.int64).contiguous()
+    def _times(t, dev, floating):
+        """The reference embeds `timesteps.float()` (layer_no.py:12).  Integer times go to the kernels as int64 frame
+        indices (what every reference caller passes); floating-point times, integral or not, as that fp32 cast.  The
+        cast is an autograd op, so dL/dtimes reaches the caller's tensor in its own dtype and on its own device."""
+        return t.to(device=dev, dtype=torch.float32 if floating else torch.int64).contiguous()
 
     def forward(self, x, h, edge_index, edge_fea, v=None, loc_mean=None, timesteps_in=None, timesteps_out=None):
         T = self.num_timesteps
@@ -177,12 +176,14 @@ class EGNO(nn.Module):
         loc_mean = _require_cuda_f32("loc_mean", loc_mean, lead + (n0, 3))
         edge_fea = _require_cuda_f32("edge_fea", edge_fea, lead + (B * N * (N - 1), self.in_edge_nf))
         self._edges.validate(edge_index, B, N, dev)
-        tsteps = self._integral_times("timesteps_out", timesteps_out, dev)
+        # one kind of time for the call: floating point when either tensor is (an integer tensor beside it is exact in fp32)
+        floating = timesteps_out.is_floating_point() or (L > 1 and timesteps_in.is_floating_point())
+        tsteps = self._times(timesteps_out, dev, floating)
         tsteps_in = None
         if L > 1:
             if timesteps_in.shape[0] != B:
                 raise ValueError(f"timesteps_in must be [B={B}, {L}], got {tuple(timesteps_in.shape)}")
-            tsteps_in = self._integral_times("timesteps_in", timesteps_in, dev)
+            tsteps_in = self._times(timesteps_in, dev, floating)
         cfg = (B, N, T, self.n_layers, self.num_modes if self.use_time_conv else 1, self.in_node_nf, self.in_edge_nf,
                self.time_emb_dim, 1 if self.use_time_conv else 0, L)
         from ._lib import load_library

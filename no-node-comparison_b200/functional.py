@@ -159,9 +159,11 @@ class EgnoFunction(torch.autograd.Function):
         h_out = torch.empty((Nn, 64), device=dev, dtype=torch.float32)
         saved = torch.empty(lib.nb_egno_saved_floats(ctypes.byref(cfg)), device=dev, dtype=torch.float32) if need_grad else None
         ws = torch.empty(lib.nb_egno_workspace_floats(ctypes.byref(cfg), 2 if need_grad else 0), device=dev, dtype=torch.float32)
-        check(lib.nb_egno_forward(ctypes.byref(cfg), _ptr(flat), _ptr(x), _ptr(nodes), _ptr(edge_fea), _ptr(v),
-                                  _ptr(loc_mean), _ptr(tsteps), _ptr(tsteps_in), _ptr(x_out), _ptr(v_out), _ptr(h_out),
-                                  _ptr(saved), _ptr(ws), _stream_ptr(dev)), "nb_egno_forward")
+        # int64 frame indices, or fp32 times (any real value) through the _ft entry points
+        fwd = "nb_egno_forward_ft" if tsteps.is_floating_point() else "nb_egno_forward"
+        check(getattr(lib, fwd)(ctypes.byref(cfg), _ptr(flat), _ptr(x), _ptr(nodes), _ptr(edge_fea), _ptr(v),
+                                _ptr(loc_mean), _ptr(tsteps), _ptr(tsteps_in), _ptr(x_out), _ptr(v_out), _ptr(h_out),
+                                _ptr(saved), _ptr(ws), _stream_ptr(dev)), fwd)
         ctx.cfg_tuple = cfg_tuple
         ctx.dp_group = dp_group
         ctx.param_shapes = [p.shape for p in params]
@@ -187,6 +189,9 @@ class EgnoFunction(torch.autograd.Function):
         ws = torch.empty(lib.nb_egno_workspace_floats(ctypes.byref(cfg), 1), device=dev, dtype=torch.float32)
         want_nodes, want_ef, want_lm = ctx.needs_input_grad[4], ctx.needs_input_grad[5], ctx.needs_input_grad[7]
         g_nodes = g_ef = g_lm = None
+        if tsteps.is_floating_point():
+            return EgnoFunction._backward_ft(ctx, lib, cfg, flat, nodes, edge_fea, loc_mean, tsteps, tsteps_in, saved,
+                                             gx_out, gv_out, gh_out, grad_flat, gx_in, gv_in, ws)
         if want_nodes or want_ef or want_lm:
             # per-shard input gradients: under data parallelism nothing beyond the parameter bucket is reduced
             if want_ef:
@@ -205,13 +210,40 @@ class EgnoFunction(torch.autograd.Function):
                                        _ptr(tsteps), _ptr(tsteps_in), _ptr(saved), _ptr(gx_out), _ptr(gv_out), _ptr(gh_out),
                                        _ptr(grad_flat), _ptr(gx_in), _ptr(gv_in), _ptr(ws), _stream_ptr(dev)),
                   "nb_egno_backward")
+        return EgnoFunction._finish(ctx, grad_flat, gx_in, g_nodes, g_ef, gv_in, g_lm, None, None)
+
+    @staticmethod
+    def _backward_ft(ctx, lib, cfg, flat, nodes, edge_fea, loc_mean, tsteps, tsteps_in, saved, gx_out, gv_out, gh_out,
+                     grad_flat, gx_in, gv_in, ws):
+        """Floating-point times: nb_egno_backward_ft, which also returns dL/dtimesteps_out / dL/dtimesteps_in when asked
+        (per shard under data parallelism, like the other input gradients)."""
+        dev = flat.device
+        want = ctx.needs_input_grad
+        if want[5]:
+            _require_edge_grad_impl(lib)
+        g_nodes = torch.empty_like(nodes) if want[4] else None
+        g_ef = torch.empty_like(edge_fea) if want[5] else None
+        g_lm = torch.empty_like(loc_mean) if want[7] else None
+        g_t = torch.empty_like(tsteps) if want[8] else None
+        g_t_in = torch.empty_like(tsteps_in) if want[9] else None
+        iws = None
+        if want[4] or want[5]:
+            iws = torch.empty(lib.nb_egno_input_grad_workspace_floats(ctypes.byref(cfg)), device=dev, dtype=torch.float32)
+        check(lib.nb_egno_backward_ft(ctypes.byref(cfg), _ptr(flat), _ptr(nodes), _ptr(edge_fea), _ptr(loc_mean),
+                                      _ptr(tsteps), _ptr(tsteps_in), _ptr(saved), _ptr(gx_out), _ptr(gv_out), _ptr(gh_out),
+                                      _ptr(grad_flat), _ptr(gx_in), _ptr(gv_in), _ptr(g_nodes), _ptr(g_ef), _ptr(g_lm),
+                                      _ptr(g_t), _ptr(g_t_in), _ptr(ws), _ptr(iws), _stream_ptr(dev)), "nb_egno_backward_ft")
+        return EgnoFunction._finish(ctx, grad_flat, gx_in, g_nodes, g_ef, gv_in, g_lm, g_t, g_t_in)
+
+    @staticmethod
+    def _finish(ctx, grad_flat, gx_in, g_nodes, g_ef, gv_in, g_lm, g_t, g_t_in):
         _maybe_allreduce(grad_flat, ctx.dp_group)
         grads, o = [], 0
         for shp in ctx.param_shapes:
             n = shp.numel()
             grads.append(grad_flat[o:o + n].view(shp))
             o += n
-        return (None, None, None, gx_in, g_nodes, g_ef, gv_in, g_lm, None, None, *grads)
+        return (None, None, None, gx_in, g_nodes, g_ef, gv_in, g_lm, g_t, g_t_in, *grads)
 
 
 class SegnoFunction(torch.autograd.Function):
