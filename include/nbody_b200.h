@@ -259,8 +259,8 @@ int nb_profile_read(double* ms /*[NB_PROFILE_CATEGORIES]*/, long long* counts /*
 
 /* Edge-tile implementation: 2 = tcgen05 tensor-core tiles whose node gathers and receiver / sender reductions are
  * one-hot MMAs (default, product path; graphs with more than 27 nodes are walked in receiver x sender blocks by the same
- * kernels, template parameter BLK), 1 = tcgen05 tiles with CUDA-core gathers / reductions, 0 = fp32 SIMT tiles (kept as
- * an independent cross-check and for the host emulator of the test suite).  All are CUDA kernels of this library.
+ * kernels, template parameter BLK), 0 = fp32 SIMT tiles (kept as an independent cross-check and for the host emulator of
+ * the test suite).  Both are CUDA kernels of this library; any other value returns NB_ERR_INVALID.
  * The three nb_set_* switches below are process-wide TEST hooks (variant cross-checks); they are not meant to be flipped
  * while another thread is inside a forward / backward call. */
 int nb_set_edge_impl(int impl);

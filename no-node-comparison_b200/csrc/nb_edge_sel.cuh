@@ -1,6 +1,6 @@
 // nb_edge_sel.cuh — fused E_GCL edge tiles with ALL gathers and scatters on the tensor cores.
 //
-// Same math and unit / tile decomposition as nb_edge.cuh / nb_edge_tc.cuh.  What changes is how per-node data reaches
+// Same math and unit / tile decomposition as nb_edge.cuh.  What changes is how per-node data reaches
 // the edge rows and how per-edge data is reduced back onto nodes: both go through a one-hot *selector* tile
 //
 //     Sel[row][col]   (128 edge rows x 64 columns, bf16, exact 0/1 entries plus a few split scalars)
@@ -30,10 +30,28 @@
 #ifndef NB_EMU
 #include "nb_edge.cuh"
 #include "nb_tc.cuh"
-#include "nb_edge_tc.cuh"
 
 #define NB_SEL_MAX_GN 27
 #define NB_SEL_XC0 54  // first scalar column of the selector / first weight row of the node tile
+
+// stage a [64][64] fp32 weight matrix (row-major, row = output unit) as a split-bf16 operand tile
+__device__ __forceinline__ void nb_tc_stage_weight(unsigned char* hi, unsigned char* lo, const float* __restrict__ W,
+                                                   int tid) {
+  for (int idx = tid; idx < 64 * 8; idx += NB_THREADS) {
+    int o = idx >> 3, j = idx & 7;
+    float v[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) v[i] = __ldg(W + o * NB_H + 8 * j + i);
+    nb_tc_store8(hi, lo, o, j, v);
+  }
+}
+
+// fp32 [128][64] scratch with 16-byte chunks XOR-swizzled by (row & 7): conflict-free for row-owner writes and
+// for column-owner reads
+__device__ __forceinline__ float* nb_scratch_chunk(float* S, int r, int j4) { return S + r * NB_H + ((j4 ^ (r & 7)) << 2); }
+__device__ __forceinline__ float nb_scratch_get(const float* S, int r, int c) {
+  return S[r * NB_H + ((((c >> 2) ^ (r & 7))) << 2) + (c & 3)];
+}
 
 // one unit of work of a selector kernel (see "Units" above)
 struct NbSelUnit {

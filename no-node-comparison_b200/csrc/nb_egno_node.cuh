@@ -64,37 +64,18 @@ __global__ void __launch_bounds__(NB_THREADS, 2) k_egno_node_fwd(NbEgnoNodeFwdAr
     const int64_t gr0 = (int64_t)blockIdx.x * NB_TILE + row;
     nb_enf_load32(a.h + gr0 * NB_H + cb, (int)blockIdx.x < ntiles && gr0 < a.rows, v);
   }
-  uint64_t* wbar = bar + 2;   // weight images have landed (NB_WIMG_BULK)
-  if (NB_WIMG_BULK) {
-    if (tid == 0) {
-      nb_mbar_init(bar, 1);
-      nb_mbar_init(wbar, 1);
-      nb_mbar_fence_init();
-      nb_bulk_g2s(base, a.img, (uint32_t)NB_ENF_W_BYTES, wbar);
-    }
-  } else {
-    const uint4* src = reinterpret_cast<const uint4*>(a.img);
-    uint4* dst = reinterpret_cast<uint4*>(base);
-    constexpr int NCOPY = (int)NB_ENF_W_BYTES / 16 / NB_THREADS;   // 16 per thread
-    static_assert(NCOPY == 16, "weight-image copy is unrolled for 16 chunks per thread");
-#pragma unroll
-    for (int half = 0; half < 2; ++half) {
-      uint4 t[8];
-#pragma unroll
-      for (int i = 0; i < 8; ++i) t[i] = __ldg(src + tid + (half * 8 + i) * NB_THREADS);
-#pragma unroll
-      for (int i = 0; i < 8; ++i) dst[tid + (half * 8 + i) * NB_THREADS] = t[i];
-    }
+  uint64_t* wbar = bar + 2;   // weight images have landed
+  if (tid == 0) {
+    nb_mbar_init(bar, 1);
+    nb_mbar_init(wbar, 1);
+    nb_mbar_fence_init();
+    nb_bulk_g2s(base, a.img, (uint32_t)NB_ENF_W_BYTES, wbar);
   }
   if (tid < NB_H) {
     sb5[tid] = __ldg(a.b5 + tid);
     sb6[tid] = __ldg(a.b6 + tid);
     sbv1[tid] = __ldg(a.bv1 + tid);
     swv2[tid] = __ldg(a.wv2 + tid);
-  }
-  if (!NB_WIMG_BULK && tid == 0) {
-    nb_mbar_init(bar, 1);
-    nb_mbar_fence_init();
   }
   if (warp == 0) nb_tmem_alloc(tmem_slot, 256);
   nb_fence_async_smem();
@@ -123,7 +104,7 @@ __global__ void __launch_bounds__(NB_THREADS, 2) k_egno_node_fwd(NbEgnoNodeFwdAr
     nb_tc_fence_before();
     __syncthreads();   // (also: every thread has finished the previous tile's reads of D1 / cpart)
     if (NB_ISSUER(0)) {
-      if (NB_WIMG_BULK && tile == (int)blockIdx.x) nb_mbar_wait(wbar, 0);
+      if (tile == (int)blockIdx.x) nb_mbar_wait(wbar, 0);
       nb_tc_fence_after();
       nb_issue_w3_ta(tm, a0h, a0l, NB_ENF_WH(0), NB_ENF_WL(0), false, idesc_fwd, 0u);        // U5  = h W5a^T
       nb_issue_w3_ta(tm, a1h, a1l, NB_ENF_WH(1), NB_ENF_WL(1), false, idesc_fwd, 1u);        //     + M W5b^T
@@ -187,7 +168,7 @@ __global__ void __launch_bounds__(NB_THREADS, 2) k_egno_node_fwd(NbEgnoNodeFwdAr
     nb_enf_store32(a.h_out + off, live, v);
     nb_tc_fence_before();
   }
-  if (NB_WIMG_BULK && (int)blockIdx.x >= ntiles && tid == 0) nb_mbar_wait(wbar, 0);   // never exit under a copy in flight
+  if ((int)blockIdx.x >= ntiles && tid == 0) nb_mbar_wait(wbar, 0);   // never exit under a copy in flight
   nb_tc_fence_before();
   __syncthreads();
   if (warp == 0) nb_tmem_dealloc(tm, 256);
@@ -251,31 +232,14 @@ __global__ void __launch_bounds__(NB_THREADS, 2) k_egno_node_bwd(NbEgnoNodeBwdAr
     const int64_t gr0 = (int64_t)blockIdx.x * NB_TILE + row;
     nb_enf_load32(a.UV + gr0 * NB_H + cb, (int)blockIdx.x < ntiles && gr0 < a.rows, v);
   }
-  uint64_t* wbar = bar + 2;   // weight images have landed (NB_WIMG_BULK)
-  if (NB_WIMG_BULK) {
-    if (tid == 0) {
-      nb_mbar_init(bar, 1);
-      nb_mbar_init(wbar, 1);
-      nb_mbar_fence_init();
-      nb_bulk_g2s(base, a.img, (uint32_t)NB_ENF_W_BYTES, wbar);
-    }
-  } else {
-    const uint4* src = reinterpret_cast<const uint4*>(a.img);
-    uint4* dst = reinterpret_cast<uint4*>(base);
-#pragma unroll
-    for (int half = 0; half < 2; ++half) {
-      uint4 t[8];
-#pragma unroll
-      for (int i = 0; i < 8; ++i) t[i] = __ldg(src + tid + (half * 8 + i) * NB_THREADS);
-#pragma unroll
-      for (int i = 0; i < 8; ++i) dst[tid + (half * 8 + i) * NB_THREADS] = t[i];
-    }
+  uint64_t* wbar = bar + 2;   // weight images have landed
+  if (tid == 0) {
+    nb_mbar_init(bar, 1);
+    nb_mbar_init(wbar, 1);
+    nb_mbar_fence_init();
+    nb_bulk_g2s(base, a.img, (uint32_t)NB_ENF_W_BYTES, wbar);
   }
   if (tid < NB_H) swv2[tid] = __ldg(a.wv2 + tid);
-  if (!NB_WIMG_BULK && tid == 0) {
-    nb_mbar_init(bar, 1);
-    nb_mbar_fence_init();
-  }
   if (warp == 0) nb_tmem_alloc(tmem_slot, 256);
   nb_fence_async_smem();
   nb_tc_fence_before();
@@ -333,7 +297,7 @@ __global__ void __launch_bounds__(NB_THREADS, 2) k_egno_node_bwd(NbEgnoNodeBwdAr
     nb_tc_fence_before();
     __syncthreads();
     if (NB_ISSUER(0)) {
-      if (NB_WIMG_BULK && tile == (int)blockIdx.x) nb_mbar_wait(wbar, 0);
+      if (tile == (int)blockIdx.x) nb_mbar_wait(wbar, 0);
       nb_tc_fence_after();
       nb_issue_w3_ta(tm, a0h, a0l, NB_ENF_WH(2), NB_ENF_WL(2), true, idesc_mn, 0u);        // gh W6
       nb_issue_w3_ta(tm + 64, a1h, a1l, NB_ENF_WH(3), NB_ENF_WL(3), true, idesc_mn, 0u);   // gh1 = GUV Wv1
@@ -389,7 +353,7 @@ __global__ void __launch_bounds__(NB_THREADS, 2) k_egno_node_bwd(NbEgnoNodeBwdAr
         (red[(4 * h2 + 0) * 32 + j] + red[(4 * h2 + 1) * 32 + j]) + (red[(4 * h2 + 2) * 32 + j] + red[(4 * h2 + 3) * 32 + j]);
   }
   if (tid == 0) a.partial[(int64_t)blockIdx.x * 65 + 64] = (red[8 * 32 + 0] + red[8 * 32 + 1]) + (red[8 * 32 + 2] + red[8 * 32 + 3]);
-  if (NB_WIMG_BULK && (int)blockIdx.x >= ntiles && tid == 0) nb_mbar_wait(wbar, 0);   // never exit under a copy in flight
+  if ((int)blockIdx.x >= ntiles && tid == 0) nb_mbar_wait(wbar, 0);   // never exit under a copy in flight
   if (warp == 0) nb_tmem_dealloc(tm, 256);
 }
 
@@ -427,28 +391,14 @@ __global__ void __launch_bounds__(NB_THREADS, 2) k_egno_pair(NbEgnoPairArgs a) {
     const int64_t gr0 = (int64_t)blockIdx.x * NB_TILE + row;
     nb_enf_load32(a.A0 + gr0 * NB_H + cb, (int)blockIdx.x < ntiles && gr0 < a.rows, v);
   }
-  uint64_t* wbar = bar + 2;   // weight images have landed (NB_WIMG_BULK)
-  if (NB_WIMG_BULK) {
-    if (tid == 0) {
-      nb_mbar_init(bar, 1);
-      nb_mbar_init(wbar, 1);
-      nb_mbar_fence_init();
-      nb_bulk_g2s(base, a.img, (uint32_t)NB_EPR_W_BYTES, wbar);
-    }
-  } else {
-    const uint4* src = reinterpret_cast<const uint4*>(a.img);
-    uint4* dst = reinterpret_cast<uint4*>(base);
-    uint4 t[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) t[i] = __ldg(src + tid + i * NB_THREADS);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) dst[tid + i * NB_THREADS] = t[i];
+  uint64_t* wbar = bar + 2;   // weight images have landed
+  if (tid == 0) {
+    nb_mbar_init(bar, 1);
+    nb_mbar_init(wbar, 1);
+    nb_mbar_fence_init();
+    nb_bulk_g2s(base, a.img, (uint32_t)NB_EPR_W_BYTES, wbar);
   }
   if (tid < NB_H) sbias[tid] = (PQ && a.bias) ? __ldg(a.bias + tid) : 0.f;
-  if (!NB_WIMG_BULK && tid == 0) {
-    nb_mbar_init(bar, 1);
-    nb_mbar_fence_init();
-  }
   if (warp == 0) nb_tmem_alloc(tmem_slot, 256);
   nb_fence_async_smem();
   nb_tc_fence_before();
@@ -474,7 +424,7 @@ __global__ void __launch_bounds__(NB_THREADS, 2) k_egno_pair(NbEgnoPairArgs a) {
     nb_tc_fence_before();
     __syncthreads();
     if (NB_ISSUER(0)) {
-      if (NB_WIMG_BULK && tile == (int)blockIdx.x) nb_mbar_wait(wbar, 0);
+      if (tile == (int)blockIdx.x) nb_mbar_wait(wbar, 0);
       nb_tc_fence_after();
       if (PQ) {
         nb_issue_w3_ta(tm, a0h, a0l, NB_ENF_WH(0), NB_ENF_WL(0), false, idesc, 0u);
@@ -504,7 +454,7 @@ __global__ void __launch_bounds__(NB_THREADS, 2) k_egno_pair(NbEgnoPairArgs a) {
     }
     nb_tc_fence_before();
   }
-  if (NB_WIMG_BULK && (int)blockIdx.x >= ntiles && tid == 0) nb_mbar_wait(wbar, 0);   // never exit under a copy in flight
+  if ((int)blockIdx.x >= ntiles && tid == 0) nb_mbar_wait(wbar, 0);   // never exit under a copy in flight
   nb_tc_fence_before();
   __syncthreads();
   if (warp == 0) nb_tmem_dealloc(tm, 256);

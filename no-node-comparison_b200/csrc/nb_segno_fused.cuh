@@ -521,31 +521,12 @@ __global__ void __launch_bounds__(NB_THREADS, 1) k_segno_node_bwd(NbSegnoNodeBwd
       nb_snb_load32(a.gh_in + gr0 * NB_H + cb, live0 && a.gh_in, r);
     }
   }
-  uint64_t* wbar = bar + 2;   // weight images have landed (NB_WIMG_BULK: one TMA bulk copy, see nb_bulk_g2s)
-  if (NB_WIMG_BULK) {
-    if (tid == 0) {
-      nb_mbar_init(bar, 1);
-      nb_mbar_init(wbar, 1);
-      nb_mbar_fence_init();
-      nb_bulk_g2s(base, a.img, (uint32_t)(5 * 2 * NB_TC_TILE_BYTES(64)), wbar);
-    }
-  } else {
-    const uint4* src = reinterpret_cast<const uint4*>(a.img);
-    uint4* dst = reinterpret_cast<uint4*>(base);
-    constexpr int NCOPY = 5 * 2 * (int)NB_TC_TILE_BYTES(64) / 16 / NB_THREADS;   // 20 per thread
-    static_assert(NCOPY == 20, "weight-image copy is unrolled for 20 chunks per thread");
-#pragma unroll
-    for (int half = 0; half < 2; ++half) {
-      uint4 t[10];
-#pragma unroll
-      for (int i = 0; i < 10; ++i) t[i] = __ldg(src + tid + (half * 10 + i) * NB_THREADS);
-#pragma unroll
-      for (int i = 0; i < 10; ++i) dst[tid + (half * 10 + i) * NB_THREADS] = t[i];
-    }
-  }
-  if (!NB_WIMG_BULK && tid == 0) {
+  uint64_t* wbar = bar + 2;   // weight images have landed (one TMA bulk copy, see nb_bulk_g2s)
+  if (tid == 0) {
     nb_mbar_init(bar, 1);
+    nb_mbar_init(wbar, 1);
     nb_mbar_fence_init();
+    nb_bulk_g2s(base, a.img, (uint32_t)(5 * 2 * NB_TC_TILE_BYTES(64)), wbar);
   }
   if (warp == 0) nb_tmem_alloc(tmem_slot, 512);
   {  // integrator backward: independent element-wise work, issued while the weight copies are in flight
@@ -591,7 +572,7 @@ __global__ void __launch_bounds__(NB_THREADS, 1) k_segno_node_bwd(NbSegnoNodeBwd
       nb_tc_fence_before();
       __syncthreads();
       if (NB_ISSUER(0)) {
-        if (NB_WIMG_BULK && tile == (int)blockIdx.x) nb_mbar_wait(wbar, 0);
+        if (tile == (int)blockIdx.x) nb_mbar_wait(wbar, 0);
         nb_tc_fence_after();
         nb_issue_w3_ta(tm, a0h, a0l, NB_SNB_WH(0), NB_SNB_WL(0), true, idesc_mn, 0u);
         nb_issue_w3_ta(tm, a1h, a1l, NB_SNB_WH(1), NB_SNB_WL(1), true, idesc_mn, 1u);
@@ -614,7 +595,7 @@ __global__ void __launch_bounds__(NB_THREADS, 1) k_segno_node_bwd(NbSegnoNodeBwd
     nb_tc_fence_before();
     __syncthreads();
     if (NB_ISSUER(0)) {
-      if (NB_WIMG_BULK && HEAD && tile == (int)blockIdx.x) nb_mbar_wait(wbar, 0);
+      if (HEAD && tile == (int)blockIdx.x) nb_mbar_wait(wbar, 0);
       nb_tc_fence_after();
       nb_issue_w3_ta(tm, a0h, a0l, NB_SNB_WH(4), NB_SNB_WL(4), true, idesc_mn, 0u);
       nb_mma_commit(bar);
@@ -651,7 +632,7 @@ __global__ void __launch_bounds__(NB_THREADS, 1) k_segno_node_bwd(NbSegnoNodeBwd
     nb_snb_store32(a.gM + off, live, v);
     nb_tc_fence_before();
   }
-  if (NB_WIMG_BULK && (int)blockIdx.x >= ntiles && tid == 0) nb_mbar_wait(wbar, 0);   // never exit under a copy in flight
+  if ((int)blockIdx.x >= ntiles && tid == 0) nb_mbar_wait(wbar, 0);   // never exit under a copy in flight
   nb_tc_fence_before();
   __syncthreads();
   if (warp == 0) nb_tmem_dealloc(tm, 512);

@@ -76,9 +76,6 @@ __device__ __forceinline__ bool nb_elect_one() {
 // images of the node kernels are stored in global memory in their shared-memory tile layout, so a whole set of tiles is
 // one such copy: no register staging, and the copy runs underneath the first tile's row loads.  The data is written and
 // (by tcgen05.mma) read through the async proxy: the reader only has to wait for the barrier.
-#ifndef NB_WIMG_BULK
-#define NB_WIMG_BULK 1
-#endif
 __device__ __forceinline__ void nb_bulk_g2s(void* dst_smem, const void* src_gmem, uint32_t bytes, uint64_t* bar) {
   const uint32_t b = nb_smem_u32(bar);
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(b), "r"(bytes) : "memory");

@@ -12,7 +12,6 @@
 #include "nb_sim.cuh"
 #include "nb_edge.cuh"
 #include "nb_tc.cuh"
-#include "nb_edge_tc.cuh"
 #include "nb_edge_sel.cuh"
 #include "nb_node_tc.cuh"
 #include "nb_segno_fused.cuh"
@@ -66,10 +65,8 @@ struct NbSide {
 static NbSide* side_get() {
   static NbSide tab[64];
   static bool tried[64];
-  static int off = -1;
-  if (off < 0) { const char* e = getenv("NB_B200_SIDE_STREAM"); off = (e && e[0] == '0') ? 1 : 0; }
   int dev = 0;
-  if (off || cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
   NbSide& x = tab[dev];
   if (!tried[dev]) {
     tried[dev] = true;
@@ -472,9 +469,8 @@ static int q_flush_wgrad(void* st) {
   if (g_node_impl == 1) {
     // CTAs per SM over all jobs of the batch.  Three fit (and were the choice while the launch had the GPU to itself); on
     // the second stream, sharing the SMs with the next layer's kernels, two measured better (same box, alternating:
-    // 3.241 / 3.241 ms per EGNO step with 3, 3.207 / 3.225 with 2, 3.277 with 1; NB_B200_WGRAD_CTAS for A/B).
-    static int ctas = 0;
-    if (!ctas) { const char* e = getenv("NB_B200_WGRAD_CTAS"); ctas = (e && e[0] >= '1' && e[0] <= '3') ? e[0] - '0' : 2; }
+    // 3.241 / 3.241 ms per EGNO step with 3, 3.207 / 3.225 with 2, 3.277 with 1).
+    const int ctas = 2;
     int per_job = ctas * nb_num_sms() / wb.njobs;
     if (per_job < 16) per_job = 16;
     if (per_job > nb_num_sms()) per_job = nb_num_sms();
@@ -623,9 +619,9 @@ static NbEdgeGeom edge_geom(int n_gt, int B, int N, int nef, int clamp_edge) {
   return g;
 }
 
-// 2 = tcgen05 edge tiles with tensor-core gathers / scatters (nb_edge_sel.cuh; product path on sm_100a for N <= 27,
-//     larger graphs run variant 1), 1 = tcgen05 edge tiles with CUDA-core gathers / reductions (nb_edge_tc.cuh),
-// 0 = fp32 SIMT tiles (cross-check; the only variant the host emulator can run)
+// 2 = tcgen05 edge tiles with tensor-core gathers / scatters (nb_edge_sel.cuh; product path on sm_100a, whole-graph
+//     units for N <= 27 and the blocked walk up to N = 255), 0 = fp32 SIMT tiles (cross-check; the only variant the
+//     host emulator can run)
 #ifdef NB_EMU
 static int g_edge_impl = 0;
 #else
@@ -635,7 +631,7 @@ extern "C" int nb_set_edge_impl(int impl) {
 #ifdef NB_EMU
   if (impl != 0) { nb_set_error("the host emulator only runs the SIMT edge tiles"); return NB_ERR_INVALID; }
 #endif
-  if (impl < 0 || impl > 2) { nb_set_error("edge impl must be 0 (SIMT), 1 (tcgen05) or 2 (tcgen05 + selector MMAs)"); return NB_ERR_INVALID; }
+  if (impl != 0 && impl != 2) { nb_set_error("edge impl must be 0 (SIMT) or 2 (tcgen05 + selector MMAs)"); return NB_ERR_INVALID; }
   g_edge_impl = impl;
   return NB_OK;
 }
@@ -708,15 +704,6 @@ static int launch_edge_fwd(NbEdgeFwdArgs& a, void* st) {
     }
     prof_end(0, pi_sel, st);
     return nb_check_launch("k_edge_fwd_sel");
-  }
-  if (g_edge_impl >= 1) {
-    const size_t smem_tc = NB_EDGE_FWD_TC_SMEM;
-    NB_SET_SMEM(k_edge_fwd_tc, smem_tc);
-    int grid_tc = imin(a.g.n_units, 3 * nb_num_sms());
-    int pi_tc = prof_begin(0, st);
-    NB_LAUNCH_COUNTED(k_edge_fwd_tc, (unsigned)grid_tc, NB_THREADS, smem_tc, st, a);
-    prof_end(0, pi_tc, st);
-    return nb_check_launch("k_edge_fwd_tc");
   }
 #endif
   const size_t smem = NB_EDGE_FWD_SMEM_FLOATS * sizeof(float);
@@ -799,19 +786,6 @@ static int launch_edge_bwd(NbEdgeBwdArgs& a, float* dst, const EdgeGradDst& d, i
     }
     prof_end(1, pi_sel, st);
     NB_TRY(nb_check_launch("k_edge_bwd_sel"));
-    done = true;
-  } else if (g_edge_impl >= 1) {
-    if (a.gef) {
-      nb_set_error("edge-feature gradients need edge impl 2 (selector kernels) or 0 (SIMT); the tcgen05 cross-check "
-                   "kernels of edge impl 1 do not form them");
-      return NB_ERR_INVALID;
-    }
-    const size_t smem_tc = NB_EDGE_BWD_TC_SMEM(a.g.G * a.g.N);
-    NB_SET_SMEM(k_edge_bwd_tc, smem_tc);
-    int pi_tc = prof_begin(1, st);
-    NB_LAUNCH_COUNTED(k_edge_bwd_tc, (unsigned)grid, NB_THREADS, smem_tc, st, a);
-    prof_end(1, pi_tc, st);
-    NB_TRY(nb_check_launch("k_edge_bwd_tc"));
     done = true;
   }
 #endif
@@ -1121,12 +1095,10 @@ static inline int tconv_grid(const EgnoCtx& X, int per_sm) {
 }
 
 // the fused per-layer node kernels (nb_egno_node.cuh) need the tcgen05 variants and this call's weight images;
-// NB_B200_EGNO_NODE_FUSED=0 keeps the generic GEMM launches (A/B switch)
+// nb_set_node_fused(0) keeps the generic GEMM launches
 static bool egno_node_fused(const EgnoCtx& X) {
 #ifndef NB_EMU
-  static int off = -1;
-  if (off < 0) { const char* e = getenv("NB_B200_EGNO_NODE_FUSED"); off = (e && e[0] == '0') ? 1 : 0; }
-  return !off && g_node_fused && g_node_impl == 1 && g_wimg.n == EGNO_WIMG_PER_LAYER * X.c->n_layers;
+  return g_node_fused && g_node_impl == 1 && g_wimg.n == EGNO_WIMG_PER_LAYER * X.c->n_layers;
 #else
   (void)X;
   return false;
@@ -2082,11 +2054,7 @@ extern "C" int nb_segno_backward_ex(const NbSegnoConfig* cfg, const float* param
   // are in use; the first sub-step of the sweep (k = T - 1) and the tail (k = 0) keep the separate launches.
   bool chain = false;
 #ifndef NB_EMU
-  {
-    static int off = -1;
-    if (off < 0) { const char* e = getenv("NB_B200_SEGNO_CHAIN"); off = (e && e[0] == '0') ? 1 : 0; }
-    chain = !off && g_segno_fused && g_node_impl == 1 && g_wimg.n == SEGNO_WIMG;   // nb_set_segno_fused(0): stepwise both ways
-  }
+  chain = g_segno_fused && g_node_impl == 1 && g_wimg.n == SEGNO_WIMG;   // nb_set_segno_fused(0): stepwise both ways
 #endif
   // ---- weight gradients of the shared layers: ONE reduction per weight block over the rows of sub-steps [k0, k1) (the
   // operands of sub-step k sit k blocks apart: saved state at stride itf, the sweep's gradients at stride nh); queued on

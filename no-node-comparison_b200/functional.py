@@ -137,13 +137,6 @@ def dp_param(t: torch.Tensor, dp):
     return t if dp is None else _AllReduceGrad.apply(dp, t)
 
 
-def _require_edge_grad_impl(lib) -> None:
-    """The edge-feature gradient is formed inside the selector (impl 2) and SIMT (impl 0) edge backward kernels only."""
-    if lib.nb_get_edge_impl() == 1:
-        raise RuntimeError("gradients w.r.t. edge features are not formed by the nb_set_edge_impl(1) cross-check kernels "
-                           "(k_edge_bwd_tc); use edge impl 2 (default) or 0")
-
-
 class EgnoFunction(torch.autograd.Function):
     """x, v, h = EGNO.forward(...)   (reference: EGNO/model/egno.py:37-111)."""
 
@@ -194,8 +187,6 @@ class EgnoFunction(torch.autograd.Function):
                                              gx_out, gv_out, gh_out, grad_flat, gx_in, gv_in, ws)
         if want_nodes or want_ef or want_lm:
             # per-shard input gradients: under data parallelism nothing beyond the parameter bucket is reduced
-            if want_ef:
-                _require_edge_grad_impl(lib)
             g_nodes = torch.empty_like(nodes) if want_nodes else None
             g_ef = torch.empty_like(edge_fea) if want_ef else None
             g_lm = torch.empty_like(loc_mean) if want_lm else None
@@ -219,8 +210,6 @@ class EgnoFunction(torch.autograd.Function):
         (per shard under data parallelism, like the other input gradients)."""
         dev = flat.device
         want = ctx.needs_input_grad
-        if want[5]:
-            _require_edge_grad_impl(lib)
         g_nodes = torch.empty_like(nodes) if want[4] else None
         g_ef = torch.empty_like(edge_fea) if want[5] else None
         g_lm = torch.empty_like(loc_mean) if want[7] else None
@@ -291,8 +280,6 @@ class SegnoFunction(torch.autograd.Function):
         want_ef = ctx.needs_input_grad[6]
         g_his = g_ea = None
         if want_his or want_ef:
-            if want_ef:
-                _require_edge_grad_impl(lib)
             g_his = torch.empty_like(his) if want_his else None
             g_ea = torch.empty_like(edge_attr) if want_ef else None
             iws = torch.empty(lib.nb_segno_input_grad_workspace_floats(ctypes.byref(cfg)), device=dev, dtype=torch.float32)

@@ -495,20 +495,3 @@ def test_input_grads_are_bitwise_deterministic(c):
     a, b = (_cuda_run(c, make_model(c, d), inp, G) for _ in range(2))
     for k in NEW[c["model"]]:
         assert torch.equal(a[k], b[k]), k
-
-
-@pytest.mark.gpu
-def test_edge_grads_under_the_tc_cross_check_kernels_raise():
-    c = egno("egno_impl1", 131, B=3, N=5, T=4, L=1)
-    d = _dev()
-    lib = nb.load_library()
-    inp = make_inputs(c)
-    G = cotangents(c)
-    m = make_model(c, d)
-    assert lib.nb_set_edge_impl(1) == 0
-    try:
-        with pytest.raises(RuntimeError, match="nb_set_edge_impl\\(1\\)"):
-            _cuda_run(c, m, inp, G)
-    finally:
-        lib.nb_set_edge_impl(2)
-    assert lib.nb_get_edge_impl() == 2
