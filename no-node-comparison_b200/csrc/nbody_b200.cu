@@ -18,6 +18,7 @@
 #include "nb_merge.cuh"
 #include "nb_egno_node.cuh"
 #include <cstdlib>
+#include <initializer_list>
 
 // every kernel launch of this library is counted (bench.py reports it as gpu_launches)
 #define NB_LAUNCH_COUNTED(...)                             \
@@ -95,9 +96,21 @@ static void side_join(void* side_st, void* main_st) {
   cudaEventRecord(x->join, (cudaStream_t)side_st);
   cudaStreamWaitEvent((cudaStream_t)main_st, x->join, 0);
 }
+// the second side stream (deferred reductions, only with defer_available()): fork, completion slot i, wait for slot i
+static void* side2_fork(void* main_st) {
+  NbSide* x = side_get();
+  cudaEventRecord(x->fork2, (cudaStream_t)main_st);
+  cudaStreamWaitEvent(x->s2, x->fork2, 0);
+  return (void*)x->s2;
+}
+static void side2_done(int i) { cudaEventRecord(side_get()->done2[i], side_get()->s2); }
+static void side2_wait(void* main_st, int i) { cudaStreamWaitEvent((cudaStream_t)main_st, side_get()->done2[i], 0); }
 #else
 static void* side_fork(void* main_st) { return main_st; }
 static void side_join(void*, void*) {}
+static void* side2_fork(void* main_st) { return main_st; }
+static void side2_done(int) {}
+static void side2_wait(void*, int) {}
 #endif
 
 // ============================================================================= errors / device info
@@ -450,6 +463,11 @@ static float* q_alloc(int64_t nfloats, void* st) {
   g_q.pused += nfloats;
   return p;
 }
+static int q_partial(float** p, int64_t nfloats, void* st) {
+  *p = q_alloc(nfloats, st);
+  if (!*p) { nb_set_error("partial-sum workspace too small"); return NB_ERR_INVALID; }
+  return NB_OK;
+}
 static int launch_finalize(NbFinArgs& f, void* st) {
   int total = 0;
   for (int s = 0; s < f.nseg; ++s) total += f.seg[s].count;
@@ -457,6 +475,15 @@ static int launch_finalize(NbFinArgs& f, void* st) {
   if (g_q.fb.njobs == NB_MAX_FIN_JOBS) NB_TRY(q_flush_fin(st, false));
   g_q.fb.job[g_q.fb.njobs++] = f;
   return NB_OK;
+}
+// queues the reduction of `nparts` partial slices of `plen` floats into dst at the given segments
+static int q_finalize(const float* partial, int nparts, int plen, float* dst, int accumulate,
+                      std::initializer_list<NbFinSeg> segs, void* st) {
+  NbFinArgs f;
+  memset(&f, 0, sizeof(f));
+  f.partial = partial; f.nparts = nparts; f.plen = plen; f.dst = dst; f.accumulate = accumulate;
+  for (const NbFinSeg& s : segs) f.seg[f.nseg++] = s;
+  return launch_finalize(f, st);
 }
 static int q_flush_wgrad(void* st) {
   NbWgradBatch& wb = g_q.wb;
@@ -507,15 +534,11 @@ static int q_flush_wgrad(void* st) {
   const int n = wb.njobs;
   wb.njobs = 0;
   for (int j = 0; j < n; ++j) {
-    NbFinArgs f;
-    memset(&f, 0, sizeof(f));
     const WgradFin& wf = g_q.wfin[j];
-    f.partial = wb.job[j].partial; f.nparts = grid; f.plen = NB_WGRAD_PLEN; f.dst = wf.dst; f.accumulate = wf.accumulate;
-    f.nseg = 0;
-    f.seg[f.nseg++] = fseg(0, NB_H * NB_H, NB_H, wf.w_off, wf.so, wf.si);
-    f.seg[f.nseg - 1].klimit = wf.klimit;
-    if (wf.b_off >= 0) f.seg[f.nseg++] = fseg(NB_H * NB_H, NB_H, NB_H, wf.b_off, 0, 1);
-    NB_TRY(launch_finalize(f, st));
+    NbFinSeg w = fseg(0, NB_H * NB_H, NB_H, wf.w_off, wf.so, wf.si), b = fseg(NB_H * NB_H, NB_H, NB_H, wf.b_off, 0, 1);
+    w.klimit = wf.klimit;
+    if (wf.b_off >= 0) NB_TRY(q_finalize(wb.job[j].partial, grid, NB_WGRAD_PLEN, wf.dst, wf.accumulate, {w, b}, st));
+    else NB_TRY(q_finalize(wb.job[j].partial, grid, NB_WGRAD_PLEN, wf.dst, wf.accumulate, {w}, st));
   }
   return NB_OK;
 }
@@ -536,8 +559,8 @@ static int q_flush(void* st) {
 // graph edges.  NB_B200_WGRAD_DEFER=0 keeps the synchronous flush (A/B switch).
 struct DeferState {
   bool on;
-  int k;              // flushes issued so far
-  float* arena[2];    // partial-sum arenas, NB_PARTIAL_FLOATS each
+  int k;                     // flushes issued so far
+  float* const* arena;       // the two partial-sum arenas, NB_PARTIAL_FLOATS each
 };
 static bool defer_available() {
 #ifndef NB_EMU
@@ -549,29 +572,17 @@ static bool defer_available() {
 #endif
 }
 static int defer_flush(DeferState& D, void* main_st) {
-#ifndef NB_EMU
-  if (D.on) {
-    NbSide* x = side_get();
-    cudaStream_t ms = (cudaStream_t)main_st;
-    cudaEventRecord(x->fork2, ms);
-    cudaStreamWaitEvent(x->s2, x->fork2, 0);
-    NB_TRY(q_flush((void*)x->s2));
-    cudaEventRecord(x->done2[D.k & 1], x->s2);
-    if (D.k > 0) cudaStreamWaitEvent(ms, x->done2[(D.k - 1) & 1], 0);   // set (k + 1) & 1 is free again
-    ++D.k;
-    g_q.pbase = D.arena[D.k & 1];
-    g_q.pused = 0;
-    return nb_check_launch("deferred flush");
-  }
-#endif
-  return q_flush(main_st);
+  if (!D.on) return q_flush(main_st);
+  NB_TRY(q_flush(side2_fork(main_st)));
+  side2_done(D.k & 1);
+  if (D.k > 0) side2_wait(main_st, (D.k - 1) & 1);   // set (k + 1) & 1 is free again
+  ++D.k;
+  g_q.pbase = D.arena[D.k & 1];
+  g_q.pused = 0;
+  return nb_check_launch("deferred flush");
 }
 static void defer_join(DeferState& D, void* main_st) {
-#ifndef NB_EMU
-  if (D.on && D.k > 0) cudaStreamWaitEvent((cudaStream_t)main_st, side_get()->done2[(D.k - 1) & 1], 0);
-#else
-  (void)D; (void)main_st;
-#endif
+  if (D.on && D.k > 0) side2_wait(main_st, (D.k - 1) & 1);
 }
 
 // dst[w_off + o*so + k*si] (+)= sum_rows sum_p scale_p G_p[r][o] A_p[r][k];  dst[b_off + o] (+)= colsum(G_0) if b_off >= 0
@@ -601,6 +612,10 @@ static NbWgradPair wpair_seg(const float* G, const float* A, int a_silu, int seg
   NbWgradPair p = wpair(G, A, a_silu);
   p.seg_rows = seg_rows; p.seg_g = seg_g; p.seg_a = seg_a;
   return p;
+}
+static int wgrad_to(int rows, NbWgradPair p, float* dst, int64_t w_off, int64_t so, int64_t si, int64_t b_off,
+                    int accumulate, void* st, int klimit = 0) {
+  return wgrad_to(rows, 1, p, wpair(nullptr, nullptr), dst, w_off, so, si, b_off, accumulate, st, klimit);
 }
 
 static int ew_grid(int64_t n) { return imin(cdiv(n, 256), 8 * nb_num_sms()); }
@@ -723,19 +738,14 @@ struct EdgeGradDst {
 
 // reduction of `nparts` per-CTA partial slices of the edge backward kernel(s) into the parameter gradients
 static int edge_bwd_finalize(float* partial, int nparts, int nef, float* dst, const EdgeGradDst& d, int accumulate, void* st) {
-  NbFinArgs f;
-  memset(&f, 0, sizeof(f));
-  f.partial = partial; f.nparts = nparts; f.plen = NB_EB_PLEN; f.dst = dst; f.accumulate = accumulate;
-  f.nseg = 0;
-  f.seg[f.nseg++] = fseg(NB_EB_GW2, NB_H * NB_H, NB_H, d.W2, NB_H, 1);
-  f.seg[f.nseg++] = fseg(NB_EB_GW3, NB_H * NB_H, NB_H, d.W3, NB_H, 1);
-  f.seg[f.nseg++] = fseg(NB_EB_GB2, NB_H, NB_H, d.b2, 0, 1);
-  f.seg[f.nseg++] = fseg(NB_EB_GB3, NB_H, NB_H, d.b3, 0, 1);
-  f.seg[f.nseg++] = fseg(NB_EB_GW4, NB_H, NB_H, d.w4, 0, 1);
-  f.seg[f.nseg++] = fseg(NB_EB_GWR, NB_H, 1, d.w1 + d.col_rad, d.ldw1, 0);            // column col_rad of W1
-  f.seg[f.nseg++] = fseg(NB_EB_GWE, nef * NB_H, NB_H, d.w1 + d.col_ef, 1, d.ldw1);    // (f, c) -> W1[c][col_ef + f]
-  f.seg[f.nseg++] = fseg(NB_EB_GB4, 1, 1, d.b4, 0, 0);
-  return launch_finalize(f, st);
+  return q_finalize(partial, nparts, NB_EB_PLEN, dst, accumulate,
+                    {fseg(NB_EB_GW2, NB_H * NB_H, NB_H, d.W2, NB_H, 1), fseg(NB_EB_GW3, NB_H * NB_H, NB_H, d.W3, NB_H, 1),
+                     fseg(NB_EB_GB2, NB_H, NB_H, d.b2, 0, 1), fseg(NB_EB_GB3, NB_H, NB_H, d.b3, 0, 1),
+                     fseg(NB_EB_GW4, NB_H, NB_H, d.w4, 0, 1),
+                     fseg(NB_EB_GWR, NB_H, 1, d.w1 + d.col_rad, d.ldw1, 0),           // column col_rad of W1
+                     fseg(NB_EB_GWE, nef * NB_H, NB_H, d.w1 + d.col_ef, 1, d.ldw1),   // (f, c) -> W1[c][col_ef + f]
+                     fseg(NB_EB_GB4, 1, 1, d.b4, 0, 0)},
+                    st);
 }
 
 // run: when given, the finalisation is NOT queued here; the partial slices of consecutive launches are contiguous (the
@@ -756,8 +766,8 @@ static int launch_edge_bwd(NbEdgeBwdArgs& a, float* dst, const EdgeGradDst& d, i
     NB_TRY(q_flush(st));
     *run_parts = 0;
   }
-  float* partial = q_alloc((int64_t)grid * NB_EB_PLEN, st);
-  if (!partial) { nb_set_error("partial-sum workspace too small"); return NB_ERR_INVALID; }
+  float* partial;
+  NB_TRY(q_partial(&partial, (int64_t)grid * NB_EB_PLEN, st));
   a.partial = partial;
   if (run_base) {
     if (*run_parts == 0) *run_base = partial;
@@ -924,38 +934,61 @@ extern "C" int64_t nb_egno_saved_floats(const NbEgnoConfig* cfg) {
 
 // two tables (output times, input times) of T*B*D floats each: first region of the workspace
 static inline int64_t egno_table_floats(const NbEgnoConfig* c) { return 2 * align64((int64_t)c->T * c->B * (c->time_emb_dim > 0 ? c->time_emb_dim : 1)); }
-static inline int egno_L(const NbEgnoConfig* c) { return c->num_inputs > 1 ? c->num_inputs : 1; }
 // frame -> input map of repeat_elements_to_exact_shape (EGNO/utils.py:115-131)
 static NbFrameMap egno_frame_map(const NbEgnoConfig* c) {
   NbFrameMap fm;
   memset(&fm, 0, sizeof(fm));
-  fm.L = egno_L(c);
+  fm.L = c->num_inputs > 1 ? c->num_inputs : 1;
   const int reps = c->T / fm.L;
   for (int t = 0; t < c->T && t < NB_MAX_T; ++t) fm.m[t] = fm.L > 1 ? (t / reps < fm.L - 1 ? t / reps : fm.L - 1) : 0;
   return fm;
 }
-static void egno_geom_frames(const NbEgnoConfig* c, NbEdgeGeom& g) {
-  const NbFrameMap fm = egno_frame_map(c);
-  g.multi = fm.L > 1;
-  for (int t = 0; t < NB_MAX_T; ++t) g.tmap[t] = fm.m[t];
+struct EgnoCtx {
+  const NbEgnoConfig* c;
+  EgnoLayout lo;
+  NbTwiddle tw;
+  NbFrameMap fm;
+  int64_t Nn0, Nn;
+  const float* params;
+  void* st;
+};
+
+static int egno_ctx_init(EgnoCtx* X, const NbEgnoConfig* cfg, const float* params, void* st) {
+  NB_TRY(egno_validate(cfg));
+  X->c = cfg;
+  egno_layout(cfg, &X->lo);
+  if (cfg->use_time_conv) NB_TRY(make_twiddle(cfg->T, cfg->num_modes, &X->tw));
+  X->fm = egno_frame_map(cfg);
+  X->Nn0 = (int64_t)cfg->B * cfg->N;
+  X->Nn = X->Nn0 * cfg->T;
+  X->params = params;
+  X->st = st;
+  return NB_OK;
 }
-// embedding inputs (egno.py:50,59-76): fills the kernel arguments, builds the time table(s), materialises the input
-// rows 64 wide into ein0 (features 0..63) and ein1 (features 64.., only when F > 64)
+
+static NbEdgeGeom egno_edge_geom(const EgnoCtx& X) {
+  NbEdgeGeom g = edge_geom(X.c->T * X.c->B, X.c->B, X.c->N, X.c->in_edge_nf, 0);
+  g.multi = X.fm.L > 1;
+  for (int t = 0; t < NB_MAX_T; ++t) g.tmap[t] = X.fm.m[t];
+  return g;
+}
 // the time inputs of an EGNO call: int64 frame indices (nb_egno_forward, nb_egno_backward[_ex]) or fp32 times
 // (nb_egno_forward_ft, nb_egno_backward_ft); exactly one of the two pairs is set
 struct EgnoTimes {
   const int64_t *out, *in;
   const float *fout, *fin;
 };
-static int egno_embed_inputs(const NbEgnoConfig* cfg, const EgnoLayout& lo, NbEmbedArgs& e, const float* nodes,
-                             const EgnoTimes& ts, float* table, float* ein0, float* ein1, void* stream) {
+// embedding inputs (egno.py:50,59-76): fills the kernel arguments, builds the time table(s), materialises the input
+// rows 64 wide into ein0 (features 0..63) and ein1 (features 64.., only when F > 64)
+static int egno_embed_inputs(const EgnoCtx& X, NbEmbedArgs& e, const float* nodes, const EgnoTimes& ts, float* table,
+                             float* ein0, float* ein1, void* stream) {
+  const NbEgnoConfig* cfg = X.c;
   memset(&e, 0, sizeof(e));
   e.T = cfg->T; e.Nn0 = cfg->B * cfg->N; e.B = cfg->B; e.F0 = cfg->in_node_nf; e.D = cfg->time_emb_dim;
   e.nodes = nodes; e.tsteps = ts.out; e.tsteps_in = ts.in;
-  const NbFrameMap fm = egno_frame_map(cfg);
-  e.L = fm.L;
-  for (int t = 0; t < NB_MAX_T; ++t) e.tmap[t] = fm.m[t];
-  if (fm.L > 1 && (ts.fout ? !ts.fin : !ts.in)) { nb_set_error("num_inputs > 1 needs timesteps_in"); return NB_ERR_INVALID; }
+  e.L = X.fm.L;
+  for (int t = 0; t < NB_MAX_T; ++t) e.tmap[t] = X.fm.m[t];
+  if (X.fm.L > 1 && (ts.fout ? !ts.fin : !ts.in)) { nb_set_error("num_inputs > 1 needs timesteps_in"); return NB_ERR_INVALID; }
   const int half = e.D / 2;
   for (int k = 0; k < half; ++k) {
     float sc = (float)(log(10000.0) / (double)(half - 1));  // layer_no.py:10-11 (fp32 arange * python scalar)
@@ -968,15 +1001,15 @@ static int egno_embed_inputs(const NbEgnoConfig* cfg, const EgnoLayout& lo, NbEm
     const unsigned tg = (unsigned)imin(cdiv((int64_t)e.T * e.B * e.D, 256), 4 * nb_num_sms());
     if (ts.fout) {
       NB_LAUNCH_COUNTED(k_time_table_f, tg, 256, 0, stream, e, ts.fout, ts.fin, 0);
-      if (fm.L > 1) NB_LAUNCH_COUNTED(k_time_table_f, tg, 256, 0, stream, e, ts.fout, ts.fin, 1);
+      if (X.fm.L > 1) NB_LAUNCH_COUNTED(k_time_table_f, tg, 256, 0, stream, e, ts.fout, ts.fin, 1);
     } else {
       NB_LAUNCH_COUNTED(k_time_table, tg, 256, 0, stream, e, 0);
-      if (fm.L > 1) NB_LAUNCH_COUNTED(k_time_table, tg, 256, 0, stream, e, 1);
+      if (X.fm.L > 1) NB_LAUNCH_COUNTED(k_time_table, tg, 256, 0, stream, e, 1);
     }
     NB_TRY(nb_check_launch("k_time_table"));
   }
   NB_LAUNCH_COUNTED(k_embed_inputs, (unsigned)ew_grid(Nn * 16), 256, 0, stream, e, ein0, 0);
-  if (lo.F > NB_H) NB_LAUNCH_COUNTED(k_embed_inputs, (unsigned)ew_grid(Nn * 16), 256, 0, stream, e, ein1, NB_H);
+  if (X.lo.F > NB_H) NB_LAUNCH_COUNTED(k_embed_inputs, (unsigned)ew_grid(Nn * 16), 256, 0, stream, e, ein1, NB_H);
   return nb_check_launch("k_embed_inputs");
 }
 
@@ -985,27 +1018,85 @@ static int64_t egno_coef_floats(const NbEgnoConfig* c) {
   return align64((int64_t)ncoef * c->B * c->N * NB_H);
 }
 
+// ---- workspace layouts: each function carves the regions of one workspace, in order, from `base`.  With base ==
+// nullptr it only counts: the nb_*_workspace_floats queries return its `total`, so sizes and offsets have one source.
+struct Carve {
+  float* base;
+  int64_t used;
+  float* take(int64_t n) { float* p = base ? base + used : nullptr; used += n; return p; }
+};
+
+// EGNO forward; inference (nothing saved) adds two ping-pong layer sets
+struct EgnoFwdWs {
+  float *wimg, *ttab, *P, *Q, *coef, *ycoef, *infer;
+  int64_t total;
+};
+static EgnoFwdWs egno_fwd_ws(const NbEgnoConfig* c, bool infer, float* base) {
+  const int64_t Nn = (int64_t)c->T * c->B * c->N, nh = align64(Nn * NB_H), cf = egno_coef_floats(c);
+  Carve w = {base, 0};
+  EgnoFwdWs s;
+  s.wimg = w.take(wimg_floats(EGNO_WIMG_PER_LAYER * c->n_layers)); s.ttab = w.take(egno_table_floats(c));
+  s.P = w.take(nh); s.Q = w.take(nh); s.coef = w.take(cf); s.ycoef = w.take(cf);
+  s.infer = infer ? w.take(2 * align64(egno_layer_floats(Nn, (int64_t)c->B * c->N))) : nullptr;
+  s.total = w.used;
+  return s;
+}
+
+// EGNO backward.  A buffer set holds everything a queued weight-gradient job reads and the next layer rewrites; with
+// deferred flushes layer l uses set l & 1 and partial-sum arena l & 1 (see defer_flush), otherwise set 0 and arena 0.
+struct EgnoBwdSet {
+  float *gh, *GU5, *GUV, *gP, *gQ, *coef, *gycoef;
+};
+struct EgnoBwdWs {
+  float *wimg, *ttab, *P, *Q, *ycoef, *gcoef, *ghA, *gM, *gx[2], *gvA, *gvB, *gFsum, *arena[2];
+  EgnoBwdSet set[2];
+  int64_t total;
+};
+static EgnoBwdWs egno_bwd_ws(const NbEgnoConfig* c, float* base) {
+  const int64_t Nn = (int64_t)c->T * c->B * c->N, nh = align64(Nn * NB_H), n3 = align64(Nn * 3), cf = egno_coef_floats(c);
+  Carve w = {base, 0};
+  EgnoBwdWs s;
+  EgnoBwdSet &s0 = s.set[0], &s1 = s.set[1];
+  s.wimg = w.take(wimg_floats(EGNO_WIMG_PER_LAYER * c->n_layers)); s.ttab = w.take(egno_table_floats(c));
+  s.P = w.take(nh); s.Q = w.take(nh);
+  s0.coef = w.take(cf); s.ycoef = w.take(cf); s0.gycoef = w.take(cf); s.gcoef = w.take(cf);
+  s.ghA = w.take(nh); s0.gh = w.take(nh); s0.GU5 = w.take(nh); s0.GUV = w.take(nh); s.gM = w.take(nh); s0.gP = w.take(nh);
+  s0.gQ = w.take(nh);
+  s.gx[0] = w.take(n3); s.gx[1] = w.take(n3); s.gvA = w.take(n3); s.gvB = w.take(n3); s.gFsum = w.take(n3);
+  s.arena[0] = w.take(NB_PARTIAL_FLOATS);
+  s1.gh = w.take(nh); s1.GU5 = w.take(nh); s1.GUV = w.take(nh); s1.gP = w.take(nh); s1.gQ = w.take(nh);
+  s1.coef = w.take(cf); s1.gycoef = w.take(cf);
+  s.arena[1] = w.take(NB_PARTIAL_FLOATS);
+  s.total = w.used;
+  return s;
+}
+
+// input-gradient workspace of nb_egno_backward_ex: the per-row edge-feature gradients of every layer launch (each
+// launch writes its own slice of T * B*N(N-1) * in_edge_nf floats, no read-modify-write across layers), then the
+// embedding-output gradient summed over the T frames
+static inline int64_t egno_edge_rows(const NbEgnoConfig* c) { return (int64_t)c->B * c->N * (c->N - 1); }
+struct EgnoInputGradWs { float *gef_rows, *gh_sum; int64_t ef_slice, total; };
+static EgnoInputGradWs egno_input_grad_ws(const NbEgnoConfig* c, float* base) {
+  Carve w = {base, 0};
+  EgnoInputGradWs s;
+  s.ef_slice = (int64_t)c->T * egno_edge_rows(c) * c->in_edge_nf;
+  s.gef_rows = w.take(align64(s.ef_slice * c->n_layers));
+  s.gh_sum = w.take(align64((int64_t)c->B * c->N * NB_H));
+  s.total = w.used;
+  return s;
+}
+
 extern "C" int64_t nb_egno_workspace_floats(const NbEgnoConfig* cfg, int mode) {
   if (egno_validate(cfg) != NB_OK) return -1;
   if (mode < 0 || mode > 2) { nb_set_error("workspace mode must be 0 (inference), 1 (backward) or 2 (training forward)"); return -1; }
-  int64_t Nn = (int64_t)cfg->T * cfg->B * cfg->N;
-  int64_t nh = align64(Nn * NB_H), n3 = align64(Nn * 3), cf = egno_coef_floats(cfg);
-  const int64_t tab = egno_table_floats(cfg) + wimg_floats(EGNO_WIMG_PER_LAYER * cfg->n_layers);   // + weight images
-  if (mode == NB_WS_FORWARD_TRAIN) return tab + 2 * nh + 2 * cf;                     // `saved` holds the layer sets
-  if (mode == NB_WS_FORWARD_INFER) return tab + 2 * nh + 2 * cf + 2 * align64(egno_layer_floats(Nn, (int64_t)cfg->B * cfg->N));  // + ping-pong
-  return tab + 2 * nh /*P,Q*/ + 4 * cf + 2 * nh /*gh*/ + 5 * nh /*GU5 GUV gM gP gQ*/ + 4 * n3 /*gx, gv*/ + n3 /*gFsum*/ +
-         NB_PARTIAL_FLOATS +
-         5 * nh + 2 * cf + NB_PARTIAL_FLOATS;   // second set of gh, GU5, GUV, gP, gQ, coef, gycoef, arena (defer_flush)
+  if (mode == NB_WS_BACKWARD) return egno_bwd_ws(cfg, nullptr).total;
+  return egno_fwd_ws(cfg, mode == NB_WS_FORWARD_INFER, nullptr).total;
 }
 
-struct EgnoCtx {
-  const NbEgnoConfig* c;
-  EgnoLayout lo;
-  NbTwiddle tw;
-  int64_t Nn0, Nn;
-  const float* params;
-  void* st;
-};
+extern "C" int64_t nb_egno_input_grad_workspace_floats(const NbEgnoConfig* cfg) {
+  if (egno_validate(cfg) != NB_OK) return -1;
+  return egno_input_grad_ws(cfg, nullptr).total;
+}
 
 // the 64 x 64 weight blocks the node GEMMs of a layer multiply with (forward: as stored; backward: transposed views of
 // the same images): first edge layer's h_row / h_col columns, node_net layer 1 (h | M halves) and 2, node_v_net layer 1
@@ -1023,18 +1114,6 @@ static int egno_weight_images(const EgnoCtx& X, float* scratch) {
     W[n] = X.params + L.v_w1; ld[n++] = NB_H;
   }
   return wimg_prepare(W, ld, n, scratch, X.st);
-}
-
-static int egno_ctx_init(EgnoCtx* X, const NbEgnoConfig* cfg, const float* params, void* st) {
-  NB_TRY(egno_validate(cfg));
-  X->c = cfg;
-  egno_layout(cfg, &X->lo);
-  if (cfg->use_time_conv) NB_TRY(make_twiddle(cfg->T, cfg->num_modes, &X->tw));
-  X->Nn0 = (int64_t)cfg->B * cfg->N;
-  X->Nn = X->Nn0 * cfg->T;
-  X->params = params;
-  X->st = st;
-  return NB_OK;
 }
 
 // ---- temporal conv on h: mixing GEMMs coef -> ycoef (shared by forward and the backward's recompute)
@@ -1093,6 +1172,17 @@ static NbTconvArgs tconv_args(const EgnoCtx& X, int l) {
 static inline int tconv_grid(const EgnoCtx& X, int per_sm) {
   return imin(cdiv(X.Nn0, NB_TCV_ROWS), (int64_t)per_sm * nb_num_sms());
 }
+// k_tconv_fwd / k_tconv_bwd are instantiated for T <= 10 (the configured case, smaller register arrays) and NB_MAX_T
+static int launch_tconv(const EgnoCtx& X, const NbTconvArgs& tc, bool bwd) {
+  const bool t10 = X.c->T <= 10;
+  void (*k)(NbTconvArgs) = bwd ? (t10 ? k_tconv_bwd<10> : k_tconv_bwd<NB_MAX_T>) : (t10 ? k_tconv_fwd<10> : k_tconv_fwd<NB_MAX_T>);
+  const size_t smem = bwd ? NB_TCONV_BWD_SMEM : NB_TCONV_FWD_SMEM;
+  int pi = prof_begin(4, X.st);
+  NB_SET_SMEM(k, smem);
+  NB_LAUNCH_COUNTED(k, (unsigned)tconv_grid(X, bwd ? 2 : 3), 256, smem, X.st, tc);
+  prof_end(4, pi, X.st);
+  return nb_check_launch(bwd ? "k_tconv_bwd" : "k_tconv_fwd");
+}
 
 // the fused per-layer node kernels (nb_egno_node.cuh) need the tcgen05 variants and this call's weight images;
 // nb_set_node_fused(0) keeps the generic GEMM launches
@@ -1105,6 +1195,177 @@ static bool egno_node_fused(const EgnoCtx& X) {
 #endif
 }
 
+static NbEdgeW egno_edge_w(const EgnoCtx& X, int l) {
+  const EgnoLayerOff& L = X.lo.L[l];
+  NbEdgeW w;
+  w.W1 = X.params + L.e_w1; w.ldw1 = X.lo.E; w.col_rad = 0; w.col_ef = 1 + 2 * NB_H;
+  w.W2 = X.params + L.e_w2; w.b2 = X.params + L.e_b2; w.W3 = X.params + L.c_w1; w.b3 = X.params + L.c_b1;
+  w.w4 = X.params + L.c_w2; w.b4 = X.params + L.c_b2;
+  return w;
+}
+
+// ---- EGNO stages: each makes its own choice between the fused kernel and the generic launches; egno_forward /
+// egno_backward only order them around the stream fork / join and flush points.
+
+// h = Linear([nodes | time embeddings]) (egno.py:72-76): inputs materialised 64 wide (scratch: P, Q), then one GEMM;
+// and x, v replicated over T (egno.py:89-96)
+static int egno_embed_fwd(const EgnoCtx& X, const float* nodes, const EgnoTimes& times, const EgnoFwdWs& ws,
+                          const float* x, const float* v, const EgnoLayerBufs& b0) {
+  NbEmbedArgs e;
+  NB_TRY(egno_embed_inputs(X, e, nodes, times, ws.ttab, ws.P, ws.Q, X.st));
+  NbGemmArgs ga = gemm_args((int)X.Nn);
+  ga.nsrc = 1; ga.src[0] = gsrc(ws.P, NB_H, 0, X.params + X.lo.emb_w, 1, X.lo.F);
+  ga.src[0].kmax = X.lo.F < NB_H ? X.lo.F : NB_H;
+  if (X.lo.F > NB_H) {
+    ga.nsrc = 2; ga.src[1] = gsrc(ws.Q, NB_H, 0, X.params + X.lo.emb_w + NB_H, 1, X.lo.F);
+    ga.src[1].kmax = X.lo.F - NB_H;
+  }
+  ga.bias = X.params + X.lo.emb_b; ga.out = b0.h0;
+  NB_TRY(launch_gemm(ga, X.st));
+  const int n3 = (int)(X.Nn0 * 3);
+  NB_LAUNCH_COUNTED(k_replicate3, (unsigned)ew_grid(X.Nn * 3), 256, 0, X.st, x, b0.x0, n3, X.c->T, X.fm);
+  NB_LAUNCH_COUNTED(k_replicate3, (unsigned)ew_grid(X.Nn * 3), 256, 0, X.st, v, b0.v0, n3, X.c->T, X.fm);
+  return nb_check_launch("k_replicate3");
+}
+
+// dW_emb = gh^T [nodes | time embeddings], db_emb = column sums of gh: the inputs re-materialised 64 wide in P, Q (unless
+// `built` already) are reduced by the weight-gradient kernel; columns >= F are not written
+static int egno_embed_bwd(const EgnoCtx& X, NbEmbedArgs& e, bool built, const float* nodes, const EgnoTimes& times,
+                          const EgnoBwdWs& ws, const float* gh, float* grad) {
+  if (!built) NB_TRY(egno_embed_inputs(X, e, nodes, times, ws.ttab, ws.P, ws.Q, X.st));
+  const int F = X.lo.F;
+  NB_TRY(wgrad_to((int)X.Nn, wpair(gh, ws.P), grad, X.lo.emb_w, F, 1, X.lo.emb_b, 0, X.st, F < NB_H ? F : NB_H));
+  if (F > NB_H) NB_TRY(wgrad_to((int)X.Nn, wpair(gh, ws.Q), grad, X.lo.emb_w + NB_H, F, 1, -1, 0, X.st, F - NB_H));
+  return NB_OK;
+}
+
+// (x - mean, v) <- (x - mean, v) + conv(.)     (egno.py:103-108, layer_no.py:151-178)
+static NbTcxArgs tcx_args(const EgnoCtx& X, int l, const EgnoLayerBufs& b, const float* v0, const float* loc_mean) {
+  NbTcxArgs t;
+  memset(&t, 0, sizeof(t));
+  t.tw = X.tw; t.n3 = (int)(X.Nn0 * 3); t.x0 = b.x0; t.v0 = v0; t.mean = loc_mean; t.W = X.params + X.lo.L[l].tcx;
+  for (int tt = 0; tt < NB_MAX_T; ++tt) t.tmap[tt] = X.fm.m[tt];
+  return t;
+}
+static int egno_tcx_fwd(const EgnoCtx& X, int l, const EgnoLayerBufs& b, const float* v0, const float* loc_mean, void* st) {
+  NbTcxArgs t = tcx_args(X, l, b, v0, loc_mean);
+  t.x1 = b.x1; t.v1 = b.v1;
+  NB_LAUNCH_COUNTED(k_tcx_fwd, (unsigned)ew_grid(X.Nn0 * 3), 256, 0, st, t);
+  return nb_check_launch("k_tcx_fwd");
+}
+// on `st`, its partials reduced by the next flush; dL/dloc_mean right behind it, where both planes are final
+static int egno_tcx_bwd(const EgnoCtx& X, int l, const EgnoLayerBufs& b, const float* v0, const float* loc_mean,
+                        float* gx1, float* gv1, float* gx0, float* gv0, float* g_loc_mean, float* grad, void* st) {
+  const int nw = 2 * 2 * X.c->num_modes * 2;
+  NbTcxArgs t = tcx_args(X, l, b, v0, loc_mean);
+  t.gx1 = gx1; t.gv1 = gv1; t.gx0 = gx0; t.gv0 = gv0;
+  const int grid = imin(cdiv(X.Nn0 * 3, 256), 2 * nb_num_sms());
+  NB_TRY(q_partial(&t.partial, (int64_t)grid * nw, X.st));
+  NB_LAUNCH_COUNTED(k_tcx_bwd, (unsigned)grid, 256, 0, st, t);
+  NB_TRY(nb_check_launch("k_tcx_bwd"));
+  if (g_loc_mean) {
+    NB_LAUNCH_COUNTED(k_loc_mean_grad, (unsigned)ew_grid(X.Nn0 * 3), 256, 0, st, (const float*)gx1, (const float*)gx0,
+                      g_loc_mean, (int)(X.Nn0 * 3), X.c->T, l == X.c->n_layers - 1 ? 0 : 1);
+    NB_TRY(nb_check_launch("k_loc_mean_grad"));
+  }
+  return q_finalize(t.partial, grid, nw, grad, 0, {fseg(0, nw, nw, X.lo.L[l].tcx, 0, 1)}, X.st);
+}
+
+// h1 = h0 + LeakyReLU(conv(h0))      (layer_no.py:96-126): the fused kernel (mask: the LeakyReLU's sign bits for the
+// backward, training only), or DFT, mode-mixing GEMMs and inverse DFT through coef / ycoef
+static int egno_tconv_fwd(const EgnoCtx& X, int l, const EgnoLayerBufs& b, uint32_t* mask, float* coef, float* ycoef) {
+  if (egno_tconv_fused(X)) {
+    NbTconvArgs tc = tconv_args(X, l);
+    tc.x = b.h0; tc.out = b.h1; tc.mask = mask;
+    return launch_tconv(X, tc, false);
+  }
+  NbDftArgs d = dft_args(X);
+  d.x = b.h0; d.coef = coef;
+  NB_LAUNCH_COUNTED(k_dft_fwd, (unsigned)ew_grid(X.Nn0 * 16), 256, 0, X.st, d);
+  NB_TRY(nb_check_launch("k_dft_fwd"));
+  NB_TRY(egno_tc_mix(X, l, coef, ycoef));
+  d.ycoef = ycoef; d.out = b.h1;
+  NB_LAUNCH_COUNTED(k_idft_fwd, (unsigned)ew_grid(X.Nn0 * 16), 256, 0, X.st, d);
+  return nb_check_launch("k_idft_fwd");
+}
+// its backward dL/dh1 (gout) -> dL/dh0 (S.gh) and the mixing weight gradients: reduced by the next flush after the fused
+// kernel, here in the generic path (before the inverse DFT overwrites S.gh, which queued jobs of the layer above read)
+static int egno_tconv_bwd(const EgnoCtx& X, int l, const EgnoLayerBufs& b, const float* gout, const EgnoBwdSet& S,
+                          const EgnoBwdWs& ws, float* grad) {
+  const int modes = X.c->num_modes;
+  const bool fused = egno_tconv_fused(X);
+  NbDftArgs d = dft_args(X);
+  if (fused) {
+    NbTconvArgs tc = tconv_args(X, l);
+    tc.x = b.h0; tc.gout = gout; tc.gx = S.gh; tc.coef = S.coef; tc.gycoef = S.gycoef; tc.mask = b.tmask;
+    NB_TRY(launch_tconv(X, tc, true));
+  } else {
+    d.x = b.h0; d.coef = S.coef;
+    NB_LAUNCH_COUNTED(k_dft_fwd, (unsigned)ew_grid(X.Nn0 * 16), 256, 0, X.st, d);
+    NB_TRY(nb_check_launch("k_dft_fwd"));
+    NB_TRY(egno_tc_mix(X, l, S.coef, ws.ycoef));
+    d.ycoef = ws.ycoef; d.gout = gout; d.gycoef = S.gycoef;
+    NB_LAUNCH_COUNTED(k_idft_bwd, (unsigned)ew_grid(X.Nn0 * 16), 256, 0, X.st, d);
+    NB_TRY(nb_check_launch("k_idft_bwd"));
+  }
+  const float* W = X.params + X.lo.L[l].tc;
+  const int64_t plane = X.Nn0 * NB_H;
+  const int64_t tk = (int64_t)modes * 2, tn = (int64_t)NB_H * modes * 2;  // B[k=o][n=i] = W[i][o][m][c]
+  NbGemmArgs gj[2 * NB_MAX_T];
+  int ngj = 0;
+  for (int m = 0; m < modes; ++m) {
+    int ci = nb_coef_index(X.tw, m);
+    const float *Wr = W + m * 2, *Wi = W + m * 2 + 1;
+    const float *C = S.coef + ci * plane, *Sn = S.coef + (ci + 1) * plane;
+    const float *gPm = S.gycoef + ci * plane, *gQm = S.gycoef + (ci + 1) * plane;
+    const int64_t wr_off = X.lo.L[l].tc + m * 2, wi_off = X.lo.L[l].tc + m * 2 + 1;
+    if (m == 0 || m == X.tw.nyq) {
+      if (!fused) {
+        NbGemmArgs a = gemm_args((int)X.Nn0);  // gC = gP Wr^T
+        a.nsrc = 1; a.src[0] = gsrc(gPm, NB_H, 0, Wr, tk, tn);
+        a.out = ws.gcoef + ci * plane;
+        gj[ngj++] = a;
+      }
+      NB_TRY(wgrad_to((int)X.Nn0, wpair(C, gPm), grad, wr_off, tn, tk, -1, 0, X.st));
+    } else {
+      if (!fused) {
+        NbGemmArgs a = gemm_args((int)X.Nn0);  // gC = gP Wr^T + gQ Wi^T
+        a.nsrc = 2;
+        a.src[0] = gsrc(gPm, NB_H, 0, Wr, tk, tn);
+        a.src[1] = gsrc(gQm, NB_H, 0, Wi, tk, tn);
+        a.out = ws.gcoef + ci * plane;
+        gj[ngj++] = a;
+        NbGemmArgs s2 = gemm_args((int)X.Nn0);  // gS = gP Wi^T - gQ Wr^T
+        s2.nsrc = 2;
+        s2.src[0] = gsrc(gPm, NB_H, 0, Wi, tk, tn);
+        s2.src[1] = gsrc(gQm, NB_H, 0, Wr, tk, tn, -1.f);
+        s2.out = ws.gcoef + (ci + 1) * plane;
+        gj[ngj++] = s2;
+      }
+      // dWr[i][o] = sum C_i gP_o - S_i gQ_o ; dWi[i][o] = sum S_i gP_o + C_i gQ_o
+      NB_TRY(wgrad_to((int)X.Nn0, 2, wpair(C, gPm), wpair(Sn, gQm, 0, -1.f), grad, wr_off, tn, tk, -1, 0, X.st));
+      NB_TRY(wgrad_to((int)X.Nn0, 2, wpair(Sn, gPm), wpair(C, gQm), grad, wi_off, tn, tk, -1, 0, X.st));
+    }
+  }
+  if (fused) return NB_OK;
+  NB_TRY(launch_gemm_batch(gj, ngj, X.st));
+  NB_TRY(q_flush(X.st));
+  d.gcoef = ws.gcoef; d.gx = S.gh;
+  NB_LAUNCH_COUNTED(k_dft_bwd, (unsigned)ew_grid(X.Nn0 * 16), 256, 0, X.st, d);
+  return nb_check_launch("k_dft_bwd");
+}
+
+#ifndef NB_EMU
+template <bool FWD>
+static int launch_egno_pair(const EgnoCtx& X, const NbEgnoPairArgs& pa) {
+  NB_SET_SMEM(k_egno_pair<FWD>, NB_EPR_SMEM);
+  int pi = prof_begin(2, X.st);
+  NB_LAUNCH_COUNTED(k_egno_pair<FWD>, (unsigned)imin(cdiv(X.Nn, NB_TILE), 2 * nb_num_sms()), NB_THREADS, NB_EPR_SMEM, X.st, pa);
+  prof_end(2, pi, X.st);
+  return nb_check_launch("k_egno_pair");
+}
+#endif
+// P = h W1[:, h_row]^T + b1, Q = h W1[:, h_col]^T: the per-node halves of the first edge layer (basic.py:98,170)
 static int egno_pq(const EgnoCtx& X, int l, const float* h1, float* P, float* Q) {
   const EgnoLayerOff& L = X.lo.L[l];
   const int E = X.lo.E;
@@ -1113,11 +1374,7 @@ static int egno_pq(const EgnoCtx& X, int l, const float* h1, float* P, float* Q)
     NbEgnoPairArgs pa;
     memset(&pa, 0, sizeof(pa));
     pa.rows = (int)X.Nn; pa.img = g_wimg.img[EGNO_WIMG_PER_LAYER * l]; pa.A0 = h1; pa.bias = X.params + L.e_b1; pa.O0 = P; pa.O1 = Q;
-    NB_SET_SMEM(k_egno_pair<true>, NB_EPR_SMEM);
-    int pi = prof_begin(2, X.st);
-    NB_LAUNCH_COUNTED(k_egno_pair<true>, (unsigned)imin(cdiv(X.Nn, NB_TILE), 2 * nb_num_sms()), NB_THREADS, NB_EPR_SMEM, X.st, pa);
-    prof_end(2, pi, X.st);
-    return nb_check_launch("k_egno_pair");
+    return launch_egno_pair<true>(X, pa);
   }
 #endif
   NbGemmArgs a = gemm_args((int)X.Nn);  // P = h W1[:, h_row]^T + b1   (cols 1..64, basic.py:98,170)
@@ -1129,14 +1386,127 @@ static int egno_pq(const EgnoCtx& X, int l, const float* h1, float* P, float* Q)
   NbGemmArgs ab[2] = {a, b};
   return launch_gemm_batch(ab, 2, X.st);
 }
-
-static NbEdgeW egno_edge_w(const EgnoCtx& X, int l) {
+// its backward: gh1 += gP W1[:, h_row] + gQ W1[:, h_col], and the weight gradients
+static int egno_pair_bwd(const EgnoCtx& X, int l, const float* h1, const float* gP, const float* gQ, float* gh1, float* grad) {
   const EgnoLayerOff& L = X.lo.L[l];
-  NbEdgeW w;
-  w.W1 = X.params + L.e_w1; w.ldw1 = X.lo.E; w.col_rad = 0; w.col_ef = 1 + 2 * NB_H;
-  w.W2 = X.params + L.e_w2; w.b2 = X.params + L.e_b2; w.W3 = X.params + L.c_w1; w.b3 = X.params + L.c_b1;
-  w.w4 = X.params + L.c_w2; w.b4 = X.params + L.c_b2;
-  return w;
+#ifndef NB_EMU
+  if (egno_node_fused(X)) {
+    NbEgnoPairArgs pa;
+    memset(&pa, 0, sizeof(pa));
+    pa.rows = (int)X.Nn; pa.img = g_wimg.img[EGNO_WIMG_PER_LAYER * l]; pa.A0 = gP; pa.A1 = gQ; pa.O0 = gh1;
+    NB_TRY(launch_egno_pair<false>(X, pa));
+  } else
+#endif
+  {
+    NbGemmArgs a = gemm_args((int)X.Nn);
+    a.nsrc = 2;
+    a.src[0] = gsrc(gP, NB_H, 0, X.params + L.e_w1 + 1, X.lo.E, 1);
+    a.src[1] = gsrc(gQ, NB_H, 0, X.params + L.e_w1 + 1 + NB_H, X.lo.E, 1);
+    a.out = gh1; a.accumulate = 1;
+    NB_TRY(launch_gemm(a, X.st));
+  }
+  NB_TRY(wgrad_to((int)X.Nn, wpair(gP, h1), grad, L.e_w1 + 1, X.lo.E, 1, L.e_b1, 0, X.st));
+  return wgrad_to((int)X.Nn, wpair(gQ, h1), grad, L.e_w1 + 1 + NB_H, X.lo.E, 1, -1, 0, X.st);
+}
+
+// node_net, node_v_net and the coordinate update (basic.py:181-186): one pass over the rows (nb_egno_node.cuh), or the
+// generic GEMMs and k_egno_xupd_fwd.  U5, UV are kept for the backward (fused inference: on chip only)
+static int egno_node_fwd(const EgnoCtx& X, int l, const EgnoLayerBufs& b, const float* h1, const float* x1,
+                         const float* v1, bool train, float* h_next, float* x_next) {
+  const EgnoLayerOff& L = X.lo.L[l];
+  const float* params = X.params;
+  const int64_t Nn = X.Nn;
+#ifndef NB_EMU
+  if (egno_node_fused(X)) {
+    NbEgnoNodeFwdArgs na;
+    memset(&na, 0, sizeof(na));
+    na.rows = (int)Nn; na.N = X.c->N; na.img = g_wimg.img[EGNO_WIMG_PER_LAYER * l + 2];
+    na.h = h1; na.M = b.M; na.b5 = params + L.n_b1; na.b6 = params + L.n_b2; na.bv1 = params + L.v_b1;
+    na.wv2 = params + L.v_w2; na.bv2 = params + L.v_b2; na.x = x1; na.v = v1; na.Fsum = b.Fsum;
+    na.U5 = train ? b.U5 : nullptr; na.UV = train ? b.UV : nullptr;
+    na.h_out = h_next; na.x_out = x_next;
+    NB_SET_SMEM(k_egno_node_fwd, NB_ENF_SMEM);
+    int pi = prof_begin(6, X.st);
+    NB_LAUNCH_COUNTED(k_egno_node_fwd, (unsigned)imin(cdiv(Nn, NB_TILE), 2 * nb_num_sms()), NB_THREADS, NB_ENF_SMEM, X.st, na);
+    prof_end(6, pi, X.st);
+    return nb_check_launch("k_egno_node_fwd");
+  }
+#endif
+  NbGemmArgs a = gemm_args((int)Nn);  // U5 = [h, M] W5^T + b5      (basic.py:183-185)
+  a.nsrc = 2;
+  a.src[0] = gsrc(h1, NB_H, 0, params + L.n_w1, 1, 2 * NB_H);
+  a.src[1] = gsrc(b.M, NB_H, 0, params + L.n_w1 + NB_H, 1, 2 * NB_H);
+  a.bias = params + L.n_b1; a.out_pre = b.U5;
+  NbGemmArgs u = gemm_args((int)Nn);  // UV = h Wv1^T + bv1         (node_v_net, pre-update h)
+  u.nsrc = 1; u.src[0] = gsrc(h1, NB_H, 0, params + L.v_w1, 1, NB_H);
+  u.bias = params + L.v_b1; u.out_pre = b.UV;
+  NbGemmArgs au[2] = {a, u};
+  NB_TRY(launch_gemm_batch(au, 2, X.st));
+  NbGemmArgs c2 = gemm_args((int)Nn);  // h' = SiLU(U5) W6^T + b6  (no residual)
+  c2.nsrc = 1; c2.src[0] = gsrc(b.U5, NB_H, 1, params + L.n_w2, 1, NB_H);
+  c2.bias = params + L.n_b2; c2.out = h_next;
+  NB_TRY(launch_gemm(c2, X.st));
+  NbXupdArgs xa;
+  memset(&xa, 0, sizeof(xa));
+  xa.rows = Nn; xa.N = X.c->N; xa.x = x1; xa.v = v1; xa.UV = b.UV; xa.w2 = params + L.v_w2; xa.b2 = params + L.v_b2;
+  xa.Fsum = b.Fsum; xa.x_out = x_next;
+  NB_LAUNCH_COUNTED(k_egno_xupd_fwd, (unsigned)imin(cdiv(Nn, 8), 8 * nb_num_sms()), 256, 0, X.st, xa);
+  return nb_check_launch("k_egno_xupd_fwd");
+}
+// its backward: x' = x + s v + clamp(mean f) gives dL/dv1 (gv_out), dL/dFsum, dL/dUV and the 64->1 head of node_v_net;
+// node_net backwards gives GU5, dL/dh1 (gh1) and dL/dM.  One pass over the rows, or k_egno_xupd_bwd and the generic GEMMs
+static int egno_node_bwd(const EgnoCtx& X, int l, const EgnoLayerBufs& b, const float* h1, const float* gh_in, float* gx,
+                         const float* gv_in, float* gv_out, const EgnoBwdSet& S, const EgnoBwdWs& ws, float* gh1, float* grad) {
+  const EgnoLayerOff& L = X.lo.L[l];
+  const float* params = X.params;
+  const int64_t Nn = X.Nn;
+  const bool fused = egno_node_fused(X);
+  const int grid = fused ? imin(cdiv(Nn, NB_TILE), 2 * nb_num_sms()) : imin(cdiv(Nn, 8), 4 * nb_num_sms());
+  float* partial;
+  NB_TRY(q_partial(&partial, (int64_t)grid * 65, X.st));
+#ifndef NB_EMU
+  if (fused) {
+    NbEgnoNodeBwdArgs na;
+    memset(&na, 0, sizeof(na));
+    na.rows = (int)Nn; na.N = X.c->N; na.img = g_wimg.img[EGNO_WIMG_PER_LAYER * l + 2];
+    na.gh = gh_in; na.U5 = b.U5; na.UV = b.UV; na.wv2 = params + L.v_w2; na.bv2 = params + L.v_b2;
+    na.gx = gx; na.gv = gv_in; na.v = b.v1; na.Fsum = b.Fsum; na.gv_out = gv_out; na.gFsum = ws.gFsum;
+    na.GU5 = S.GU5; na.GUV = S.GUV; na.gh1 = gh1; na.gM = ws.gM; na.partial = partial;
+    NB_SET_SMEM(k_egno_node_bwd, NB_ENB_SMEM);
+    int pi = prof_begin(7, X.st);
+    NB_LAUNCH_COUNTED(k_egno_node_bwd, (unsigned)grid, NB_THREADS, NB_ENB_SMEM, X.st, na);
+    prof_end(7, pi, X.st);
+    NB_TRY(nb_check_launch("k_egno_node_bwd"));
+  } else
+#endif
+  {
+    NbXupdArgs xa;
+    memset(&xa, 0, sizeof(xa));
+    xa.rows = Nn; xa.N = X.c->N; xa.v = b.v1; xa.UV = b.UV; xa.w2 = params + L.v_w2; xa.b2 = params + L.v_b2;
+    xa.Fsum = b.Fsum; xa.gx = gx; xa.gv = gv_in; xa.gv_out = gv_out; xa.gFsum = ws.gFsum; xa.GUV = S.GUV;
+    xa.partial = partial;
+    NB_LAUNCH_COUNTED(k_egno_xupd_bwd, (unsigned)grid, 256, 0, X.st, xa);
+    NB_TRY(nb_check_launch("k_egno_xupd_bwd"));
+    NbGemmArgs a = gemm_args((int)Nn);  // GU5 = (gh W6) * SiLU'(U5)
+    a.nsrc = 1; a.src[0] = gsrc(gh_in, NB_H, 0, params + L.n_w2, NB_H, 1);
+    a.epi = NB_EPI_MUL_DSILU; a.U = b.U5; a.out = S.GU5;
+    NB_TRY(launch_gemm(a, X.st));
+    NbGemmArgs g1 = gemm_args((int)Nn);  // gh1 = GU5 W5[:, :64] + GUV Wv1
+    g1.nsrc = 2;
+    g1.src[0] = gsrc(S.GU5, NB_H, 0, params + L.n_w1, 2 * NB_H, 1);
+    g1.src[1] = gsrc(S.GUV, NB_H, 0, params + L.v_w1, NB_H, 1);
+    g1.out = gh1;
+    NbGemmArgs g2 = gemm_args((int)Nn);  // gM = GU5 W5[:, 64:]
+    g2.nsrc = 1; g2.src[0] = gsrc(S.GU5, NB_H, 0, params + L.n_w1 + NB_H, 2 * NB_H, 1);
+    g2.out = ws.gM;
+    NbGemmArgs g12[2] = {g1, g2};
+    NB_TRY(launch_gemm_batch(g12, 2, X.st));
+  }
+  NB_TRY(q_finalize(partial, grid, 65, grad, 0, {fseg(0, NB_H, NB_H, L.v_w2, 0, 1), fseg(NB_H, 1, 1, L.v_b2, 0, 0)}, X.st));
+  NB_TRY(wgrad_to((int)Nn, wpair(gh_in, b.U5, 1), grad, L.n_w2, NB_H, 1, L.n_b2, 0, X.st));
+  NB_TRY(wgrad_to((int)Nn, wpair(S.GU5, h1), grad, L.n_w1, 2 * NB_H, 1, L.n_b1, 0, X.st));
+  NB_TRY(wgrad_to((int)Nn, wpair(S.GU5, b.M), grad, L.n_w1 + NB_H, 2 * NB_H, 1, -1, 0, X.st));
+  return wgrad_to((int)Nn, wpair(S.GUV, h1), grad, L.v_w1, NB_H, 1, L.v_b1, 0, X.st);
 }
 
 static int egno_forward(const NbEgnoConfig* cfg, const float* params, const float* x, const float* nodes,
@@ -1145,146 +1515,45 @@ static int egno_forward(const NbEgnoConfig* cfg, const float* params, const floa
   NB_RANGE("nb_egno_forward");
   EgnoCtx X;
   NB_TRY(egno_ctx_init(&X, cfg, params, stream));
-  const int T = cfg->T, Ln = cfg->n_layers;
-  const int64_t Nn = X.Nn, Nn0 = X.Nn0;
-  const int64_t nh = align64(Nn * NB_H), cf = egno_coef_floats(cfg), lf = align64(egno_layer_floats(Nn, X.Nn0));
+  const int Ln = cfg->n_layers;
+  const int64_t lf = align64(egno_layer_floats(X.Nn, X.Nn0));
+  const EgnoFwdWs ws = egno_fwd_ws(cfg, !saved, workspace);
   WimgGuard wimg_guard;
-  NB_TRY(egno_weight_images(X, workspace));
-  float* ttab = workspace + wimg_floats(EGNO_WIMG_PER_LAYER * Ln);
-  float* P = ttab + egno_table_floats(cfg);
-  float* Q = P + nh;
-  float* coef = Q + nh;
-  float* ycoef = coef + cf;
-  float* infer = ycoef + cf;  // two layer-sets used when nothing is saved
-  auto bufs = [&](int l) { return egno_layer_bufs(saved ? saved + (int64_t)l * lf : infer + (int64_t)(l & 1) * lf, Nn); };
+  NB_TRY(egno_weight_images(X, ws.wimg));
+  // training keeps every layer's buffers in `saved`; inference alternates two sets in the workspace
+  auto bufs = [&](int l) { return egno_layer_bufs(saved ? saved + (int64_t)l * lf : ws.infer + (int64_t)(l & 1) * lf, X.Nn); };
 
-  // ---- embedding (egno.py:50,63-76) + replication of x, v over T (egno.py:89-96)
-  EgnoLayerBufs b0 = bufs(0);
-  {
-    // h = Linear([nodes | time embeddings]) (egno.py:72-76): inputs materialised 64 wide (scratch: P, Q), then one GEMM
-    NbEmbedArgs e;
-    NB_TRY(egno_embed_inputs(cfg, X.lo, e, nodes, times, ttab, P, Q, stream));
-    {
-      NbGemmArgs ga = gemm_args((int)Nn);
-      ga.nsrc = 1; ga.src[0] = gsrc(P, NB_H, 0, params + X.lo.emb_w, 1, X.lo.F);
-      ga.src[0].kmax = X.lo.F < NB_H ? X.lo.F : NB_H;
-      if (X.lo.F > NB_H) {
-        ga.nsrc = 2; ga.src[1] = gsrc(Q, NB_H, 0, params + X.lo.emb_w + NB_H, 1, X.lo.F);
-        ga.src[1].kmax = X.lo.F - NB_H;
-      }
-      ga.bias = params + X.lo.emb_b; ga.out = b0.h0;
-      NB_TRY(launch_gemm(ga, stream));
-    }
-    const NbFrameMap fm = egno_frame_map(cfg);
-    NB_LAUNCH_COUNTED(k_replicate3, (unsigned)ew_grid(Nn * 3), 256, 0, stream, x, b0.x0, (int)(Nn0 * 3), T, fm);
-    NB_LAUNCH_COUNTED(k_replicate3, (unsigned)ew_grid(Nn * 3), 256, 0, stream, v, b0.v0, (int)(Nn0 * 3), T, fm);
-    NB_TRY(nb_check_launch("k_replicate3"));
-  }
-
-  const float* v_prev = b0.v0;
+  NB_TRY(egno_embed_fwd(X, nodes, times, ws, x, v, bufs(0)));
+  const float* v_prev = bufs(0).v0;
   for (int l = 0; l < Ln; ++l) {
     EgnoLayerBufs b = bufs(l);
-    const EgnoLayerOff& L = X.lo.L[l];
-    const float* v0 = v_prev;
-    float *h1 = b.h1, *x1 = b.x1, *v1 = b.v1;
+    const float *h1 = b.h0, *x1 = b.x0;
     void* side = stream;
     if (cfg->use_time_conv) {
-      // (x - mean, v) <- (x - mean, v) + conv(.)     (egno.py:103-108, layer_no.py:151-178): independent of the h path
-      // until the edge kernel, so it runs on the side stream underneath the 64-channel convolution and the P | Q product
-      {
-        NbTcxArgs t;
-        memset(&t, 0, sizeof(t));
-        t.tw = X.tw; t.n3 = (int)(Nn0 * 3); t.x0 = b.x0; t.v0 = v0; t.mean = loc_mean; t.W = params + L.tcx;
-        { const NbFrameMap fmx = egno_frame_map(cfg); for (int tt = 0; tt < NB_MAX_T; ++tt) t.tmap[tt] = fmx.m[tt]; }
-        t.x1 = x1; t.v1 = v1;
-        side = side_fork(stream);
-        NB_LAUNCH_COUNTED(k_tcx_fwd, (unsigned)ew_grid(Nn0 * 3), 256, 0, side, t);
-        NB_TRY(nb_check_launch("k_tcx_fwd"));
-      }
-      // h <- h + LeakyReLU(conv(h))      (layer_no.py:96-126)
-      if (egno_tconv_fused(X)) {
-        NbTconvArgs tc = tconv_args(X, l);
-        tc.x = b.h0; tc.out = h1; tc.mask = saved ? b.tmask : nullptr;   // training: the LeakyReLU mask for the backward
-        int pi = prof_begin(4, stream);
-        if (T <= 10) {
-          NB_SET_SMEM(k_tconv_fwd<10>, NB_TCONV_FWD_SMEM);
-          NB_LAUNCH_COUNTED(k_tconv_fwd<10>, (unsigned)tconv_grid(X, 3), 256, NB_TCONV_FWD_SMEM, stream, tc);
-        } else {
-          NB_SET_SMEM(k_tconv_fwd<NB_MAX_T>, NB_TCONV_FWD_SMEM);
-          NB_LAUNCH_COUNTED(k_tconv_fwd<NB_MAX_T>, (unsigned)tconv_grid(X, 3), 256, NB_TCONV_FWD_SMEM, stream, tc);
-        }
-        prof_end(4, pi, stream);
-        NB_TRY(nb_check_launch("k_tconv_fwd"));
-      } else {
-        NbDftArgs d = dft_args(X);
-        d.x = b.h0; d.coef = coef;
-        NB_LAUNCH_COUNTED(k_dft_fwd, (unsigned)ew_grid(Nn0 * 16), 256, 0, stream, d);
-        NB_TRY(nb_check_launch("k_dft_fwd"));
-        NB_TRY(egno_tc_mix(X, l, coef, ycoef));
-        d.ycoef = ycoef; d.out = h1;
-        NB_LAUNCH_COUNTED(k_idft_fwd, (unsigned)ew_grid(Nn0 * 16), 256, 0, stream, d);
-        NB_TRY(nb_check_launch("k_idft_fwd"));
-      }
+      // the (x - mean, v) convolution is independent of the h path until the edge kernel: it runs on the side stream
+      // underneath the 64-channel convolution and the P | Q product
+      side = side_fork(stream);
+      NB_TRY(egno_tcx_fwd(X, l, b, v_prev, loc_mean, side));
+      NB_TRY(egno_tconv_fwd(X, l, b, saved ? b.tmask : nullptr, ws.coef, ws.ycoef));
+      h1 = b.h1; x1 = b.x1;
     } else {
-      h1 = b.h0; x1 = b.x0;
-      cudaMemcpyAsync(v1, v0, Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
+      cudaMemcpyAsync(b.v1, v_prev, X.Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
     }
     // ---- EGNN layer (basic.py:167-186)
-    float* Pl = saved ? b.P : P;  // training: kept for the backward edge tile
-    float* Ql = saved ? b.Q : Q;
-    NB_TRY(egno_pq(X, l, h1, Pl, Ql));
+    float* P = saved ? b.P : ws.P;  // training: kept for the backward edge tile
+    float* Q = saved ? b.Q : ws.Q;
+    NB_TRY(egno_pq(X, l, h1, P, Q));
     side_join(side, stream);
     NbEdgeFwdArgs ea;
-    ea.g = edge_geom(T * cfg->B, cfg->B, cfg->N, cfg->in_edge_nf, 0);
-    egno_geom_frames(cfg, ea.g);
+    ea.g = egno_edge_geom(X);
     ea.w = egno_edge_w(X, l);
-    ea.x = x1; ea.P = Pl; ea.Q = Ql; ea.ef = edge_fea; ea.M = b.M; ea.Fsum = b.Fsum;
+    ea.x = x1; ea.P = P; ea.Q = Q; ea.ef = edge_fea; ea.M = b.M; ea.Fsum = b.Fsum;
     NB_TRY(launch_edge_fwd(ea, stream));
-    float* h_next = (l + 1 < Ln) ? bufs(l + 1).h0 : h_out;
-    float* x_next = (l + 1 < Ln) ? bufs(l + 1).x0 : x_out;
-    bool node_fused = false;
-#ifndef NB_EMU
-    node_fused = egno_node_fused(X);
-    if (node_fused) {   // node_net, node_v_net and the coordinate update in one pass over the rows (nb_egno_node.cuh)
-      NbEgnoNodeFwdArgs na;
-      memset(&na, 0, sizeof(na));
-      na.rows = (int)Nn; na.N = cfg->N; na.img = g_wimg.img[EGNO_WIMG_PER_LAYER * l + 2];
-      na.h = h1; na.M = b.M; na.b5 = params + L.n_b1; na.b6 = params + L.n_b2; na.bv1 = params + L.v_b1;
-      na.wv2 = params + L.v_w2; na.bv2 = params + L.v_b2; na.x = x1; na.v = v1; na.Fsum = b.Fsum;
-      na.U5 = saved ? b.U5 : nullptr; na.UV = saved ? b.UV : nullptr;   // inference: the pre-activations stay on chip
-      na.h_out = h_next; na.x_out = x_next;
-      NB_SET_SMEM(k_egno_node_fwd, NB_ENF_SMEM);
-      int pi = prof_begin(6, stream);
-      NB_LAUNCH_COUNTED(k_egno_node_fwd, (unsigned)imin(cdiv(Nn, NB_TILE), 2 * nb_num_sms()), NB_THREADS, NB_ENF_SMEM, stream, na);
-      prof_end(6, pi, stream);
-      NB_TRY(nb_check_launch("k_egno_node_fwd"));
-    }
-#endif
-    if (!node_fused) {
-      NbGemmArgs a = gemm_args((int)Nn);  // U5 = [h, M] W5^T + b5      (basic.py:183-185)
-      a.nsrc = 2;
-      a.src[0] = gsrc(h1, NB_H, 0, params + L.n_w1, 1, 2 * NB_H);
-      a.src[1] = gsrc(b.M, NB_H, 0, params + L.n_w1 + NB_H, 1, 2 * NB_H);
-      a.bias = params + L.n_b1; a.out_pre = b.U5;
-      NbGemmArgs u = gemm_args((int)Nn);  // UV = h Wv1^T + bv1         (node_v_net, pre-update h)
-      u.nsrc = 1; u.src[0] = gsrc(h1, NB_H, 0, params + L.v_w1, 1, NB_H);
-      u.bias = params + L.v_b1; u.out_pre = b.UV;
-      NbGemmArgs au[2] = {a, u};
-      NB_TRY(launch_gemm_batch(au, 2, stream));
-      NbGemmArgs c2 = gemm_args((int)Nn);  // h' = SiLU(U5) W6^T + b6  (no residual)
-      c2.nsrc = 1; c2.src[0] = gsrc(b.U5, NB_H, 1, params + L.n_w2, 1, NB_H);
-      c2.bias = params + L.n_b2; c2.out = h_next;
-      NB_TRY(launch_gemm(c2, stream));
-      NbXupdArgs xa;
-      memset(&xa, 0, sizeof(xa));
-      xa.rows = Nn; xa.N = cfg->N; xa.x = x1; xa.v = v1; xa.UV = b.UV; xa.w2 = params + L.v_w2; xa.b2 = params + L.v_b2;
-      xa.Fsum = b.Fsum; xa.x_out = x_next;
-      NB_LAUNCH_COUNTED(k_egno_xupd_fwd, (unsigned)imin(cdiv(Nn, 8), 8 * nb_num_sms()), 256, 0, stream, xa);
-      NB_TRY(nb_check_launch("k_egno_xupd_fwd"));
-    }
-    v_prev = v1;
+    const bool last = l + 1 == Ln;
+    NB_TRY(egno_node_fwd(X, l, b, h1, x1, b.v1, saved != nullptr, last ? h_out : bufs(l + 1).h0, last ? x_out : bufs(l + 1).x0));
+    v_prev = b.v1;
   }
-  cudaMemcpyAsync(v_out, v_prev, Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
+  cudaMemcpyAsync(v_out, v_prev, X.Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
   return nb_check_launch("nb_egno_forward");
 }
 
@@ -1304,21 +1573,143 @@ extern "C" int nb_egno_forward_ft(const NbEgnoConfig* cfg, const float* params, 
   return egno_forward(cfg, params, x, nodes, edge_fea, v, loc_mean, times, x_out, v_out, h_out, saved, workspace, stream);
 }
 
-// input-gradient workspace of nb_egno_backward_ex: the per-row edge-feature gradients of every layer launch
-// (n_layers * T * B*N(N-1) * in_edge_nf floats: each launch writes its own slice, no read-modify-write across layers),
-// then the embedding-output gradient summed over the T frames
-static inline int64_t egno_edge_rows(const NbEgnoConfig* c) { return (int64_t)c->B * c->N * (c->N - 1); }
-extern "C" int64_t nb_egno_input_grad_workspace_floats(const NbEgnoConfig* cfg) {
-  if (egno_validate(cfg) != NB_OK) return -1;
-  return align64((int64_t)cfg->n_layers * cfg->T * egno_edge_rows(cfg) * cfg->in_edge_nf) +
-         align64((int64_t)cfg->B * cfg->N * NB_H);
-}
-
 static int egno_backward(const NbEgnoConfig* cfg, const float* params, const float* nodes, const float* edge_fea,
                          const float* loc_mean, const EgnoTimes& times, const float* saved, const float* g_x_out,
                          const float* g_v_out, const float* g_h_out, float* grad_params, float* g_x_in, float* g_v_in,
                          float* g_nodes, float* g_edge_fea, float* g_loc_mean, float* g_t_out, float* g_t_in,
-                         float* workspace, float* input_grad_workspace, void* stream);
+                         float* workspace, float* input_grad_workspace, void* stream) {
+  NB_RANGE("nb_egno_backward");
+  EgnoCtx X;
+  NB_TRY(egno_ctx_init(&X, cfg, params, stream));
+  if (!saved) { nb_set_error("nb_egno_backward needs the saved buffer of a forward call"); return NB_ERR_INVALID; }
+  const int T = cfg->T, Ln = cfg->n_layers;
+  const int64_t Nn = X.Nn, Nn0 = X.Nn0;
+  // input gradients (single input frame only): per-row edge-feature gradients of every layer, summed at the end
+  const bool want_ef = g_edge_fea && cfg->in_edge_nf > 0;
+  if ((g_nodes || g_edge_fea || g_loc_mean) && X.fm.L > 1) {
+    nb_set_error("gradients w.r.t. nodes / edge_fea / loc_mean are implemented for num_inputs = 1 only");
+    return NB_ERR_INVALID;
+  }
+  if ((g_t_out || g_t_in) && !times.fout) {
+    nb_set_error("time gradients need floating-point times (nb_egno_backward_ft)");
+    return NB_ERR_INVALID;
+  }
+  if (g_t_in && X.fm.L == 1) {
+    nb_set_error("g_t_in needs num_inputs > 1 (a single input frame has no input times)");
+    return NB_ERR_INVALID;
+  }
+  if ((g_nodes || want_ef) && !input_grad_workspace) {
+    nb_set_error("nb_egno_backward_ex needs the input-gradient workspace (nb_egno_input_grad_workspace_floats)");
+    return NB_ERR_INVALID;
+  }
+  const EgnoInputGradWs iws = egno_input_grad_ws(cfg, input_grad_workspace);
+  const int64_t lf = align64(egno_layer_floats(Nn, Nn0));
+  EgnoBwdWs ws = egno_bwd_ws(cfg, workspace);
+  WimgGuard wimg_guard;
+  NB_TRY(egno_weight_images(X, ws.wimg));
+  DeferState D = {cfg->use_time_conv && egno_tconv_fused(X) && defer_available(), 0, ws.arena};
+  q_begin(ws.arena[0], NB_PARTIAL_FLOATS);
+  // deferred flushes: layer l writes set l & 1, its queued jobs read that set and the gh / spectral planes of the other
+  auto set_of = [&](int l) -> EgnoBwdSet& { return ws.set[D.on ? l & 1 : 0]; };
+  auto layer = [&](int l) { return egno_layer_bufs(const_cast<float*>(saved) + (int64_t)l * lf, Nn); };
+  cudaStream_t cst = (cudaStream_t)stream;
+
+  cudaMemsetAsync(grad_params, 0, X.lo.total * sizeof(float), cst);
+  // incoming gradients: gx must be writable (the edge backward accumulates into it)
+  int gxi = 0;
+  if (g_x_out) cudaMemcpyAsync(ws.gx[0], g_x_out, Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, cst);
+  else cudaMemsetAsync(ws.gx[0], 0, Nn * 3 * sizeof(float), cst);
+  const float* gv_in = g_v_out;
+  if (!gv_in) { cudaMemsetAsync(ws.gvA, 0, Nn * 3 * sizeof(float), cst); gv_in = ws.gvA; }
+  // the embedding layer's inputs (re-materialised for its weight gradient at the very end) depend on nothing but the
+  // call's inputs: with the second stream they are built there now, off the dependent chain
+  NbEmbedArgs emb_args;
+  if (D.on) NB_TRY(egno_embed_inputs(X, emb_args, nodes, times, ws.ttab, ws.P, ws.Q, side2_fork(stream)));
+  const float* gh_in = g_h_out;
+  if (!gh_in) {   // in the set "layer Ln" would have written
+    gh_in = set_of(Ln).gh;
+    cudaMemsetAsync(set_of(Ln).gh, 0, Nn * NB_H * sizeof(float), cst);
+  }
+
+  for (int l = Ln - 1; l >= 0; --l) {
+    EgnoBwdSet& S = set_of(l);
+    const EgnoLayerBufs b = layer(l);
+    const float* h1 = cfg->use_time_conv ? b.h1 : b.h0;
+    const float* x1 = cfg->use_time_conv ? b.x1 : b.x0;
+    float* gx = ws.gx[gxi];
+    // 1 + 2. coordinate update, node_v_net and node_net backwards
+    NB_TRY(egno_node_bwd(X, l, b, h1, gh_in, gx, gv_in, ws.gvB, S, ws, ws.ghA, grad_params));
+    // 3. edge tile backward (recompute from the saved P, Q)
+    {
+      NbEdgeBwdArgs ea;
+      memset(&ea, 0, sizeof(ea));
+      ea.g = egno_edge_geom(X);
+      ea.w = egno_edge_w(X, l);
+      ea.x = x1; ea.P = b.P; ea.Q = b.Q; ea.ef = edge_fea; ea.gM = ws.gM; ea.gFsum = ws.gFsum; ea.gP = S.gP; ea.gQ = S.gQ; ea.gx = gx;
+      if (want_ef) ea.gef = iws.gef_rows + (int64_t)l * iws.ef_slice;
+      const EgnoLayerOff& L = X.lo.L[l];
+      EdgeGradDst d;
+      d.w1 = L.e_w1; d.W2 = L.e_w2; d.b2 = L.e_b2; d.W3 = L.c_w1; d.b3 = L.c_b1; d.w4 = L.c_w2; d.b4 = L.c_b2;
+      d.ldw1 = X.lo.E; d.col_rad = 0; d.col_ef = 1 + 2 * NB_H; d.b_unused = 0;
+      NB_TRY(launch_edge_bwd(ea, grad_params, d, 0, stream));
+    }
+    // 4. pre-projection backward
+    NB_TRY(egno_pair_bwd(X, l, h1, S.gP, S.gQ, ws.ghA, grad_params));
+    // 5. temporal convolutions
+    if (cfg->use_time_conv) {
+      void* side = stream;
+      if (egno_tconv_fused(X)) {
+        // queued weight-gradient jobs read gh_in (= S.gh of the layer above), GU5, gP, ...: run them before S.gh is
+        // overwritten.  The spectral weight gradients of THIS layer are queued after the kernel that produces their
+        // operands (coef, gycoef) and run with the next flush, before those planes are overwritten again.
+        NB_TRY(defer_flush(D, stream));
+        // the 2-channel convolution's backward is independent of the 64-channel one: side stream, joined after it;
+        // its partial slice is reduced by the next flush (on the caller's stream, after the join)
+        side = side_fork(stream);
+      }
+      const float* v0 = l == 0 ? b.v0 : layer(l - 1).v1;
+      NB_TRY(egno_tcx_bwd(X, l, b, v0, loc_mean, gx, ws.gvB, ws.gx[gxi ^ 1], ws.gvA, g_loc_mean, grad_params, side));
+      gxi ^= 1;
+      gv_in = ws.gvA;
+      NB_TRY(egno_tconv_bwd(X, l, b, ws.ghA, S, ws, grad_params));
+      side_join(side, stream);
+      gh_in = S.gh;
+    } else {
+      NB_TRY(q_flush(stream));
+      // without the temporal conv gv1 must survive in gvB while the next layer writes its own gv1: swap roles (gh too)
+      gv_in = ws.gvB;
+      std::swap(ws.gvA, ws.gvB);
+      gh_in = ws.ghA;
+      std::swap(ws.ghA, S.gh);
+    }
+  }
+  // ---- embedding backward and the reduction of the T replicas of x, v
+  NB_TRY(egno_embed_bwd(X, emb_args, D.on, nodes, times, ws, gh_in, grad_params));
+  NB_TRY(defer_flush(D, stream));
+  const NbFrameMap& fm = X.fm;
+  if (g_x_in) NB_LAUNCH_COUNTED(k_sum_over_t, (unsigned)ew_grid(Nn0 * 3 * fm.L), 256, 0, stream, (const float*)ws.gx[gxi], g_x_in, (int)(Nn0 * 3), T, fm);
+  if (g_v_in) NB_LAUNCH_COUNTED(k_sum_over_t, (unsigned)ew_grid(Nn0 * 3 * fm.L), 256, 0, stream, gv_in, g_v_in, (int)(Nn0 * 3), T, fm);
+  if (g_nodes) {   // dL/dnodes = (sum_t dL/dh_emb[t]) W_emb[:, :in_node_nf]
+    NB_LAUNCH_COUNTED(k_sum_over_t, (unsigned)ew_grid(Nn0 * NB_H), 256, 0, stream, gh_in, iws.gh_sum, (int)(Nn0 * NB_H), T, fm);
+    NB_LAUNCH_COUNTED(k_embed_input_grad, (unsigned)ew_grid(Nn0 * cfg->in_node_nf), 256, 0, stream, (const float*)iws.gh_sum,
+                      params + X.lo.emb_w, X.lo.F, cfg->in_node_nf, Nn0, g_nodes);
+  }
+  if (want_ef)     // fixed-order sum over the n_layers * T slices of B*N(N-1) rows
+    NB_LAUNCH_COUNTED(k_sum_slices, (unsigned)ew_grid(egno_edge_rows(cfg) * cfg->in_edge_nf), 256, 0, stream,
+                      (const float*)iws.gef_rows, g_edge_fea, egno_edge_rows(cfg) * cfg->in_edge_nf, Ln * T);
+  if (g_loc_mean && !cfg->use_time_conv) cudaMemsetAsync(g_loc_mean, 0, Nn0 * 3 * sizeof(float), cst);
+  if (g_t_out || g_t_in) {   // dL/dtimes from the same gh_in as the embedding's weight gradient
+    if (cfg->time_emb_dim == 0) {   // the times are unused
+      if (g_t_out) cudaMemsetAsync(g_t_out, 0, (int64_t)cfg->B * T * sizeof(float), cst);
+    } else {
+      NB_LAUNCH_COUNTED(k_time_grad, (unsigned)cfg->B, NB_TGRAD_THREADS, 0, stream, emb_args, times.fout, times.fin, gh_in,
+                        params + X.lo.emb_w, X.lo.F, g_t_out, g_t_in);
+      NB_TRY(nb_check_launch("k_time_grad"));
+    }
+  }
+  defer_join(D, stream);
+  return nb_check_launch("nb_egno_backward");
+}
 
 extern "C" int nb_egno_backward(const NbEgnoConfig* cfg, const float* params, const float* nodes, const float* edge_fea,
                                 const float* loc_mean, const int64_t* timesteps_out, const int64_t* timesteps_in,
@@ -1349,404 +1740,6 @@ extern "C" int nb_egno_backward_ft(const NbEgnoConfig* cfg, const float* params,
   return egno_backward(cfg, params, nodes, edge_fea, loc_mean, times, saved, g_x_out, g_v_out, g_h_out, grad_params,
                        g_x_in, g_v_in, g_nodes, g_edge_fea, g_loc_mean, g_t_out, g_t_in, workspace, input_grad_workspace,
                        stream);
-}
-
-static int egno_backward(const NbEgnoConfig* cfg, const float* params, const float* nodes, const float* edge_fea,
-                         const float* loc_mean, const EgnoTimes& times, const float* saved, const float* g_x_out,
-                         const float* g_v_out, const float* g_h_out, float* grad_params, float* g_x_in, float* g_v_in,
-                         float* g_nodes, float* g_edge_fea, float* g_loc_mean, float* g_t_out, float* g_t_in,
-                         float* workspace, float* input_grad_workspace, void* stream) {
-  NB_RANGE("nb_egno_backward");
-  EgnoCtx X;
-  NB_TRY(egno_ctx_init(&X, cfg, params, stream));
-  if (!saved) { nb_set_error("nb_egno_backward needs the saved buffer of a forward call"); return NB_ERR_INVALID; }
-  const int T = cfg->T, Ln = cfg->n_layers, modes = cfg->num_modes;
-  const int64_t Nn = X.Nn, Nn0 = X.Nn0;
-  // input gradients (single input frame only): per-row edge-feature gradients of every layer, summed at the end
-  const bool want_ef = g_edge_fea && cfg->in_edge_nf > 0;
-  if ((g_nodes || g_edge_fea || g_loc_mean) && egno_L(cfg) > 1) {
-    nb_set_error("gradients w.r.t. nodes / edge_fea / loc_mean are implemented for num_inputs = 1 only");
-    return NB_ERR_INVALID;
-  }
-  if ((g_t_out || g_t_in) && !times.fout) {
-    nb_set_error("time gradients need floating-point times (nb_egno_backward_ft)");
-    return NB_ERR_INVALID;
-  }
-  if (g_t_in && egno_L(cfg) == 1) {
-    nb_set_error("g_t_in needs num_inputs > 1 (a single input frame has no input times)");
-    return NB_ERR_INVALID;
-  }
-  if ((g_nodes || want_ef) && !input_grad_workspace) {
-    nb_set_error("nb_egno_backward_ex needs the input-gradient workspace (nb_egno_input_grad_workspace_floats)");
-    return NB_ERR_INVALID;
-  }
-  const int64_t ef_slice = (int64_t)T * egno_edge_rows(cfg) * cfg->in_edge_nf;   // one layer launch
-  float* gef_rows = input_grad_workspace;
-  float* gh_sum = input_grad_workspace ? input_grad_workspace + align64(ef_slice * Ln) : nullptr;
-  const int64_t nh = align64(Nn * NB_H), n3 = align64(Nn * 3), cf = egno_coef_floats(cfg);
-  const int64_t lf = align64(egno_layer_floats(Nn, Nn0));
-  float* w = workspace;
-  WimgGuard wimg_guard;
-  NB_TRY(egno_weight_images(X, w));
-  w += wimg_floats(EGNO_WIMG_PER_LAYER * Ln);
-  float* ttab = w; w += egno_table_floats(cfg);
-  float* P = w; w += nh;
-  float* Q = w; w += nh;
-  float* coef = w; w += cf;
-  float* ycoef = w; w += cf;
-  float* gycoef = w; w += cf;
-  float* gcoef = w; w += cf;
-  float* ghA = w; w += nh;
-  float* ghB = w; w += nh;
-  float* GU5 = w; w += nh;
-  float* GUV = w; w += nh;
-  float* gM = w; w += nh;
-  float* gP = w; w += nh;
-  float* gQ = w; w += nh;
-  float* gxb[2]; gxb[0] = w; w += n3; gxb[1] = w; w += n3;
-  float* gvA = w; w += n3;
-  float* gvB = w; w += n3;
-  float* gFsum = w; w += n3;
-  float* arena0 = w; w += NB_PARTIAL_FLOATS;
-  // second set of everything a queued weight-gradient job reads and the next layer rewrites (defer_flush)
-  float* ghB_s[2]; ghB_s[0] = ghB; ghB_s[1] = w; w += nh;
-  float* GU5_s[2]; GU5_s[0] = GU5; GU5_s[1] = w; w += nh;
-  float* GUV_s[2]; GUV_s[0] = GUV; GUV_s[1] = w; w += nh;
-  float* gP_s[2]; gP_s[0] = gP; gP_s[1] = w; w += nh;
-  float* gQ_s[2]; gQ_s[0] = gQ; gQ_s[1] = w; w += nh;
-  float* coef_s[2]; coef_s[0] = coef; coef_s[1] = w; w += cf;
-  float* gycoef_s[2]; gycoef_s[0] = gycoef; gycoef_s[1] = w; w += cf;
-  DeferState D;
-  D.on = cfg->use_time_conv && egno_tconv_fused(X) && defer_available();
-  D.k = 0;
-  D.arena[0] = arena0; D.arena[1] = w;
-  q_begin(arena0, NB_PARTIAL_FLOATS);
-  cudaStream_t cst = (cudaStream_t)stream;
-
-  cudaMemsetAsync(grad_params, 0, X.lo.total * sizeof(float), cst);
-  // incoming gradients: gx must be writable (the edge backward accumulates into it)
-  int gxi = 0;
-  if (g_x_out) cudaMemcpyAsync(gxb[0], g_x_out, Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, cst);
-  else cudaMemsetAsync(gxb[0], 0, Nn * 3 * sizeof(float), cst);
-  const float* gv_in = g_v_out;
-  if (!gv_in) { cudaMemsetAsync(gvA, 0, Nn * 3 * sizeof(float), cst); gv_in = gvA; }
-  // the embedding layer's inputs (re-materialised for its weight gradient at the very end) depend on nothing but the
-  // call's inputs: with the second stream they are built there now, off the dependent chain
-  NbEmbedArgs emb_args;
-  bool embed_built = false;
-#ifndef NB_EMU
-  if (D.on) {
-    NbSide* sd = side_get();
-    cudaEventRecord(sd->fork2, cst);
-    cudaStreamWaitEvent(sd->s2, sd->fork2, 0);
-    NB_TRY(egno_embed_inputs(cfg, X.lo, emb_args, nodes, times, ttab, P, Q, (void*)sd->s2));
-    embed_built = true;
-  }
-#endif
-  const float* gh_in = g_h_out;
-  if (D.on) ghB = ghB_s[Ln & 1];   // the set "layer Ln" would have written
-  if (!gh_in) { cudaMemsetAsync(ghB, 0, Nn * NB_H * sizeof(float), cst); gh_in = ghB; }
-
-  for (int l = Ln - 1; l >= 0; --l) {
-    const EgnoLayerOff& L = X.lo.L[l];
-    if (D.on) {   // layer l writes set l & 1; its queued jobs read that set and the gh / spectral planes of set (l + 1) & 1
-      const int ps = l & 1;
-      ghB = ghB_s[ps]; GU5 = GU5_s[ps]; GUV = GUV_s[ps]; gP = gP_s[ps]; gQ = gQ_s[ps]; coef = coef_s[ps]; gycoef = gycoef_s[ps];
-    }
-    EgnoLayerBufs b = egno_layer_bufs(const_cast<float*>(saved) + (int64_t)l * lf, Nn);
-    const float* h1 = cfg->use_time_conv ? b.h1 : b.h0;
-    const float* x1 = cfg->use_time_conv ? b.x1 : b.x0;
-    const float* v0 = (l == 0) ? b.v0 : egno_layer_bufs(const_cast<float*>(saved) + (int64_t)(l - 1) * lf, Nn).v1;
-    float* gx = gxb[gxi];
-    bool node_fused = false;
-#ifndef NB_EMU
-    node_fused = egno_node_fused(X);
-    if (node_fused) {
-      // 1 + 2. coordinate update, node_v_net head and node_net backwards in one pass over the rows (nb_egno_node.cuh)
-      NbEgnoNodeBwdArgs na;
-      memset(&na, 0, sizeof(na));
-      na.rows = (int)Nn; na.N = cfg->N; na.img = g_wimg.img[EGNO_WIMG_PER_LAYER * l + 2];
-      na.gh = gh_in; na.U5 = b.U5; na.UV = b.UV; na.wv2 = params + L.v_w2; na.bv2 = params + L.v_b2;
-      na.gx = gx; na.gv = gv_in; na.v = b.v1; na.Fsum = b.Fsum; na.gv_out = gvB; na.gFsum = gFsum;
-      na.GU5 = GU5; na.GUV = GUV; na.gh1 = ghA; na.gM = gM;
-      const int grid = imin(cdiv(Nn, NB_TILE), 2 * nb_num_sms());
-      float* partial = q_alloc((int64_t)grid * 65, stream);
-      if (!partial) { nb_set_error("partial-sum workspace too small"); return NB_ERR_INVALID; }
-      na.partial = partial;
-      NB_SET_SMEM(k_egno_node_bwd, NB_ENB_SMEM);
-      int pi = prof_begin(7, stream);
-      NB_LAUNCH_COUNTED(k_egno_node_bwd, (unsigned)grid, NB_THREADS, NB_ENB_SMEM, stream, na);
-      prof_end(7, pi, stream);
-      NB_TRY(nb_check_launch("k_egno_node_bwd"));
-      NbFinArgs f;
-      memset(&f, 0, sizeof(f));
-      f.partial = partial; f.nparts = grid; f.plen = 65; f.dst = grad_params; f.nseg = 2;
-      f.seg[0] = fseg(0, NB_H, NB_H, L.v_w2, 0, 1);
-      f.seg[1] = fseg(NB_H, 1, 1, L.v_b2, 0, 0);
-      NB_TRY(launch_finalize(f, stream));
-      NB_TRY(wgrad_to((int)Nn, 1, wpair(gh_in, b.U5, 1), wpair(nullptr, nullptr), grad_params, L.n_w2, NB_H, 1,
-                      L.n_b2, 0, stream));
-      NB_TRY(wgrad_to((int)Nn, 1, wpair(GU5, h1), wpair(nullptr, nullptr), grad_params, L.n_w1, 2 * NB_H, 1,
-                      L.n_b1, 0, stream));
-      NB_TRY(wgrad_to((int)Nn, 1, wpair(GU5, b.M), wpair(nullptr, nullptr), grad_params, L.n_w1 + NB_H,
-                      2 * NB_H, 1, -1, 0, stream));
-      NB_TRY(wgrad_to((int)Nn, 1, wpair(GUV, h1), wpair(nullptr, nullptr), grad_params, L.v_w1, NB_H, 1,
-                      L.v_b1, 0, stream));
-    }
-#endif
-    // 1. x' = x + s v + clamp(mean f): gv1, gFsum, dL/dUV, and the 64->1 head of node_v_net
-    if (!node_fused) {
-      NbXupdArgs xa;
-      memset(&xa, 0, sizeof(xa));
-      xa.rows = Nn; xa.N = cfg->N; xa.v = b.v1; xa.UV = b.UV; xa.w2 = params + L.v_w2; xa.b2 = params + L.v_b2;
-      xa.Fsum = b.Fsum; xa.gx = gx; xa.gv = gv_in; xa.gv_out = gvB; xa.gFsum = gFsum; xa.GUV = GUV;
-      int grid = imin(cdiv(Nn, 8), 4 * nb_num_sms());
-      float* partial = q_alloc((int64_t)grid * 65, stream);
-      if (!partial) { nb_set_error("partial-sum workspace too small"); return NB_ERR_INVALID; }
-      xa.partial = partial;
-      NB_LAUNCH_COUNTED(k_egno_xupd_bwd, (unsigned)grid, 256, 0, stream, xa);
-      NB_TRY(nb_check_launch("k_egno_xupd_bwd"));
-      NbFinArgs f;
-      memset(&f, 0, sizeof(f));
-      f.partial = partial; f.nparts = grid; f.plen = 65; f.dst = grad_params; f.nseg = 2;
-      f.seg[0] = fseg(0, NB_H, NB_H, L.v_w2, 0, 1);
-      f.seg[1] = fseg(NB_H, 1, 1, L.v_b2, 0, 0);
-      NB_TRY(launch_finalize(f, stream));
-    }
-    // 2. node_net backward
-    if (!node_fused) {
-      NbGemmArgs a = gemm_args((int)Nn);  // GU5 = (gh W6) * SiLU'(U5)
-      a.nsrc = 1; a.src[0] = gsrc(gh_in, NB_H, 0, params + L.n_w2, NB_H, 1);
-      a.epi = NB_EPI_MUL_DSILU; a.U = b.U5; a.out = GU5;
-      NB_TRY(launch_gemm(a, stream));
-      NB_TRY(wgrad_to((int)Nn, 1, wpair(gh_in, b.U5, 1), wpair(nullptr, nullptr), grad_params, L.n_w2, NB_H, 1,
-                      L.n_b2, 0, stream));
-      NbGemmArgs g1 = gemm_args((int)Nn);  // gh1 = GU5 W5[:, :64] + GUV Wv1
-      g1.nsrc = 2;
-      g1.src[0] = gsrc(GU5, NB_H, 0, params + L.n_w1, 2 * NB_H, 1);
-      g1.src[1] = gsrc(GUV, NB_H, 0, params + L.v_w1, NB_H, 1);
-      g1.out = ghA;
-      NbGemmArgs g2 = gemm_args((int)Nn);  // gM = GU5 W5[:, 64:]
-      g2.nsrc = 1; g2.src[0] = gsrc(GU5, NB_H, 0, params + L.n_w1 + NB_H, 2 * NB_H, 1);
-      g2.out = gM;
-      NbGemmArgs g12[2] = {g1, g2};
-      NB_TRY(launch_gemm_batch(g12, 2, stream));
-      NB_TRY(wgrad_to((int)Nn, 1, wpair(GU5, h1), wpair(nullptr, nullptr), grad_params, L.n_w1, 2 * NB_H, 1,
-                      L.n_b1, 0, stream));
-      NB_TRY(wgrad_to((int)Nn, 1, wpair(GU5, b.M), wpair(nullptr, nullptr), grad_params, L.n_w1 + NB_H,
-                      2 * NB_H, 1, -1, 0, stream));
-      NB_TRY(wgrad_to((int)Nn, 1, wpair(GUV, h1), wpair(nullptr, nullptr), grad_params, L.v_w1, NB_H, 1,
-                      L.v_b1, 0, stream));
-    }
-    // 3. edge tile backward (recompute from the saved P, Q)
-    {
-      NbEdgeBwdArgs ea;
-      memset(&ea, 0, sizeof(ea));
-      ea.g = edge_geom(T * cfg->B, cfg->B, cfg->N, cfg->in_edge_nf, 0);
-      egno_geom_frames(cfg, ea.g);
-      ea.w = egno_edge_w(X, l);
-      ea.x = x1; ea.P = b.P; ea.Q = b.Q; ea.ef = edge_fea; ea.gM = gM; ea.gFsum = gFsum; ea.gP = gP; ea.gQ = gQ; ea.gx = gx;
-      if (want_ef) ea.gef = gef_rows + (int64_t)l * ef_slice;
-      EdgeGradDst d;
-      d.w1 = L.e_w1; d.W2 = L.e_w2; d.b2 = L.e_b2; d.W3 = L.c_w1; d.b3 = L.c_b1; d.w4 = L.c_w2; d.b4 = L.c_b2;
-      d.ldw1 = X.lo.E; d.col_rad = 0; d.col_ef = 1 + 2 * NB_H; d.b_unused = 0;
-      NB_TRY(launch_edge_bwd(ea, grad_params, d, 0, stream));
-    }
-    // 4. pre-projection backward: gh1 += gP W1[:, h_row] + gQ W1[:, h_col]
-    {
-#ifndef NB_EMU
-      if (egno_node_fused(X)) {
-        NbEgnoPairArgs pa;
-        memset(&pa, 0, sizeof(pa));
-        pa.rows = (int)Nn; pa.img = g_wimg.img[EGNO_WIMG_PER_LAYER * l]; pa.A0 = gP; pa.A1 = gQ; pa.O0 = ghA;
-        NB_SET_SMEM(k_egno_pair<false>, NB_EPR_SMEM);
-        int pi = prof_begin(2, stream);
-        NB_LAUNCH_COUNTED(k_egno_pair<false>, (unsigned)imin(cdiv(Nn, NB_TILE), 2 * nb_num_sms()), NB_THREADS, NB_EPR_SMEM, stream, pa);
-        prof_end(2, pi, stream);
-        NB_TRY(nb_check_launch("k_egno_pair"));
-      } else
-#endif
-      {
-      NbGemmArgs a = gemm_args((int)Nn);
-      a.nsrc = 2;
-      a.src[0] = gsrc(gP, NB_H, 0, params + L.e_w1 + 1, X.lo.E, 1);
-      a.src[1] = gsrc(gQ, NB_H, 0, params + L.e_w1 + 1 + NB_H, X.lo.E, 1);
-      a.out = ghA; a.accumulate = 1;
-      NB_TRY(launch_gemm(a, stream));
-      }
-      NB_TRY(wgrad_to((int)Nn, 1, wpair(gP, h1), wpair(nullptr, nullptr), grad_params, L.e_w1 + 1, X.lo.E, 1,
-                      L.e_b1, 0, stream));
-      NB_TRY(wgrad_to((int)Nn, 1, wpair(gQ, h1), wpair(nullptr, nullptr), grad_params, L.e_w1 + 1 + NB_H,
-                      X.lo.E, 1, -1, 0, stream));
-    }
-    // 5. temporal convolutions
-    if (cfg->use_time_conv) {
-      float* gx0 = gxb[gxi ^ 1];
-      void* side = stream;
-      if (egno_tconv_fused(X)) {
-        // queued weight-gradient jobs read gh_in (= ghB of the layer above), GU5, gP, ...: run them before ghB is
-        // overwritten.  The spectral weight gradients of THIS layer are queued after the kernel that produces their
-        // operands (coef, gycoef) and run with the next flush, before those planes are overwritten again.
-        NB_TRY(defer_flush(D, stream));
-        // the 2-channel convolution's backward is independent of the 64-channel one: side stream, joined after it;
-        // its partial slice is reduced by the next flush (on the caller's stream, after the join)
-        side = side_fork(stream);
-      }
-      {
-        NbTcxArgs t;
-        memset(&t, 0, sizeof(t));
-        t.tw = X.tw; t.n3 = (int)(Nn0 * 3); t.x0 = b.x0; t.v0 = v0; t.mean = loc_mean; t.W = params + L.tcx;
-      { const NbFrameMap fmx = egno_frame_map(cfg); for (int tt = 0; tt < NB_MAX_T; ++tt) t.tmap[tt] = fmx.m[tt]; }
-        t.gx1 = gx; t.gv1 = gvB; t.gx0 = gx0; t.gv0 = gvA;
-        int grid = imin(cdiv(Nn0 * 3, 256), 2 * nb_num_sms());
-        float* partial = q_alloc((int64_t)grid * 2 * 2 * modes * 2, stream);
-        if (!partial) { nb_set_error("partial-sum workspace too small"); return NB_ERR_INVALID; }
-        t.partial = partial;
-        NB_LAUNCH_COUNTED(k_tcx_bwd, (unsigned)grid, 256, 0, side, t);
-        NB_TRY(nb_check_launch("k_tcx_bwd"));
-        if (g_loc_mean) {   // same stream, right behind k_tcx_bwd: both planes are final there
-          NB_LAUNCH_COUNTED(k_loc_mean_grad, (unsigned)ew_grid(Nn0 * 3), 256, 0, side, (const float*)gx, (const float*)gx0,
-                            g_loc_mean, (int)(Nn0 * 3), T, l == Ln - 1 ? 0 : 1);
-          NB_TRY(nb_check_launch("k_loc_mean_grad"));
-        }
-        NbFinArgs f;
-        memset(&f, 0, sizeof(f));
-        int nw = 2 * 2 * modes * 2;
-        f.partial = partial; f.nparts = grid; f.plen = nw; f.dst = grad_params; f.nseg = 1;
-        f.seg[0] = fseg(0, nw, nw, L.tcx, 0, 1);
-        NB_TRY(launch_finalize(f, stream));
-      }
-      gxi ^= 1;
-      gv_in = gvA;
-      if (egno_tconv_fused(X)) {
-        NbTconvArgs tc = tconv_args(X, l);
-        tc.x = b.h0; tc.gout = ghA; tc.gx = ghB; tc.coef = coef; tc.gycoef = gycoef; tc.mask = b.tmask;
-        int pi = prof_begin(4, stream);
-        if (T <= 10) {
-          NB_SET_SMEM(k_tconv_bwd<10>, NB_TCONV_BWD_SMEM);
-          NB_LAUNCH_COUNTED(k_tconv_bwd<10>, (unsigned)tconv_grid(X, 2), 256, NB_TCONV_BWD_SMEM, stream, tc);
-        } else {
-          NB_SET_SMEM(k_tconv_bwd<NB_MAX_T>, NB_TCONV_BWD_SMEM);
-          NB_LAUNCH_COUNTED(k_tconv_bwd<NB_MAX_T>, (unsigned)tconv_grid(X, 2), 256, NB_TCONV_BWD_SMEM, stream, tc);
-        }
-        prof_end(4, pi, stream);
-        NB_TRY(nb_check_launch("k_tconv_bwd"));
-        side_join(side, stream);
-        const int64_t plane = Nn0 * NB_H;
-        const int64_t tk = (int64_t)modes * 2, tn = (int64_t)NB_H * modes * 2;
-        for (int m = 0; m < modes; ++m) {
-          int ci = nb_coef_index(X.tw, m);
-          const float *C = coef + ci * plane, *S = coef + (ci + 1) * plane;
-          const float *gPm = gycoef + ci * plane, *gQm = gycoef + (ci + 1) * plane;
-          const int64_t wr_off = L.tc + m * 2, wi_off = L.tc + m * 2 + 1;
-          if (m == 0 || m == X.tw.nyq) {
-            NB_TRY(wgrad_to((int)Nn0, 1, wpair(C, gPm), wpair(nullptr, nullptr), grad_params, wr_off, tn, tk, -1, 0, stream));
-          } else {
-            NB_TRY(wgrad_to((int)Nn0, 2, wpair(C, gPm), wpair(S, gQm, 0, -1.f), grad_params, wr_off, tn, tk, -1, 0, stream));
-            NB_TRY(wgrad_to((int)Nn0, 2, wpair(S, gPm), wpair(C, gQm), grad_params, wi_off, tn, tk, -1, 0, stream));
-          }
-        }
-      } else
-      {
-        NbDftArgs d = dft_args(X);
-        d.x = b.h0; d.coef = coef;
-        NB_LAUNCH_COUNTED(k_dft_fwd, (unsigned)ew_grid(Nn0 * 16), 256, 0, stream, d);
-        NB_TRY(nb_check_launch("k_dft_fwd"));
-        NB_TRY(egno_tc_mix(X, l, coef, ycoef));
-        d.ycoef = ycoef; d.gout = ghA; d.gycoef = gycoef;
-        NB_LAUNCH_COUNTED(k_idft_bwd, (unsigned)ew_grid(Nn0 * 16), 256, 0, stream, d);
-        NB_TRY(nb_check_launch("k_idft_bwd"));
-        const float* W = params + L.tc;
-        const int64_t plane = Nn0 * NB_H;
-        const int64_t tk = (int64_t)modes * 2, tn = (int64_t)NB_H * modes * 2;  // B[k=o][n=i] = W[i][o][m][c]
-        NbGemmArgs gj[2 * NB_MAX_T];
-        int ngj = 0;
-        for (int m = 0; m < modes; ++m) {
-          int ci = nb_coef_index(X.tw, m);
-          const float *Wr = W + m * 2, *Wi = W + m * 2 + 1;
-          const float *C = coef + ci * plane, *S = coef + (ci + 1) * plane;
-          const float *gPm = gycoef + ci * plane, *gQm = gycoef + (ci + 1) * plane;
-          const int64_t wr_off = L.tc + m * 2, wi_off = L.tc + m * 2 + 1;
-          if (m == 0 || m == X.tw.nyq) {
-            NbGemmArgs a = gemm_args((int)Nn0);  // gC = gP Wr^T
-            a.nsrc = 1; a.src[0] = gsrc(gPm, NB_H, 0, Wr, tk, tn);
-            a.out = gcoef + ci * plane;
-            gj[ngj++] = a;
-            NB_TRY(wgrad_to((int)Nn0, 1, wpair(C, gPm), wpair(nullptr, nullptr), grad_params, wr_off, tn, tk,
-                            -1, 0, stream));
-          } else {
-            NbGemmArgs a = gemm_args((int)Nn0);  // gC = gP Wr^T + gQ Wi^T
-            a.nsrc = 2;
-            a.src[0] = gsrc(gPm, NB_H, 0, Wr, tk, tn);
-            a.src[1] = gsrc(gQm, NB_H, 0, Wi, tk, tn);
-            a.out = gcoef + ci * plane;
-            gj[ngj++] = a;
-            NbGemmArgs s2 = gemm_args((int)Nn0);  // gS = gP Wi^T - gQ Wr^T
-            s2.nsrc = 2;
-            s2.src[0] = gsrc(gPm, NB_H, 0, Wi, tk, tn);
-            s2.src[1] = gsrc(gQm, NB_H, 0, Wr, tk, tn, -1.f);
-            s2.out = gcoef + (ci + 1) * plane;
-            gj[ngj++] = s2;
-            // dWr[i][o] = sum C_i gP_o - S_i gQ_o ; dWi[i][o] = sum S_i gP_o + C_i gQ_o
-            NB_TRY(wgrad_to((int)Nn0, 2, wpair(C, gPm), wpair(S, gQm, 0, -1.f), grad_params, wr_off, tn, tk,
-                            -1, 0, stream));
-            NB_TRY(wgrad_to((int)Nn0, 2, wpair(S, gPm), wpair(C, gQm), grad_params, wi_off, tn, tk, -1, 0,
-                            stream));
-          }
-        }
-        NB_TRY(launch_gemm_batch(gj, ngj, stream));
-        // queued weight-gradient jobs read gh_in / GU5 / gP / coefficients: run them before ghB is overwritten
-        NB_TRY(q_flush(stream));
-        d.gcoef = gcoef; d.gx = ghB;
-        NB_LAUNCH_COUNTED(k_dft_bwd, (unsigned)ew_grid(Nn0 * 16), 256, 0, stream, d);
-        NB_TRY(nb_check_launch("k_dft_bwd"));
-      }
-      gh_in = ghB;
-    } else {
-      NB_TRY(q_flush(stream));
-      gv_in = gvB;
-      // without the temporal conv gv1 must survive in gvB while the next layer writes its own gv1: swap roles
-      float* tmp = gvA; gvA = gvB; gvB = tmp;
-      gh_in = ghA;
-      float* t2 = ghA; ghA = ghB; ghB = t2;
-    }
-  }
-  // ---- embedding backward and the reduction of the T replicas of x, v
-  {
-    // dW_emb = gh^T [nodes | time embeddings], db_emb = column sums of gh: the inputs are re-materialised 64 wide
-    // (scratch: P, Q, free by now) and reduced by the weight-gradient kernel; columns >= F are not written.
-    if (!embed_built) NB_TRY(egno_embed_inputs(cfg, X.lo, emb_args, nodes, times, ttab, P, Q, stream));
-    const int F = X.lo.F;
-    NB_TRY(wgrad_to((int)Nn, 1, wpair(gh_in, P), wpair(nullptr, nullptr), grad_params, X.lo.emb_w, F, 1, X.lo.emb_b, 0,
-                    stream, F < NB_H ? F : NB_H));
-    if (F > NB_H)
-      NB_TRY(wgrad_to((int)Nn, 1, wpair(gh_in, Q), wpair(nullptr, nullptr), grad_params, X.lo.emb_w + NB_H, F, 1, -1, 0,
-                      stream, F - NB_H));
-    NB_TRY(defer_flush(D, stream));
-  }
-  const NbFrameMap fm = egno_frame_map(cfg);
-  if (g_x_in) NB_LAUNCH_COUNTED(k_sum_over_t, (unsigned)ew_grid(Nn0 * 3 * fm.L), 256, 0, stream, (const float*)gxb[gxi], g_x_in, (int)(Nn0 * 3), T, fm);
-  if (g_v_in) NB_LAUNCH_COUNTED(k_sum_over_t, (unsigned)ew_grid(Nn0 * 3 * fm.L), 256, 0, stream, gv_in, g_v_in, (int)(Nn0 * 3), T, fm);
-  if (g_nodes) {   // dL/dnodes = (sum_t dL/dh_emb[t]) W_emb[:, :in_node_nf]
-    NB_LAUNCH_COUNTED(k_sum_over_t, (unsigned)ew_grid(Nn0 * NB_H), 256, 0, stream, gh_in, gh_sum, (int)(Nn0 * NB_H), T, fm);
-    NB_LAUNCH_COUNTED(k_embed_input_grad, (unsigned)ew_grid(Nn0 * cfg->in_node_nf), 256, 0, stream, (const float*)gh_sum,
-                      params + X.lo.emb_w, X.lo.F, cfg->in_node_nf, Nn0, g_nodes);
-  }
-  if (want_ef)     // fixed-order sum over the n_layers * T slices of B*N(N-1) rows
-    NB_LAUNCH_COUNTED(k_sum_slices, (unsigned)ew_grid(egno_edge_rows(cfg) * cfg->in_edge_nf), 256, 0, stream,
-                      (const float*)gef_rows, g_edge_fea, egno_edge_rows(cfg) * cfg->in_edge_nf, Ln * T);
-  if (g_loc_mean && !cfg->use_time_conv) cudaMemsetAsync(g_loc_mean, 0, Nn0 * 3 * sizeof(float), cst);
-  if (g_t_out || g_t_in) {   // dL/dtimes from the same gh_in as the embedding's weight gradient
-    if (cfg->time_emb_dim == 0) {   // the times are unused
-      if (g_t_out) cudaMemsetAsync(g_t_out, 0, (int64_t)cfg->B * T * sizeof(float), cst);
-    } else {
-      NB_LAUNCH_COUNTED(k_time_grad, (unsigned)cfg->B, NB_TGRAD_THREADS, 0, stream, emb_args, times.fout, times.fin, gh_in,
-                        params + X.lo.emb_w, X.lo.F, g_t_out, g_t_in);
-      NB_TRY(nb_check_launch("k_time_grad"));
-    }
-  }
-  defer_join(D, stream);
-  return nb_check_launch("nb_egno_backward");
 }
 
 // ============================================================================= SEGNO
@@ -1813,27 +1806,86 @@ extern "C" int64_t nb_segno_saved_floats(const NbSegnoConfig* cfg) {
   if (segno_validate(cfg) != NB_OK) return -1;
   return segno_iter_floats((int64_t)cfg->B * cfg->N) * cfg->T;
 }
-extern "C" int64_t nb_segno_workspace_floats(const NbSegnoConfig* cfg, int mode) {
-  if (segno_validate(cfg) != NB_OK) return -1;
-  if (mode < 0 || mode > 2) { nb_set_error("workspace mode must be 0 (inference), 1 (backward) or 2 (training forward)"); return -1; }
-  int64_t Nn = (int64_t)cfg->B * cfg->N;
-  int64_t nh = align64(Nn * NB_H), n3 = align64(Nn * 3);
-  const int64_t wi = wimg_floats(SEGNO_WIMG);
-  if (mode == NB_WS_FORWARD_TRAIN) return wi + 2 * nh /*P,Q*/ + 3 * n3 /*Fsum, v ping-pong*/;
-  if (mode == NB_WS_FORWARD_INFER) return wi + 2 * nh + 3 * n3 + 2 * segno_iter_floats(Nn);
-  // backward: gh / GU5 / gP / gQ are kept PER sub-step, so that the weight-gradient reductions of all sub-steps run as a few
-  // large batches at the end of the sweep instead of one small batch (+ finalize) per sub-step
-  return wi + 2 * (int64_t)cfg->T * nh /*P_k, Q_k*/ + nh /*gM*/ + (int64_t)(cfg->T + 1) * nh /*gh_k*/ +
-         3 * (int64_t)cfg->T * nh /*GU5_k gP_k gQ_k*/ + 4 * n3 + SEGNO_PARTIAL_FLOATS;
-}
-
 struct SegnoCtx {
   const NbSegnoConfig* c;
   SegnoLayout lo;
   int64_t Nn;
+  float inv_T, cw;   // the integrator's step 1 / T and coords_weight
   const float* params;
   void* st;
 };
+
+static int segno_ctx_init(SegnoCtx* X, const NbSegnoConfig* cfg, const float* params, void* st) {
+  NB_TRY(segno_validate(cfg));
+  X->c = cfg; segno_layout(cfg, &X->lo); X->Nn = (int64_t)cfg->B * cfg->N; X->params = params; X->st = st;
+  X->inv_T = (float)(1.0 / (double)cfg->T); X->cw = cfg->coords_weight;
+  return NB_OK;
+}
+// the buffers sub-step k saved in the forward
+static SegnoIterBufs segno_saved(const SegnoCtx& X, const float* saved, int k) {
+  return segno_iter_bufs(const_cast<float*>(saved) + (int64_t)k * segno_iter_floats(X.Nn), X.Nn);
+}
+
+// SEGNO forward; inference (nothing saved) adds two ping-pong sub-step sets
+struct SegnoFwdWs {
+  float *wimg, *P, *Q, *Fsum, *v[2], *infer;
+  int64_t total;
+};
+static SegnoFwdWs segno_fwd_ws(const NbSegnoConfig* c, bool infer, float* base) {
+  const int64_t Nn = (int64_t)c->B * c->N, nh = align64(Nn * NB_H), n3 = align64(Nn * 3);
+  Carve w = {base, 0};
+  SegnoFwdWs s;
+  s.wimg = w.take(wimg_floats(SEGNO_WIMG));
+  s.P = w.take(nh); s.Q = w.take(nh); s.Fsum = w.take(n3); s.v[0] = w.take(n3); s.v[1] = w.take(n3);
+  s.infer = infer ? w.take(2 * segno_iter_floats(Nn)) : nullptr;
+  s.total = w.used;
+  return s;
+}
+
+// SEGNO backward: P, Q, gh, GU5, gP, gQ are kept PER sub-step (nh floats apart), so that the weight-gradient
+// reductions of all sub-steps run as a few large batches instead of one small batch (+ finalize) per sub-step.  gh has
+// T + 1 slots: the gradient entering sub-step k sits at slot k + 1, slot k receives its output
+struct SegnoBwdWs {
+  float *wimg, *P, *Q, *gM, *gh, *GU5, *gP, *gQ, *gx, *gv[2], *gFsum, *partial;
+  int64_t nh, total;
+};
+static SegnoBwdWs segno_bwd_ws(const NbSegnoConfig* c, float* base) {
+  const int64_t Nn = (int64_t)c->B * c->N, T = c->T, nh = align64(Nn * NB_H), n3 = align64(Nn * 3);
+  Carve w = {base, 0};
+  SegnoBwdWs s;
+  s.nh = nh;
+  s.wimg = w.take(wimg_floats(SEGNO_WIMG));
+  s.P = w.take(T * nh); s.Q = w.take(T * nh); s.gM = w.take(nh); s.gh = w.take((T + 1) * nh);
+  s.GU5 = w.take(T * nh); s.gP = w.take(T * nh); s.gQ = w.take(T * nh);
+  s.gx = w.take(n3); s.gv[0] = w.take(n3); s.gv[1] = w.take(n3); s.gFsum = w.take(n3);
+  s.partial = w.take(SEGNO_PARTIAL_FLOATS);
+  s.total = w.used;
+  return s;
+}
+
+// input-gradient workspace of nb_segno_backward_ex: the per-row edge-attribute gradients of every sub-step launch (a
+// slice of B*N(N-1) * in_edge_nf floats each), summed in a fixed order at the end
+struct SegnoInputGradWs { float* gef_rows; int64_t ef_slice, total; };
+static SegnoInputGradWs segno_input_grad_ws(const NbSegnoConfig* c, float* base) {
+  Carve w = {base, 0};
+  SegnoInputGradWs s;
+  s.ef_slice = (int64_t)c->B * c->N * (c->N - 1) * c->in_edge_nf;
+  s.gef_rows = w.take(align64(c->T * s.ef_slice));
+  s.total = w.used;
+  return s;
+}
+
+extern "C" int64_t nb_segno_workspace_floats(const NbSegnoConfig* cfg, int mode) {
+  if (segno_validate(cfg) != NB_OK) return -1;
+  if (mode < 0 || mode > 2) { nb_set_error("workspace mode must be 0 (inference), 1 (backward) or 2 (training forward)"); return -1; }
+  if (mode == NB_WS_BACKWARD) return segno_bwd_ws(cfg, nullptr).total;
+  return segno_fwd_ws(cfg, mode == NB_WS_FORWARD_INFER, nullptr).total;
+}
+
+extern "C" int64_t nb_segno_input_grad_workspace_floats(const NbSegnoConfig* cfg) {
+  if (segno_validate(cfg) != NB_OK) return -1;
+  return segno_input_grad_ws(cfg, nullptr).total;
+}
 
 static int segno_weight_images(const SegnoCtx& X, float* scratch) {
   const float* W[SEGNO_WIMG] = {X.params + X.lo.e_w1, X.params + X.lo.e_w1 + NB_H, X.params + X.lo.n_w1, X.params + X.lo.n_w1 + NB_H,
@@ -1873,109 +1925,215 @@ static void segno_embed_args(const SegnoCtx& X, const float* his, NbEmbedArgs* e
   e->nodes = his; e->tsteps = nullptr; e->W = X.params + X.lo.emb_w; e->bias = X.params + X.lo.emb_b;
 }
 
+// ---- SEGNO stages (see the EGNO stages)
+
+// h = his W_emb^T + b_emb (model.py:73)
+static int segno_embed_fwd(const SegnoCtx& X, const float* his, float* h) {
+  NbEmbedArgs e;
+  segno_embed_args(X, his, &e);
+  e.out = h;
+  const size_t smem = ((size_t)e.F0 * NB_H + 4 * e.F0) * sizeof(float);
+  NB_LAUNCH_COUNTED(k_embed_fwd, (unsigned)imin(cdiv(X.Nn, 4), 8 * nb_num_sms()), 256, smem, X.st, e);
+  return nb_check_launch("k_embed_fwd");
+}
+
+static int embed_bwd_grid(int64_t rows) { return imin(cdiv(rows, 32), 2 * nb_num_sms()); }
+// grad[embedding.weight | embedding.bias] = dL/dW, dL/db of h = his W^T + b over eb.e.Nn0 rows (overwritten)
+static int segno_embed_bwd(NbEmbedBwdArgs& eb, const SegnoLayout& lo, float* grad, void* st) {
+  const int F = eb.e.F0, grid = embed_bwd_grid(eb.e.Nn0), plen = NB_H * F + NB_H;
+  NB_TRY(q_partial(&eb.partial, (int64_t)grid * plen, st));
+  const size_t smem = (32 * (size_t)F + 32 * NB_H) * sizeof(float);
+  NB_LAUNCH_COUNTED(k_embed_bwd, (unsigned)grid, 256, smem, st, eb);
+  NB_TRY(nb_check_launch("k_embed_bwd"));
+  NB_TRY(q_finalize(eb.partial, grid, plen, grad, 0,
+                    {fseg(0, NB_H * F, NB_H * F, lo.emb_w, 0, 1), fseg(NB_H * F, NB_H, NB_H, lo.emb_b, 0, 1)}, st));
+  return q_flush(st);
+}
+
+// the whole forward as one kernel, node state in shared memory (nb_segno_fused.cuh), for the tcgen05 variants and
+// whole-graph selector units (N <= 27); otherwise *done = false and the call runs one sub-step at a time
+static int segno_fused_fwd(const SegnoCtx& X, const SegnoFwdWs& ws, const float* his, const float* x, const float* v,
+                           const float* edge_attr, float* x_out, float* h_out, float* v_out, float* saved, bool* done) {
+  *done = false;
+#ifndef NB_EMU
+  const NbSegnoConfig* cfg = X.c;
+  NbEdgeGeom fg = edge_geom(cfg->B, cfg->B, cfg->N, cfg->in_edge_nf, 1);
+  if (!(g_segno_fused && g_edge_impl == 2 && g_node_impl == 1 && sel_geom(fg) && !fg.blk)) return NB_OK;
+  *done = true;
+  // embedding into scratch (the fused kernel writes h_k of every sub-step into `saved` itself)
+  if (!cfg->h_given) NB_TRY(segno_embed_fwd(X, his, ws.P));
+  const float* params = X.params;
+  NbSegnoFusedArgs fa;
+  memset(&fa, 0, sizeof(fa));
+  fa.g = fg; fa.T = cfg->T; fa.recurrent = cfg->recurrent; fa.inv_T = X.inv_T; fa.cw = X.cw;
+  fa.W1 = params + X.lo.e_w1; fa.b1 = params + X.lo.e_b1; fa.ldw1 = X.lo.E; fa.col_rad = 2 * NB_H; fa.col_ef = 2 * NB_H + 1;
+  fa.W2 = params + X.lo.e_w2; fa.b2 = params + X.lo.e_b2; fa.W3 = params + X.lo.c_w1; fa.b3 = params + X.lo.c_b1;
+  fa.w4 = params + X.lo.c_w2; fa.b4 = params + X.lo.c_b2;
+  fa.W5 = params + X.lo.n_w1; fa.b5 = params + X.lo.n_b1; fa.W6 = params + X.lo.n_w2; fa.b6 = params + X.lo.n_b2;
+  fa.h_in = cfg->h_given ? his : ws.P; fa.x_in = x; fa.v_in = v; fa.ef = edge_attr;
+  fa.h_out = h_out; fa.x_out = x_out; fa.v_out = v_out; fa.saved = saved; fa.iter_stride = segno_iter_floats(X.Nn);
+  const size_t fsm = NB_SEGNO_FUSED_SMEM(fg.G * fg.EPG);
+  NB_SET_SMEM(k_segno_fused_fwd, fsm);
+  int pi = prof_begin(5, X.st);
+  NB_LAUNCH_COUNTED(k_segno_fused_fwd, (unsigned)imin(fg.n_units, nb_num_sms()), NB_SB_THREADS, fsm, X.st, fa);
+  prof_end(5, pi, X.st);
+  return nb_check_launch("k_segno_fused_fwd");
+#else
+  return NB_OK;
+#endif
+}
+
+// one sub-step (gcl.py:76-94, model.py:95-102): edge layer, integrator, node_mlp
+static int segno_step_fwd(const SegnoCtx& X, const SegnoFwdWs& ws, const SegnoIterBufs& b, const float* v,
+                          const float* edge_attr, float* h_next, float* x_next, float* v_next) {
+  const NbSegnoConfig* cfg = X.c;
+  const float* params = X.params;
+  NB_TRY(segno_pq(X, b.h, ws.P, ws.Q));
+  NbEdgeFwdArgs ea;
+  ea.g = edge_geom(cfg->B, cfg->B, cfg->N, cfg->in_edge_nf, 1);
+  ea.w = segno_edge_w(X);
+  ea.x = b.x; ea.P = ws.P; ea.Q = ws.Q; ea.ef = edge_attr; ea.M = b.M; ea.Fsum = ws.Fsum;
+  NB_TRY(launch_edge_fwd(ea, X.st));
+  NbIntegArgs ia;
+  memset(&ia, 0, sizeof(ia));
+  ia.n3 = X.Nn * 3; ia.N = cfg->N; ia.inv_T = X.inv_T; ia.cw = X.cw;
+  ia.x = b.x; ia.v = v; ia.Fsum = ws.Fsum; ia.x_out = x_next; ia.v_out = v_next;
+  NB_LAUNCH_COUNTED(k_segno_integ_fwd, (unsigned)ew_grid(X.Nn * 3), 256, 0, X.st, ia);
+  NB_TRY(nb_check_launch("k_segno_integ_fwd"));
+  NbGemmArgs a = gemm_args((int)X.Nn);  // U5 = [h, M] W5^T + b5      (gcl.py:89-92)
+  a.nsrc = 2;
+  a.src[0] = gsrc(b.h, NB_H, 0, params + X.lo.n_w1, 1, 2 * NB_H);
+  a.src[1] = gsrc(b.M, NB_H, 0, params + X.lo.n_w1 + NB_H, 1, 2 * NB_H);
+  a.bias = params + X.lo.n_b1; a.out_pre = b.U5;
+  NB_TRY(launch_gemm(a, X.st));
+  NbGemmArgs c2 = gemm_args((int)X.Nn);  // h' = h + SiLU(U5) W6^T + b6   (recurrent, gcl.py:93-94)
+  c2.nsrc = 1; c2.src[0] = gsrc(b.U5, NB_H, 1, params + X.lo.n_w2, 1, NB_H);
+  c2.bias = params + X.lo.n_b2; c2.out = h_next;
+  if (cfg->recurrent) c2.R = b.h;
+  return launch_gemm(c2, X.st);
+}
+
 extern "C" int nb_segno_forward(const NbSegnoConfig* cfg, const float* params, const float* his, const float* x,
                                 const float* v, const float* edge_attr, float* x_out, float* h_out, float* v_out,
                                 float* saved, float* workspace, void* stream) {
   NB_RANGE("nb_segno_forward");
-  NB_TRY(segno_validate(cfg));
   SegnoCtx X;
-  X.c = cfg; segno_layout(cfg, &X.lo); X.Nn = (int64_t)cfg->B * cfg->N; X.params = params; X.st = stream;
-  const int64_t Nn = X.Nn, nh = align64(Nn * NB_H), n3 = align64(Nn * 3), itf = segno_iter_floats(Nn);
+  NB_TRY(segno_ctx_init(&X, cfg, params, stream));
+  const int64_t Nn = X.Nn, itf = segno_iter_floats(Nn);
   const int T = cfg->T;
+  const SegnoFwdWs ws = segno_fwd_ws(cfg, !saved, workspace);
   WimgGuard wimg_guard;
-  float* P = workspace + wimg_floats(SEGNO_WIMG);
-  float* Q = P + nh;
-  float* Fsum = Q + nh;
-  float* vb[2] = {Fsum + n3, Fsum + 2 * n3};
-  float* infer = Fsum + 3 * n3;
-  auto bufs = [&](int k) { return segno_iter_bufs(saved ? saved + (int64_t)k * itf : infer + (int64_t)(k & 1) * itf, Nn); };
+  bool fused = false;
+  NB_TRY(segno_fused_fwd(X, ws, his, x, v, edge_attr, x_out, h_out, v_out, saved, &fused));
+  if (fused) return NB_OK;
+  NB_TRY(segno_weight_images(X, ws.wimg));
+  // training keeps every sub-step's buffers in `saved`; inference alternates two sets in the workspace
+  auto bufs = [&](int k) { return segno_iter_bufs(saved ? saved + (int64_t)k * itf : ws.infer + (int64_t)(k & 1) * itf, Nn); };
   cudaStream_t cst = (cudaStream_t)stream;
-
-#ifndef NB_EMU
-  {
-    NbEdgeGeom fg = edge_geom(cfg->B, cfg->B, cfg->N, cfg->in_edge_nf, 1);
-    if (g_segno_fused && g_edge_impl == 2 && g_node_impl == 1 && sel_geom(fg) && !fg.blk) {
-      // embedding into scratch (the fused kernel writes h_k of every sub-step into `saved` itself)
-      if (!cfg->h_given) {
-        NbEmbedArgs e;
-        segno_embed_args(X, his, &e);
-        e.out = P;
-        const size_t esm = ((size_t)e.F0 * NB_H + 4 * e.F0) * sizeof(float);
-        NB_LAUNCH_COUNTED(k_embed_fwd, (unsigned)imin(cdiv(Nn, 4), 8 * nb_num_sms()), 256, esm, stream, e);
-        NB_TRY(nb_check_launch("k_embed_fwd"));
-      }
-      NbSegnoFusedArgs fa;
-      memset(&fa, 0, sizeof(fa));
-      fa.g = fg; fa.T = T; fa.recurrent = cfg->recurrent; fa.inv_T = (float)(1.0 / (double)T); fa.cw = cfg->coords_weight;
-      fa.W1 = params + X.lo.e_w1; fa.b1 = params + X.lo.e_b1; fa.ldw1 = X.lo.E; fa.col_rad = 2 * NB_H; fa.col_ef = 2 * NB_H + 1;
-      fa.W2 = params + X.lo.e_w2; fa.b2 = params + X.lo.e_b2; fa.W3 = params + X.lo.c_w1; fa.b3 = params + X.lo.c_b1;
-      fa.w4 = params + X.lo.c_w2; fa.b4 = params + X.lo.c_b2;
-      fa.W5 = params + X.lo.n_w1; fa.b5 = params + X.lo.n_b1; fa.W6 = params + X.lo.n_w2; fa.b6 = params + X.lo.n_b2;
-      fa.h_in = cfg->h_given ? his : P; fa.x_in = x; fa.v_in = v; fa.ef = edge_attr;
-      fa.h_out = h_out; fa.x_out = x_out; fa.v_out = v_out; fa.saved = saved; fa.iter_stride = itf;
-      const size_t fsm = NB_SEGNO_FUSED_SMEM(fg.G * fg.EPG);
-      NB_SET_SMEM(k_segno_fused_fwd, fsm);
-      int pi = prof_begin(5, stream);
-      NB_LAUNCH_COUNTED(k_segno_fused_fwd, (unsigned)imin(fg.n_units, nb_num_sms()), NB_SB_THREADS, fsm, stream, fa);
-      prof_end(5, pi, stream);
-      return nb_check_launch("k_segno_fused_fwd");
-    }
-  }
-#endif
-  NB_TRY(segno_weight_images(X, workspace));
-  SegnoIterBufs b0 = bufs(0);
-  {
-    if (cfg->h_given) {
-      cudaMemcpyAsync(b0.h, his, Nn * NB_H * sizeof(float), cudaMemcpyDeviceToDevice, cst);
-    } else {
-      NbEmbedArgs e;
-      segno_embed_args(X, his, &e);
-      e.out = b0.h;
-      const size_t smem = ((size_t)e.F0 * NB_H + 4 * e.F0) * sizeof(float);
-      NB_LAUNCH_COUNTED(k_embed_fwd, (unsigned)imin(cdiv(Nn, 4), 8 * nb_num_sms()), 256, smem, stream, e);
-      NB_TRY(nb_check_launch("k_embed_fwd"));
-    }
-    cudaMemcpyAsync(b0.x, x, Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, cst);
-  }
+  const SegnoIterBufs b0 = bufs(0);
+  if (cfg->h_given) cudaMemcpyAsync(b0.h, his, Nn * NB_H * sizeof(float), cudaMemcpyDeviceToDevice, cst);
+  else NB_TRY(segno_embed_fwd(X, his, b0.h));
+  cudaMemcpyAsync(b0.x, x, Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, cst);
   const float* vcur = v;
   for (int k = 0; k < T; ++k) {
-    SegnoIterBufs b = bufs(k);
-    float* h_next = (k + 1 < T) ? bufs(k + 1).h : h_out;
-    float* x_next = (k + 1 < T) ? bufs(k + 1).x : x_out;
-    float* v_next = (k + 1 < T) ? vb[k & 1] : v_out;
-    NB_TRY(segno_pq(X, b.h, P, Q));
-    NbEdgeFwdArgs ea;
-    ea.g = edge_geom(cfg->B, cfg->B, cfg->N, cfg->in_edge_nf, 1);
-    ea.w = segno_edge_w(X);
-    ea.x = b.x; ea.P = P; ea.Q = Q; ea.ef = edge_attr; ea.M = b.M; ea.Fsum = Fsum;
-    NB_TRY(launch_edge_fwd(ea, stream));
-    NbIntegArgs ia;
-    memset(&ia, 0, sizeof(ia));
-    ia.n3 = Nn * 3; ia.N = cfg->N; ia.inv_T = (float)(1.0 / (double)T); ia.cw = cfg->coords_weight;
-    ia.x = b.x; ia.v = vcur; ia.Fsum = Fsum; ia.x_out = x_next; ia.v_out = v_next;
-    NB_LAUNCH_COUNTED(k_segno_integ_fwd, (unsigned)ew_grid(Nn * 3), 256, 0, stream, ia);
-    NB_TRY(nb_check_launch("k_segno_integ_fwd"));
-    NbGemmArgs a = gemm_args((int)Nn);  // U5 = [h, M] W5^T + b5      (gcl.py:89-92)
-    a.nsrc = 2;
-    a.src[0] = gsrc(b.h, NB_H, 0, params + X.lo.n_w1, 1, 2 * NB_H);
-    a.src[1] = gsrc(b.M, NB_H, 0, params + X.lo.n_w1 + NB_H, 1, 2 * NB_H);
-    a.bias = params + X.lo.n_b1; a.out_pre = b.U5;
-    NB_TRY(launch_gemm(a, stream));
-    NbGemmArgs c2 = gemm_args((int)Nn);  // h' = h + SiLU(U5) W6^T + b6   (recurrent, gcl.py:93-94)
-    c2.nsrc = 1; c2.src[0] = gsrc(b.U5, NB_H, 1, params + X.lo.n_w2, 1, NB_H);
-    c2.bias = params + X.lo.n_b2; c2.out = h_next;
-    if (cfg->recurrent) c2.R = b.h;
-    NB_TRY(launch_gemm(c2, stream));
+    const bool last = k + 1 == T;
+    float* v_next = last ? v_out : ws.v[k & 1];
+    NB_TRY(segno_step_fwd(X, ws, bufs(k), vcur, edge_attr, last ? h_out : bufs(k + 1).h, last ? x_out : bufs(k + 1).x, v_next));
     vcur = v_next;
   }
   return nb_check_launch("nb_segno_forward");
 }
 
-// input-gradient workspace of nb_segno_backward_ex: the per-row edge-attribute gradients of every sub-step launch
-// (T * B*N(N-1) * in_edge_nf floats), summed in a fixed order at the end
-extern "C" int64_t nb_segno_input_grad_workspace_floats(const NbSegnoConfig* cfg) {
-  if (segno_validate(cfg) != NB_OK) return -1;
-  return align64((int64_t)cfg->T * cfg->B * cfg->N * (cfg->N - 1) * cfg->in_edge_nf);
+// The node-level chain between the edge sweeps of two sub-steps is ONE launch (k_segno_node_bwd) when the tcgen05 node
+// kernels and their weight images are in use; nb_set_segno_fused(0) runs it stepwise
+static bool segno_chain() {
+#ifndef NB_EMU
+  return g_segno_fused && g_node_impl == 1 && g_wimg.n == SEGNO_WIMG;
+#else
+  return false;
+#endif
+}
+// the chain launch: node_mlp and integrator backward of sub-step j after edge layer 1's h halves backwards of j + 1, or
+// (FIRST, j = T - 1) from the incoming g_h_out (null: zero)
+template <bool FIRST>
+static int segno_node_bwd(const SegnoCtx& X, const SegnoBwdWs& ws, const float* saved, int j, const float* g_h_out,
+                          const float* gv_in, float* gv_out) {
+#ifndef NB_EMU
+  const int64_t nh = ws.nh;
+  NbSegnoNodeBwdArgs na;
+  memset(&na, 0, sizeof(na));
+  na.rows = (int)X.Nn; na.recurrent = X.c->recurrent; na.img = g_wimg.img[0];
+  if (FIRST) {
+    na.gh_in = g_h_out;
+  } else {
+    na.gP = ws.gP + (int64_t)(j + 1) * nh; na.gQ = ws.gQ + (int64_t)(j + 1) * nh; na.gh_k = ws.gh + (int64_t)(j + 1) * nh;
+  }
+  na.U5 = segno_saved(X, saved, j).U5;
+  na.GU5 = ws.GU5 + (int64_t)j * nh; na.gh_km1 = ws.gh + (int64_t)j * nh; na.gM = ws.gM;
+  na.n3 = X.Nn * 3; na.N = X.c->N; na.inv_T = X.inv_T; na.cw = X.cw;
+  na.gx = ws.gx; na.gv = gv_in; na.gv_out = gv_out; na.gFsum = ws.gFsum;
+  NB_SET_SMEM(k_segno_node_bwd<FIRST>, NB_SNB_SMEM);
+  int pi = prof_begin(2, X.st);
+  NB_LAUNCH_COUNTED(k_segno_node_bwd<FIRST>, (unsigned)imin(cdiv(X.Nn, NB_TILE), nb_num_sms()), NB_THREADS, NB_SNB_SMEM, X.st, na);
+  prof_end(2, pi, X.st);
+  return nb_check_launch("k_segno_node_bwd");
+#else
+  nb_set_error("the host emulator runs SEGNO one sub-step at a time");
+  return NB_ERR_INVALID;
+#endif
+}
+// the stepwise node_mlp and integrator backward of sub-step k (gh_in: dL/dh entering it)
+static int segno_step_bwd(const SegnoCtx& X, const SegnoBwdWs& ws, const float* saved, int k, const float* gh_in,
+                          const float* gv_in, float* gv_out) {
+  const SegnoLayout& lo = X.lo;
+  const float* params = X.params;
+  float* GU5 = ws.GU5 + (int64_t)k * ws.nh;
+  NbGemmArgs a = gemm_args((int)X.Nn);  // GU5 = (gh W6) * SiLU'(U5)
+  a.nsrc = 1; a.src[0] = gsrc(gh_in, NB_H, 0, params + lo.n_w2, NB_H, 1);
+  a.epi = NB_EPI_MUL_DSILU; a.U = segno_saved(X, saved, k).U5; a.out = GU5;
+  NB_TRY(launch_gemm(a, X.st));
+  NbGemmArgs g1 = gemm_args((int)X.Nn);  // gh = GU5 W5[:, :64] (+ gh: residual)
+  g1.nsrc = 1; g1.src[0] = gsrc(GU5, NB_H, 0, params + lo.n_w1, 2 * NB_H, 1);
+  if (X.c->recurrent) g1.R = gh_in;
+  g1.out = ws.gh + (int64_t)k * ws.nh;
+  NbGemmArgs g2 = gemm_args((int)X.Nn);  // gM = GU5 W5[:, 64:]
+  g2.nsrc = 1; g2.src[0] = gsrc(GU5, NB_H, 0, params + lo.n_w1 + NB_H, 2 * NB_H, 1);
+  g2.out = ws.gM;
+  NbGemmArgs g12[2] = {g1, g2};
+  NB_TRY(launch_gemm_batch(g12, 2, X.st));
+  NbIntegArgs ia;   // integrator backward
+  memset(&ia, 0, sizeof(ia));
+  ia.n3 = X.Nn * 3; ia.N = X.c->N; ia.inv_T = X.inv_T; ia.cw = X.cw;
+  ia.gx = ws.gx; ia.gv = gv_in; ia.gx_out = ws.gx; ia.gv_out = gv_out; ia.gFsum = ws.gFsum;
+  NB_LAUNCH_COUNTED(k_segno_integ_bwd, (unsigned)ew_grid(X.Nn * 3), 256, 0, X.st, ia);
+  return nb_check_launch("k_segno_integ_bwd");
+}
+// weight gradients of the shared layers: ONE reduction per weight block over the rows of sub-steps [k0, k1) (the
+// operands of sub-step k sit k blocks apart: saved state at stride itf, the sweep's gradients at stride nh); queued on
+// `st`, every job accumulates onto grad
+static int segno_queue_wgrads(const SegnoCtx& X, const SegnoBwdWs& ws, const float* saved, const float* g_h_out, int k0,
+                              int k1, float* grad, void* st) {
+  const SegnoLayout& lo = X.lo;
+  const int64_t nh = ws.nh, itf = segno_iter_floats(X.Nn), Nn = X.Nn;
+  const int T = X.c->T;
+  const SegnoIterBufs b0 = segno_saved(X, saved, k0);
+  const int rows = (int)(Nn * (k1 - k0)), sr = (int)Nn;
+  const float* ghin0 = ws.gh + (int64_t)(k0 + 1) * nh;   // gh entering sub-step k = slot k + 1 ...
+  // ... except for the last sub-step when the caller supplied dL/dh_out: that one lives in the caller's buffer
+  if (g_h_out && k1 == T) {
+    if (k1 - 1 > k0) {
+      NB_TRY(wgrad_to((int)(Nn * (k1 - 1 - k0)), wpair_seg(ghin0, b0.U5, 1, sr, nh, itf), grad, lo.n_w2, NB_H, 1, lo.n_b2, 1, st));
+      NB_TRY(q_flush_wgrad(st));   // same destination as the job below: separate reduction batches
+      NB_TRY(q_flush_fin(st, false));
+    }
+    NB_TRY(wgrad_to((int)Nn, wpair(g_h_out, segno_saved(X, saved, T - 1).U5, 1), grad, lo.n_w2, NB_H, 1, lo.n_b2, 1, st));
+  } else {
+    NB_TRY(wgrad_to(rows, wpair_seg(ghin0, b0.U5, 1, sr, nh, itf), grad, lo.n_w2, NB_H, 1, lo.n_b2, 1, st));
+  }
+  NB_TRY(wgrad_to(rows, wpair_seg(ws.GU5 + (int64_t)k0 * nh, b0.h, 0, sr, nh, itf), grad, lo.n_w1, 2 * NB_H, 1, lo.n_b1, 1, st));
+  NB_TRY(wgrad_to(rows, wpair_seg(ws.GU5 + (int64_t)k0 * nh, b0.M, 0, sr, nh, itf), grad, lo.n_w1 + NB_H, 2 * NB_H, 1, -1, 1, st));
+  NB_TRY(wgrad_to(rows, wpair_seg(ws.gP + (int64_t)k0 * nh, b0.h, 0, sr, nh, itf), grad, lo.e_w1, lo.E, 1, lo.e_b1, 1, st));
+  return wgrad_to(rows, wpair_seg(ws.gQ + (int64_t)k0 * nh, b0.h, 0, sr, nh, itf), grad, lo.e_w1 + NB_H, lo.E, 1, -1, 1, st);
 }
 
 extern "C" int nb_segno_backward(const NbSegnoConfig* cfg, const float* params, const float* his,
@@ -1992,7 +2150,8 @@ extern "C" int nb_segno_backward_ex(const NbSegnoConfig* cfg, const float* param
                                     float* g_v_in, float* g_h_in, float* g_his, float* g_edge_attr, float* workspace,
                                     float* input_grad_workspace, void* stream) {
   NB_RANGE("nb_segno_backward");
-  NB_TRY(segno_validate(cfg));
+  SegnoCtx X;
+  NB_TRY(segno_ctx_init(&X, cfg, params, stream));
   if (!saved) { nb_set_error("nb_segno_backward needs the saved buffer of a forward call"); return NB_ERR_INVALID; }
   if (g_his && cfg->h_given) {
     nb_set_error("g_his is the gradient of the raw node features: with h_given = 1 the hidden state's gradient is g_h_in");
@@ -2003,252 +2162,115 @@ extern "C" int nb_segno_backward_ex(const NbSegnoConfig* cfg, const float* param
     nb_set_error("nb_segno_backward_ex needs the input-gradient workspace (nb_segno_input_grad_workspace_floats)");
     return NB_ERR_INVALID;
   }
-  const int64_t ef_slice = (int64_t)cfg->B * cfg->N * (cfg->N - 1) * cfg->in_edge_nf;   // one sub-step launch
-  SegnoCtx X;
-  X.c = cfg; segno_layout(cfg, &X.lo); X.Nn = (int64_t)cfg->B * cfg->N; X.params = params; X.st = stream;
   const SegnoLayout& lo = X.lo;
-  const int64_t Nn = X.Nn, nh = align64(Nn * NB_H), n3 = align64(Nn * 3), itf = segno_iter_floats(Nn);
+  const int64_t Nn = X.Nn;
   const int T = cfg->T;
-  float* w = workspace;
+  const SegnoBwdWs ws = segno_bwd_ws(cfg, workspace);
+  const SegnoInputGradWs iws = segno_input_grad_ws(cfg, input_grad_workspace);
+  const int64_t nh = ws.nh;
   WimgGuard wimg_guard;
-  NB_TRY(segno_weight_images(X, w));
-  w += wimg_floats(SEGNO_WIMG);
-  float* P_all = w; w += (int64_t)T * nh;   // first edge layer's per-node halves of EVERY sub-step: one GEMM launch over the
-  float* Q_all = w; w += (int64_t)T * nh;   // saved hidden states before the sweep instead of one small launch per sub-step
-  float* gM = w; w += nh;
-  float* gh_all = w; w += (int64_t)(T + 1) * nh;    // gh entering sub-step k at slot k + 1; slot k receives its output
-  float* GU5_all = w; w += (int64_t)T * nh;
-  float* gP_all = w; w += (int64_t)T * nh;
-  float* gQ_all = w; w += (int64_t)T * nh;
-  float* gx = w; w += n3;
-  float* gvb[2]; gvb[0] = w; w += n3; gvb[1] = w; w += n3;
-  float* gFsum = w; w += n3;
+  NB_TRY(segno_weight_images(X, ws.wimg));
   // the last quarter of the partial-sum scratch belongs to the deferred reductions (below); it is only ever touched on
   // the second stream, which is in order, so one arena serves every deferred flush
   const int64_t def_cap = SEGNO_PARTIAL_FLOATS / 4;
-  float* def_arena = w + (SEGNO_PARTIAL_FLOATS - def_cap);
-  q_begin(w, SEGNO_PARTIAL_FLOATS - def_cap);
+  float* def_arena = ws.partial + (SEGNO_PARTIAL_FLOATS - def_cap);
+  q_begin(ws.partial, SEGNO_PARTIAL_FLOATS - def_cap);
   cudaStream_t cst = (cudaStream_t)stream;
 
   cudaMemsetAsync(grad_params, 0, lo.total * sizeof(float), cst);
-  if (g_x_out) cudaMemcpyAsync(gx, g_x_out, Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, cst);
-  else cudaMemsetAsync(gx, 0, Nn * 3 * sizeof(float), cst);
-  const float* gv_in = g_v_out;
-  int gvi = 0;
-  const float* gh_in = g_h_out;
-  if (!gh_in) { cudaMemsetAsync(gh_all + (int64_t)T * nh, 0, Nn * NB_H * sizeof(float), cst); gh_in = gh_all + (int64_t)T * nh; }
+  if (g_x_out) cudaMemcpyAsync(ws.gx, g_x_out, Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, cst);
+  else cudaMemsetAsync(ws.gx, 0, Nn * 3 * sizeof(float), cst);
+  if (!g_h_out) cudaMemsetAsync(ws.gh + (int64_t)T * nh, 0, Nn * NB_H * sizeof(float), cst);
+  // dL/dh and dL/dv entering sub-step k's node_mlp / integrator backward, and the dL/dv leaving it (a ping-pong pair)
+  auto gh_in = [&](int k) { return k == T - 1 && g_h_out ? g_h_out : ws.gh + (int64_t)(k + 1) * nh; };
+  auto gv_out = [&](int k) { return ws.gv[(T - 1 - k) & 1]; };
+  auto gv_in = [&](int k) -> const float* { return k == T - 1 ? g_v_out : gv_out(k + 1); };
 
-  if (align64(Nn * NB_H) == Nn * NB_H) {
-    NB_TRY(segno_pq(X, segno_iter_bufs(const_cast<float*>(saved), Nn).h, P_all, Q_all, T, itf));
-  } else {   // row blocks of P_all / Q_all are padded: one launch per sub-step
-    for (int k = 0; k < T; ++k)
-      NB_TRY(segno_pq(X, segno_iter_bufs(const_cast<float*>(saved) + (int64_t)k * itf, Nn).h, P_all + (int64_t)k * nh, Q_all + (int64_t)k * nh));
+  // edge layer 1's per-node halves of EVERY sub-step: one GEMM launch over the saved hidden states before the sweep
+  // instead of one small launch per sub-step
+  if (nh == Nn * NB_H) {
+    NB_TRY(segno_pq(X, segno_saved(X, saved, 0).h, ws.P, ws.Q, T, segno_iter_floats(Nn)));
+  } else {   // row blocks of P / Q are padded: one launch per sub-step
+    for (int k = 0; k < T; ++k) NB_TRY(segno_pq(X, segno_saved(X, saved, k).h, ws.P + (int64_t)k * nh, ws.Q + (int64_t)k * nh));
   }
   EdgeGradDst ed;
   ed.w1 = lo.e_w1; ed.W2 = lo.e_w2; ed.b2 = lo.e_b2; ed.W3 = lo.c_w1; ed.b3 = lo.c_b1; ed.w4 = lo.c_w2; ed.b4 = lo.c_b2;
   ed.ldw1 = lo.E; ed.col_rad = 2 * NB_H; ed.col_ef = 2 * NB_H + 1; ed.b_unused = 0;
   float* run_base = nullptr;   // the edge kernels' per-CTA partial slices of consecutive sub-steps are contiguous:
   int run_parts = 0;           // one reduction over all of them after the sweep
-  // The node-level chain between the edge sweeps of sub-steps k and k - 1 (edge layer 1's h halves backwards, node_mlp
-  // backwards, integrator backwards) is ONE launch (k_segno_node_bwd) when the tcgen05 node kernels and their weight images
-  // are in use; the first sub-step of the sweep (k = T - 1) and the tail (k = 0) keep the separate launches.
-  bool chain = false;
-#ifndef NB_EMU
-  chain = g_segno_fused && g_node_impl == 1 && g_wimg.n == SEGNO_WIMG;   // nb_set_segno_fused(0): stepwise both ways
-#endif
-  // ---- weight gradients of the shared layers: ONE reduction per weight block over the rows of sub-steps [k0, k1) (the
-  // operands of sub-step k sit k blocks apart: saved state at stride itf, the sweep's gradients at stride nh); queued on
-  // `st`, every job accumulates onto grad_params
-  auto queue_wgrads = [&](int k0, int k1, void* st) -> int {
-    const SegnoIterBufs b0 = segno_iter_bufs(const_cast<float*>(saved) + (int64_t)k0 * itf, Nn);
-    const int rows = (int)(Nn * (k1 - k0)), sr = (int)Nn;
-    const float* ghin0 = gh_all + (int64_t)(k0 + 1) * nh;   // gh entering sub-step k = slot k + 1 ...
-    // ... except for the last sub-step when the caller supplied dL/dh_out: that one lives in the caller's buffer
-    if (g_h_out && k1 == T) {
-      if (k1 - 1 > k0) {
-        NB_TRY(wgrad_to((int)(Nn * (k1 - 1 - k0)), 1, wpair_seg(ghin0, b0.U5, 1, sr, nh, itf), wpair(nullptr, nullptr), grad_params, lo.n_w2,
-                        NB_H, 1, lo.n_b2, 1, st));
-        NB_TRY(q_flush_wgrad(st));   // same destination as the job below: separate reduction batches
-        NB_TRY(q_flush_fin(st, false));
-      }
-      const SegnoIterBufs bl = segno_iter_bufs(const_cast<float*>(saved) + (int64_t)(T - 1) * itf, Nn);
-      NB_TRY(wgrad_to((int)Nn, 1, wpair(g_h_out, bl.U5, 1), wpair(nullptr, nullptr), grad_params, lo.n_w2, NB_H, 1, lo.n_b2, 1, st));
-    } else {
-      NB_TRY(wgrad_to(rows, 1, wpair_seg(ghin0, b0.U5, 1, sr, nh, itf), wpair(nullptr, nullptr), grad_params, lo.n_w2, NB_H, 1,
-                      lo.n_b2, 1, st));
-    }
-    NB_TRY(wgrad_to(rows, 1, wpair_seg(GU5_all + (int64_t)k0 * nh, b0.h, 0, sr, nh, itf), wpair(nullptr, nullptr), grad_params, lo.n_w1,
-                    2 * NB_H, 1, lo.n_b1, 1, st));
-    NB_TRY(wgrad_to(rows, 1, wpair_seg(GU5_all + (int64_t)k0 * nh, b0.M, 0, sr, nh, itf), wpair(nullptr, nullptr), grad_params,
-                    lo.n_w1 + NB_H, 2 * NB_H, 1, -1, 1, st));
-    NB_TRY(wgrad_to(rows, 1, wpair_seg(gP_all + (int64_t)k0 * nh, b0.h, 0, sr, nh, itf), wpair(nullptr, nullptr), grad_params, lo.e_w1,
-                    lo.E, 1, lo.e_b1, 1, st));
-    NB_TRY(wgrad_to(rows, 1, wpair_seg(gQ_all + (int64_t)k0 * nh, b0.h, 0, sr, nh, itf), wpair(nullptr, nullptr), grad_params,
-                    lo.e_w1 + NB_H, lo.E, 1, -1, 1, st));
-    return NB_OK;
-  };
   // Deferred reductions.  A sweep leaves most of the GPU idle (the node chain runs 40 CTAs; the second half of every edge
   // launch 108 of 148), and the reductions above used to run after it, alone.  With the second stream (defer_available)
-  // the sub-steps the sweep has finished are reduced every NB_SEGNO_DEFER_CHUNK sub-steps underneath the rest of the
-  // sweep: their operands are per-sub-step buffers nobody rewrites, the partial slices live in their own arena, every
+  // the sub-steps the sweep has finished are reduced every DEFER_CHUNK sub-steps underneath the rest of the sweep:
+  // their operands are per-sub-step buffers nobody rewrites, the partial slices live in their own arena, every
   // reduction still has a fixed order.  The caller's stream joins before its own last reduction touches grad_params.
+  const bool chain = segno_chain();
   const int DEFER_CHUNK = 3;
   const bool defer = chain && defer_available();
   int k_hi = T;             // sub-steps [0, k_hi) still have to be reduced
   bool deferred_any = false;
-  bool head_done = false;   // the node_mlp / integrator backward of sub-step k already ran (inside the chain launch)
+  // the sweep: the last sub-step's node-level backward, then per sub-step k the edge backward and the node-level chain
+  // into sub-step k - 1 (one launch, or the stepwise GEMMs)
+  if (chain) NB_TRY(segno_node_bwd<true>(X, ws, saved, T - 1, g_h_out, gv_in(T - 1), gv_out(T - 1)));
+  else NB_TRY(segno_step_bwd(X, ws, saved, T - 1, gh_in(T - 1), gv_in(T - 1), gv_out(T - 1)));
   for (int k = T - 1; k >= 0; --k) {
-    SegnoIterBufs b = segno_iter_bufs(const_cast<float*>(saved) + (int64_t)k * itf, Nn);
-    float* gh_new = gh_all + (int64_t)k * nh;
-    float* GU5 = GU5_all + (int64_t)k * nh;
-    float* gP = gP_all + (int64_t)k * nh;
-    float* gQ = gQ_all + (int64_t)k * nh;
-#ifndef NB_EMU
-    if (!head_done && chain) {   // first sub-step of the sweep: the chain without its first product
-      NbSegnoNodeBwdArgs na;
-      memset(&na, 0, sizeof(na));
-      na.rows = (int)Nn; na.recurrent = cfg->recurrent; na.img = g_wimg.img[0];
-      na.gh_in = g_h_out; na.U5 = b.U5;      // g_h_out == null: dL/dh_out = 0
-      na.GU5 = GU5; na.gh_km1 = gh_new; na.gM = gM;
-      na.n3 = Nn * 3; na.N = cfg->N; na.inv_T = (float)(1.0 / (double)T); na.cw = cfg->coords_weight;
-      na.gx = gx; na.gv = gv_in; na.gv_out = gvb[gvi]; na.gFsum = gFsum;
-      NB_SET_SMEM(k_segno_node_bwd<true>, NB_SNB_SMEM);
-      int pi = prof_begin(2, stream);
-      NB_LAUNCH_COUNTED(k_segno_node_bwd<true>, (unsigned)imin(cdiv(Nn, NB_TILE), nb_num_sms()), NB_THREADS, NB_SNB_SMEM, stream, na);
-      prof_end(2, pi, stream);
-      NB_TRY(nb_check_launch("k_segno_node_bwd"));
-      gv_in = gvb[gvi];
-      gvi ^= 1;
-      head_done = true;
-    }
-#endif
-    if (!head_done) {
-    // node_mlp backward
-    NbGemmArgs a = gemm_args((int)Nn);  // GU5 = (gh W6) * SiLU'(U5)
-    a.nsrc = 1; a.src[0] = gsrc(gh_in, NB_H, 0, params + lo.n_w2, NB_H, 1);
-    a.epi = NB_EPI_MUL_DSILU; a.U = b.U5; a.out = GU5;
-    NB_TRY(launch_gemm(a, stream));
-    NbGemmArgs g1 = gemm_args((int)Nn);  // gh = GU5 W5[:, :64] (+ gh: residual)
-    g1.nsrc = 1; g1.src[0] = gsrc(GU5, NB_H, 0, params + lo.n_w1, 2 * NB_H, 1);
-    if (cfg->recurrent) g1.R = gh_in;
-    g1.out = gh_new;
-    NbGemmArgs g2 = gemm_args((int)Nn);  // gM = GU5 W5[:, 64:]
-    g2.nsrc = 1; g2.src[0] = gsrc(GU5, NB_H, 0, params + lo.n_w1 + NB_H, 2 * NB_H, 1);
-    g2.out = gM;
-    NbGemmArgs g12[2] = {g1, g2};
-    NB_TRY(launch_gemm_batch(g12, 2, stream));
-    // integrator backward
-    NbIntegArgs ia;
-    memset(&ia, 0, sizeof(ia));
-    ia.n3 = Nn * 3; ia.N = cfg->N; ia.inv_T = (float)(1.0 / (double)T); ia.cw = cfg->coords_weight;
-    ia.gx = gx; ia.gv = gv_in; ia.gx_out = gx; ia.gv_out = gvb[gvi]; ia.gFsum = gFsum;
-    NB_LAUNCH_COUNTED(k_segno_integ_bwd, (unsigned)ew_grid(Nn * 3), 256, 0, stream, ia);
-    NB_TRY(nb_check_launch("k_segno_integ_bwd"));
-    gv_in = gvb[gvi];
-    gvi ^= 1;
-    }
-    head_done = false;
-    // edge tile backward
     NbEdgeBwdArgs ea;
     memset(&ea, 0, sizeof(ea));
     ea.g = edge_geom(cfg->B, cfg->B, cfg->N, cfg->in_edge_nf, 1);
     ea.w = segno_edge_w(X);
-    ea.x = b.x; ea.P = P_all + (int64_t)k * nh; ea.Q = Q_all + (int64_t)k * nh; ea.ef = edge_attr; ea.gM = gM; ea.gFsum = gFsum; ea.gP = gP; ea.gQ = gQ; ea.gx = gx;
-    if (want_ef) ea.gef = input_grad_workspace + (int64_t)k * ef_slice;
+    ea.x = segno_saved(X, saved, k).x; ea.P = ws.P + (int64_t)k * nh; ea.Q = ws.Q + (int64_t)k * nh; ea.ef = edge_attr;
+    ea.gM = ws.gM; ea.gFsum = ws.gFsum; ea.gP = ws.gP + (int64_t)k * nh; ea.gQ = ws.gQ + (int64_t)k * nh; ea.gx = ws.gx;
+    if (want_ef) ea.gef = iws.gef_rows + (int64_t)k * iws.ef_slice;
     NB_TRY(launch_edge_bwd(ea, grad_params, ed, 1, stream, &run_base, &run_parts));
-#ifndef NB_EMU
     if (defer && k > 0 && k_hi - k >= DEFER_CHUNK) {   // sub-steps [k, k_hi): every operand is final once this launch is done
-      NbSide* sd = side_get();
-      cudaEventRecord(sd->fork2, cst);
-      cudaStreamWaitEvent(sd->s2, sd->fork2, 0);
+      void* s2 = side2_fork(stream);
       float* const sv_base = g_q.pbase;
       const int64_t sv_cap = g_q.pcap, sv_used = g_q.pused;
       g_q.pbase = def_arena; g_q.pcap = def_cap; g_q.pused = 0;
-      int rc = edge_bwd_finalize(run_base, run_parts, cfg->in_edge_nf, grad_params, ed, 1, (void*)sd->s2);
+      int rc = edge_bwd_finalize(run_base, run_parts, cfg->in_edge_nf, grad_params, ed, 1, s2);
       run_parts = 0;   // the next launch starts a new run right behind this one
-      if (rc == NB_OK) rc = queue_wgrads(k, k_hi, (void*)sd->s2);
-      if (rc == NB_OK) rc = q_flush((void*)sd->s2);
+      if (rc == NB_OK) rc = segno_queue_wgrads(X, ws, saved, g_h_out, k, k_hi, grad_params, s2);
+      if (rc == NB_OK) rc = q_flush(s2);
       g_q.pbase = sv_base; g_q.pcap = sv_cap; g_q.pused = sv_used;
       NB_TRY(rc);
-      cudaEventRecord(sd->done2[0], sd->s2);
+      side2_done(0);
       k_hi = k;
       deferred_any = true;
     }
     if (chain && k > 0) {
-      const SegnoIterBufs bm = segno_iter_bufs(const_cast<float*>(saved) + (int64_t)(k - 1) * itf, Nn);
-      NbSegnoNodeBwdArgs na;
-      memset(&na, 0, sizeof(na));
-      na.rows = (int)Nn; na.recurrent = cfg->recurrent; na.img = g_wimg.img[0];
-      na.gP = gP; na.gQ = gQ; na.gh_k = gh_new; na.U5 = bm.U5;
-      na.GU5 = GU5_all + (int64_t)(k - 1) * nh; na.gh_km1 = gh_all + (int64_t)(k - 1) * nh; na.gM = gM;
-      na.n3 = Nn * 3; na.N = cfg->N; na.inv_T = (float)(1.0 / (double)T); na.cw = cfg->coords_weight;
-      na.gx = gx; na.gv = gv_in; na.gv_out = gvb[gvi]; na.gFsum = gFsum;
-      NB_SET_SMEM(k_segno_node_bwd<false>, NB_SNB_SMEM);
-      int pi = prof_begin(2, stream);
-      NB_LAUNCH_COUNTED(k_segno_node_bwd<false>, (unsigned)imin(cdiv(Nn, NB_TILE), nb_num_sms()), NB_THREADS, NB_SNB_SMEM, stream, na);
-      prof_end(2, pi, stream);
-      NB_TRY(nb_check_launch("k_segno_node_bwd"));
-      gv_in = gvb[gvi];
-      gvi ^= 1;
-      gh_in = gh_new;
-      head_done = true;
-      continue;
+      NB_TRY(segno_node_bwd<false>(X, ws, saved, k - 1, nullptr, gv_in(k - 1), gv_out(k - 1)));
+    } else {
+      NbGemmArgs pa = gemm_args((int)Nn);  // gh_k += gP W1[:, h_row] + gQ W1[:, h_col]
+      pa.nsrc = 2;
+      pa.src[0] = gsrc(ws.gP + (int64_t)k * nh, NB_H, 0, params + lo.e_w1, lo.E, 1);
+      pa.src[1] = gsrc(ws.gQ + (int64_t)k * nh, NB_H, 0, params + lo.e_w1 + NB_H, lo.E, 1);
+      pa.out = ws.gh + (int64_t)k * nh; pa.accumulate = 1;
+      NB_TRY(launch_gemm(pa, stream));
+      if (k > 0) NB_TRY(segno_step_bwd(X, ws, saved, k - 1, gh_in(k - 1), gv_in(k - 1), gv_out(k - 1)));
     }
-#endif
-    NbGemmArgs pa = gemm_args((int)Nn);  // gh += gP W1[:, h_row] + gQ W1[:, h_col]
-    pa.nsrc = 2;
-    pa.src[0] = gsrc(gP, NB_H, 0, params + lo.e_w1, lo.E, 1);
-    pa.src[1] = gsrc(gQ, NB_H, 0, params + lo.e_w1 + NB_H, lo.E, 1);
-    pa.out = gh_new; pa.accumulate = 1;
-    NB_TRY(launch_gemm(pa, stream));
-    gh_in = gh_new;
   }
   // ---- what the deferred flushes have not taken: the remaining sub-steps' reductions on the caller's stream, after the
   // second stream's last finalisation (both accumulate onto grad_params)
-  {
-#ifndef NB_EMU
-    if (deferred_any) cudaStreamWaitEvent(cst, side_get()->done2[0], 0);
-#endif
-    if (run_parts > 0) NB_TRY(edge_bwd_finalize(run_base, run_parts, cfg->in_edge_nf, grad_params, ed, 1, stream));
-    NB_TRY(queue_wgrads(0, k_hi, stream));
-    NB_TRY(q_flush(stream));
-  }
+  if (deferred_any) side2_wait(stream, 0);
+  if (run_parts > 0) NB_TRY(edge_bwd_finalize(run_base, run_parts, cfg->in_edge_nf, grad_params, ed, 1, stream));
+  NB_TRY(segno_queue_wgrads(X, ws, saved, g_h_out, 0, k_hi, grad_params, stream));
+  NB_TRY(q_flush(stream));
   if (cfg->h_given) {
-    NB_TRY(q_flush(stream));
-    if (g_h_in) cudaMemcpyAsync(g_h_in, gh_in, Nn * NB_H * sizeof(float), cudaMemcpyDeviceToDevice, cst);
-  } else
-  {
+    if (g_h_in) cudaMemcpyAsync(g_h_in, ws.gh, Nn * NB_H * sizeof(float), cudaMemcpyDeviceToDevice, cst);
+  } else {
     NbEmbedBwdArgs eb;
     memset(&eb, 0, sizeof(eb));
     segno_embed_args(X, his, &eb.e);
-    eb.g = gh_in;
-    const int F = cfg->in_node_nf;
-    int grid = imin(cdiv(Nn, 32), 2 * nb_num_sms());
-    float* partial = q_alloc((int64_t)grid * (NB_H * F + NB_H), stream);
-    if (!partial) { nb_set_error("partial-sum workspace too small"); return NB_ERR_INVALID; }
-    eb.partial = partial;
-    const size_t smem = (32 * (size_t)F + 32 * NB_H) * sizeof(float);
-    NB_LAUNCH_COUNTED(k_embed_bwd, (unsigned)grid, 256, smem, stream, eb);
-    NB_TRY(nb_check_launch("k_embed_bwd"));
-    NbFinArgs f;
-    memset(&f, 0, sizeof(f));
-    f.partial = partial; f.nparts = grid; f.plen = NB_H * F + NB_H; f.dst = grad_params; f.nseg = 2;
-    f.seg[0] = fseg(0, NB_H * F, NB_H * F, lo.emb_w, 0, 1);
-    f.seg[1] = fseg(NB_H * F, NB_H, NB_H, lo.emb_b, 0, 1);
-    NB_TRY(launch_finalize(f, stream));
-    NB_TRY(q_flush(stream));
+    eb.g = ws.gh;   // dL/dh entering the first sub-step
+    NB_TRY(segno_embed_bwd(eb, lo, grad_params, stream));
     if (g_his)   // dL/dhis = dL/dh_emb W_emb
-      NB_LAUNCH_COUNTED(k_embed_input_grad, (unsigned)ew_grid(Nn * F), 256, 0, stream, gh_in, params + lo.emb_w, F, F, Nn,
-                        g_his);
+      NB_LAUNCH_COUNTED(k_embed_input_grad, (unsigned)ew_grid(Nn * cfg->in_node_nf), 256, 0, stream, ws.gh, params + lo.emb_w,
+                        cfg->in_node_nf, cfg->in_node_nf, Nn, g_his);
   }
   if (want_ef)     // fixed-order sum over the T sub-step slices
-    NB_LAUNCH_COUNTED(k_sum_slices, (unsigned)ew_grid(ef_slice), 256, 0, stream, (const float*)input_grad_workspace,
-                      g_edge_attr, ef_slice, T);
-  if (g_x_in) cudaMemcpyAsync(g_x_in, gx, Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, cst);
-  if (g_v_in) {
-    if (gv_in) cudaMemcpyAsync(g_v_in, gv_in, Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, cst);
-    else cudaMemsetAsync(g_v_in, 0, Nn * 3 * sizeof(float), cst);
-  }
+    NB_LAUNCH_COUNTED(k_sum_slices, (unsigned)ew_grid(iws.ef_slice), 256, 0, stream, (const float*)iws.gef_rows,
+                      g_edge_attr, iws.ef_slice, T);
+  if (g_x_in) cudaMemcpyAsync(g_x_in, ws.gx, Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, cst);
+  if (g_v_in) cudaMemcpyAsync(g_v_in, gv_out(0), Nn * 3 * sizeof(float), cudaMemcpyDeviceToDevice, cst);
   return nb_check_launch("nb_segno_backward");
 }
 
@@ -2259,19 +2281,12 @@ extern "C" int nb_segno_backward_ex(const NbSegnoConfig* cfg, const float* param
 extern "C" int nb_segno_embed_forward(const NbSegnoConfig* cfg, const float* params, int64_t rows, const float* his, float* h,
                                       void* stream) {
   NB_RANGE("nb_segno_embed_forward");
-  NB_TRY(segno_validate(cfg));
+  SegnoCtx X;
+  NB_TRY(segno_ctx_init(&X, cfg, params, stream));
   if (rows < 1 || rows > 2000000000LL || !params || !his || !h) { nb_set_error("nb_segno_embed_forward: bad rows / null pointer"); return NB_ERR_INVALID; }
-  SegnoLayout lo;
-  segno_layout(cfg, &lo);
-  NbEmbedArgs e;
-  memset(&e, 0, sizeof(e));
-  e.T = 1; e.Nn0 = (int)rows; e.B = 1; e.F0 = cfg->in_node_nf; e.D = 0;
-  e.nodes = his; e.W = params + lo.emb_w; e.bias = params + lo.emb_b; e.out = h;
-  const size_t esm = ((size_t)e.F0 * NB_H + 4 * e.F0) * sizeof(float);
-  NB_LAUNCH_COUNTED(k_embed_fwd, (unsigned)imin(cdiv(rows, 4), 8 * nb_num_sms()), 256, esm, stream, e);
-  return nb_check_launch("k_embed_fwd");
+  X.Nn = rows;
+  return segno_embed_fwd(X, his, h);
 }
-static int embed_bwd_grid(int64_t rows) { return imin(cdiv(rows, 32), 2 * nb_num_sms()); }
 extern "C" int64_t nb_segno_embed_backward_workspace_floats(const NbSegnoConfig* cfg, int64_t rows) {
   if (!cfg || rows < 1) return -1;
   return (int64_t)embed_bwd_grid(rows) * (NB_H * cfg->in_node_nf + NB_H) + 64;
@@ -2288,21 +2303,8 @@ extern "C" int nb_segno_embed_backward(const NbSegnoConfig* cfg, int64_t rows, c
   memset(&eb, 0, sizeof(eb));
   eb.e.T = 1; eb.e.Nn0 = (int)rows; eb.e.B = 1; eb.e.F0 = cfg->in_node_nf; eb.e.D = 0; eb.e.nodes = his;
   eb.g = g_h;
-  const int F = cfg->in_node_nf, grid = embed_bwd_grid(rows);
   q_begin(workspace, nb_segno_embed_backward_workspace_floats(cfg, rows));
-  float* partial = q_alloc((int64_t)grid * (NB_H * F + NB_H), stream);
-  if (!partial) { nb_set_error("partial-sum workspace too small"); return NB_ERR_INVALID; }
-  eb.partial = partial;
-  const size_t smem = (32 * (size_t)F + 32 * NB_H) * sizeof(float);
-  NB_LAUNCH_COUNTED(k_embed_bwd, (unsigned)grid, 256, smem, stream, eb);
-  NB_TRY(nb_check_launch("k_embed_bwd"));
-  NbFinArgs f;
-  memset(&f, 0, sizeof(f));
-  f.partial = partial; f.nparts = grid; f.plen = NB_H * F + NB_H; f.dst = grad_params; f.nseg = 2;
-  f.seg[0] = fseg(0, NB_H * F, NB_H * F, lo.emb_w, 0, 1);
-  f.seg[1] = fseg(NB_H * F, NB_H, NB_H, lo.emb_b, 0, 1);
-  NB_TRY(launch_finalize(f, stream));
-  return q_flush(stream);
+  return segno_embed_bwd(eb, lo, grad_params, stream);
 }
 
 static int merge_check(int32_t mode, int64_t n, int32_t L, int32_t frame) {
@@ -2362,17 +2364,12 @@ extern "C" int nb_segno_merge_backward(int32_t mode, int64_t n, int32_t L, int32
   const int grid = mode == NB_MERGE_ATTN ? merge_bwd_grid(n) : imin(cdiv(n, 8), 8 * nb_num_sms());
   if (mode == NB_MERGE_ATTN) {
     q_begin(workspace, nb_segno_merge_backward_workspace_floats(n));
-    a.partial = q_alloc((int64_t)grid * NB_AT_PLEN, stream);
-    if (!a.partial) { nb_set_error("partial-sum workspace too small"); return NB_ERR_INVALID; }
+    NB_TRY(q_partial(&a.partial, (int64_t)grid * NB_AT_PLEN, stream));
   }
   NB_LAUNCH_COUNTED(k_segno_merge_bwd, (unsigned)grid, 256, NB_MERGE_SMEM, stream, a);
   NB_TRY(nb_check_launch("k_segno_merge_bwd"));
   if (mode != NB_MERGE_ATTN) return NB_OK;
-  NbFinArgs f;
-  memset(&f, 0, sizeof(f));
-  f.partial = a.partial; f.nparts = grid; f.plen = NB_AT_PLEN; f.dst = g_attn; f.nseg = 1; f.accumulate = accumulate ? 1 : 0;
-  f.seg[0] = fseg(0, NB_AT_PLEN, NB_AT_PLEN, 0, 0, 1);
-  NB_TRY(launch_finalize(f, stream));
+  NB_TRY(q_finalize(a.partial, grid, NB_AT_PLEN, g_attn, accumulate ? 1 : 0, {fseg(0, NB_AT_PLEN, NB_AT_PLEN, 0, 0, 1)}, stream));
   return q_flush(stream);
 }
 // dst[0:n] += src[0:n]: the shared parameters' gradients of the integration segments

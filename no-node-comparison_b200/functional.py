@@ -180,52 +180,25 @@ class EgnoFunction(torch.autograd.Function):
         gx_in = torch.empty(in_shape, device=dev, dtype=torch.float32)
         gv_in = torch.empty(in_shape, device=dev, dtype=torch.float32)
         ws = torch.empty(lib.nb_egno_workspace_floats(ctypes.byref(cfg), 1), device=dev, dtype=torch.float32)
-        want_nodes, want_ef, want_lm = ctx.needs_input_grad[4], ctx.needs_input_grad[5], ctx.needs_input_grad[7]
-        g_nodes = g_ef = g_lm = None
-        if tsteps.is_floating_point():
-            return EgnoFunction._backward_ft(ctx, lib, cfg, flat, nodes, edge_fea, loc_mean, tsteps, tsteps_in, saved,
-                                             gx_out, gv_out, gh_out, grad_flat, gx_in, gv_in, ws)
-        if want_nodes or want_ef or want_lm:
-            # per-shard input gradients: under data parallelism nothing beyond the parameter bucket is reduced
-            g_nodes = torch.empty_like(nodes) if want_nodes else None
-            g_ef = torch.empty_like(edge_fea) if want_ef else None
-            g_lm = torch.empty_like(loc_mean) if want_lm else None
-            iws = torch.empty(lib.nb_egno_input_grad_workspace_floats(ctypes.byref(cfg)), device=dev, dtype=torch.float32)
-            check(lib.nb_egno_backward_ex(ctypes.byref(cfg), _ptr(flat), _ptr(nodes), _ptr(edge_fea), _ptr(loc_mean),
-                                          _ptr(tsteps), _ptr(tsteps_in), _ptr(saved), _ptr(gx_out), _ptr(gv_out),
-                                          _ptr(gh_out), _ptr(grad_flat), _ptr(gx_in), _ptr(gv_in), _ptr(g_nodes),
-                                          _ptr(g_ef), _ptr(g_lm), _ptr(ws), _ptr(iws), _stream_ptr(dev)),
-                  "nb_egno_backward_ex")
-        else:
-            check(lib.nb_egno_backward(ctypes.byref(cfg), _ptr(flat), _ptr(nodes), _ptr(edge_fea), _ptr(loc_mean),
-                                       _ptr(tsteps), _ptr(tsteps_in), _ptr(saved), _ptr(gx_out), _ptr(gv_out), _ptr(gh_out),
-                                       _ptr(grad_flat), _ptr(gx_in), _ptr(gv_in), _ptr(ws), _stream_ptr(dev)),
-                  "nb_egno_backward")
-        return EgnoFunction._finish(ctx, grad_flat, gx_in, g_nodes, g_ef, gv_in, g_lm, None, None)
-
-    @staticmethod
-    def _backward_ft(ctx, lib, cfg, flat, nodes, edge_fea, loc_mean, tsteps, tsteps_in, saved, gx_out, gv_out, gh_out,
-                     grad_flat, gx_in, gv_in, ws):
-        """Floating-point times: nb_egno_backward_ft, which also returns dL/dtimesteps_out / dL/dtimesteps_in when asked
-        (per shard under data parallelism, like the other input gradients)."""
-        dev = flat.device
+        # per-shard input gradients: under data parallelism nothing beyond the parameter bucket is reduced
         want = ctx.needs_input_grad
         g_nodes = torch.empty_like(nodes) if want[4] else None
         g_ef = torch.empty_like(edge_fea) if want[5] else None
         g_lm = torch.empty_like(loc_mean) if want[7] else None
-        g_t = torch.empty_like(tsteps) if want[8] else None
-        g_t_in = torch.empty_like(tsteps_in) if want[9] else None
         iws = None
         if want[4] or want[5]:
             iws = torch.empty(lib.nb_egno_input_grad_workspace_floats(ctypes.byref(cfg)), device=dev, dtype=torch.float32)
-        check(lib.nb_egno_backward_ft(ctypes.byref(cfg), _ptr(flat), _ptr(nodes), _ptr(edge_fea), _ptr(loc_mean),
-                                      _ptr(tsteps), _ptr(tsteps_in), _ptr(saved), _ptr(gx_out), _ptr(gv_out), _ptr(gh_out),
-                                      _ptr(grad_flat), _ptr(gx_in), _ptr(gv_in), _ptr(g_nodes), _ptr(g_ef), _ptr(g_lm),
-                                      _ptr(g_t), _ptr(g_t_in), _ptr(ws), _ptr(iws), _stream_ptr(dev)), "nb_egno_backward_ft")
-        return EgnoFunction._finish(ctx, grad_flat, gx_in, g_nodes, g_ef, gv_in, g_lm, g_t, g_t_in)
-
-    @staticmethod
-    def _finish(ctx, grad_flat, gx_in, g_nodes, g_ef, gv_in, g_lm, g_t, g_t_in):
+        args = [ctypes.byref(cfg), _ptr(flat), _ptr(nodes), _ptr(edge_fea), _ptr(loc_mean), _ptr(tsteps), _ptr(tsteps_in),
+                _ptr(saved), _ptr(gx_out), _ptr(gv_out), _ptr(gh_out), _ptr(grad_flat), _ptr(gx_in), _ptr(gv_in),
+                _ptr(g_nodes), _ptr(g_ef), _ptr(g_lm)]
+        g_t = g_t_in = None
+        if tsteps.is_floating_point():   # fp32 times: the _ft entry point, which also returns dL/dtimes when asked
+            g_t = torch.empty_like(tsteps) if want[8] else None
+            g_t_in = torch.empty_like(tsteps_in) if want[9] else None
+            bwd, args = "nb_egno_backward_ft", args + [_ptr(g_t), _ptr(g_t_in)]
+        else:
+            bwd = "nb_egno_backward_ex"
+        check(getattr(lib, bwd)(*args, _ptr(ws), _ptr(iws), _stream_ptr(dev)), bwd)
         _maybe_allreduce(grad_flat, ctx.dp_group)
         grads, o = [], 0
         for shp in ctx.param_shapes:
@@ -277,22 +250,17 @@ class SegnoFunction(torch.autograd.Function):
         ws = torch.empty(lib.nb_segno_workspace_floats(ctypes.byref(cfg), 1), device=dev, dtype=torch.float32)
         gh_in = torch.empty((Nn, 64), device=dev, dtype=torch.float32) if cfg.h_given else None
         want_his = ctx.needs_input_grad[3] and not cfg.h_given
-        want_ef = ctx.needs_input_grad[6]
-        g_his = g_ea = None
-        if want_his or want_ef:
-            g_his = torch.empty_like(his) if want_his else None
-            g_ea = torch.empty_like(edge_attr) if want_ef else None
+        g_his = torch.empty_like(his) if want_his else None
+        g_ea = torch.empty_like(edge_attr) if ctx.needs_input_grad[6] else None
+        iws = None
+        if g_ea is not None:
             iws = torch.empty(lib.nb_segno_input_grad_workspace_floats(ctypes.byref(cfg)), device=dev, dtype=torch.float32)
-            check(lib.nb_segno_backward_ex(ctypes.byref(cfg), _ptr(flat), _ptr(his), _ptr(edge_attr), _ptr(saved),
-                                           _ptr(gx_out), _ptr(gh_out), _ptr(gv_out), _ptr(grad_flat), _ptr(gx_in),
-                                           _ptr(gv_in), _ptr(gh_in), _ptr(g_his), _ptr(g_ea), _ptr(ws), _ptr(iws),
-                                           _stream_ptr(dev)), "nb_segno_backward_ex")
-            if want_his:
-                gh_in = g_his
-        else:
-            check(lib.nb_segno_backward(ctypes.byref(cfg), _ptr(flat), _ptr(his), _ptr(edge_attr), _ptr(saved),
-                                        _ptr(gx_out), _ptr(gh_out), _ptr(gv_out), _ptr(grad_flat), _ptr(gx_in),
-                                        _ptr(gv_in), _ptr(gh_in), _ptr(ws), _stream_ptr(dev)), "nb_segno_backward")
+        check(lib.nb_segno_backward_ex(ctypes.byref(cfg), _ptr(flat), _ptr(his), _ptr(edge_attr), _ptr(saved),
+                                       _ptr(gx_out), _ptr(gh_out), _ptr(gv_out), _ptr(grad_flat), _ptr(gx_in),
+                                       _ptr(gv_in), _ptr(gh_in), _ptr(g_his), _ptr(g_ea), _ptr(ws), _ptr(iws),
+                                       _stream_ptr(dev)), "nb_segno_backward_ex")
+        if want_his:
+            gh_in = g_his
         _maybe_allreduce(grad_flat, ctx.dp_group)
         grads, o = [], 0
         for shp in ctx.param_shapes:
